@@ -13,7 +13,14 @@ are exchanged on the host, every rank searches the streams it owns (static parti
 stream order.  No data-path collective (SURVEY.md 8e); torch.distributed carries the barrier, the host-side record exchange (gloo)
 and the max-over-ranks of the times.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c5|c2|c3|c4|c1] [--streams S]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c5|c2|c3|c4|c1] [--streams S] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned (rank 0), so that two builds can be compared output for output on the
+same seeded container: records.npy (float64, one row per stream, columns antiz_b200.shard.FIELDS), diff_offsets.npy (float64) and
+diff_values.npy (float32), the diff lists of all streams in stream order (written only when some stream has a diff list: the
+default workload has none), and payload_sample.npy (float32): the recompressed streams'
+plaintext as the e2e step copies it to the host (rank 0's share), sampled at PAYLOAD_SAMPLE sorted positions drawn with
+numpy.random.default_rng(0) when it is longer than that.
 """
 import argparse
 import hashlib
@@ -42,6 +49,7 @@ WORKLOADS = {
 }
 CHUNKSIZE = 524288
 SEED = 2
+PAYLOAD_SAMPLE = 8 << 20        # float32 values: 32 MB at most
 
 
 def _gen_part(args):
@@ -150,9 +158,14 @@ def run_reference_cli(files, flags):
     return dt
 
 
+def _zlib_name():
+    import zref
+    return "reference zlib 1.2.8" if zref.have_ref() else "host zlib " + zref.host_zlib().zlibVersion().decode()
+
+
 def base_config(a, desc, flags, N, nstreams):
     """the part of `config` both arms state identically (same workload, same bytes)"""
-    return {"workload": desc, "container_bytes": int(N), "generator": f"tests/corpus.py {a.workload}({nstreams}), seed {SEED}, reference zlib 1.2.8", "flags": flags, "chunksize": CHUNKSIZE}
+    return {"workload": desc, "container_bytes": int(N), "generator": f"tests/corpus.py {a.workload}({nstreams}), seed {SEED}, {_zlib_name()}", "flags": flags, "chunksize": CHUNKSIZE}
 
 
 def reference_arm(a, rank, world):
@@ -242,6 +255,21 @@ def cpu_baseline_and_parity(a, flags, data, parts):
     return cpu, par
 
 
+def dump_outputs(d, recs, payload):
+    """--dump-outputs: recs = gathered records (record tuple in shard.FIELDS order, diff offsets, diff values); payload = uint8 array"""
+    import numpy as np
+    from antiz_b200 import shard
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "records.npy"), np.array([r[0] for r in recs], dtype=np.float64).reshape(len(recs), len(shard.FIELDS)))
+    offs = [o for r in recs for o in r[1]]
+    if offs:        # (the ndiff column of records.npy says when there are none)
+        np.save(os.path.join(d, "diff_offsets.npy"), np.array(offs, dtype=np.float64))
+        np.save(os.path.join(d, "diff_values.npy"), np.frombuffer(b"".join(r[2] for r in recs), dtype=np.uint8).astype(np.float32))
+    if payload.size > PAYLOAD_SAMPLE:
+        payload = payload[np.sort(np.random.default_rng(0).integers(0, payload.size, PAYLOAD_SAMPLE))]
+    np.save(os.path.join(d, "payload_sample.npy"), payload.astype(np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -252,6 +280,7 @@ def main():
     ap.add_argument("--streams", type=int, default=int(os.environ.get("ATZ_BENCH_STREAMS", "0")))
     ap.add_argument("--cpu-sample-mb", type=float, default=0.0)
     ap.add_argument("--no-c2", action="store_true", help="skip the short configs[1] run reported under \"c2\"")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's records, diffs and a payload sample as DIR/<name>.npy")
     a = ap.parse_args()
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     if a.impl == "reference":
@@ -355,17 +384,20 @@ def main():
             dist.all_reduce(t, op=dist.ReduceOp.SUM)
             tot = [float(x) for x in t.tolist()]
         return {"n": n, "ms_dev": ms_dev, "ms_e2e": ms_e2e, "agg": agg, "records": recs, "ref_trials": tot[0], "gpu_trials": tot[1], "d2h": tot[2], "algo_bytes": tot[3],
-                "h2d_ms_last": h2d, "payload_cap": cap}
+                "h2d_ms_last": h2d, "payload_cap": cap, "payload": out_pinned.numpy()[:state["got"]]}
 
     sampler = ClockSampler(local)
     host = torch.from_numpy(data).pin_memory()                                        # e2e source: pinned host memory
     res = run_workload(host, az.Options(**okw), a.steps, a.warmup, lambda on: sampler.start() if on else None)
     clocks = sampler.finish()
     del host
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, res["records"], res["payload"])
+    del res["payload"]
     c2 = None
     if c2_data is not None:
         h2 = torch.from_numpy(c2_data).pin_memory()
-        c2 = run_workload(h2, az.Options(), 3, 3)
+        c2 = run_workload(h2, az.Options(), a.steps, 3)
         del h2
     if rank == 0:
         peaks = {}
@@ -410,8 +442,8 @@ def main():
         }
         if c2 is not None:
             n2 = c2["n"]
-            line["c2"] = {"workload": WORKLOADS["c2"][0], "container_bytes": int(n2), "steps": 3, "value": n2 * 3 / (c2["ms_dev"] / 1e3) / 1e6, "unit": "MB/s",
-                          "e2e": n2 * 3 / (c2["ms_e2e"] / 1e3) / 1e6, "ms_per_step": c2["ms_dev"] / 3, "streams": len(c2["records"])}
+            line["c2"] = {"workload": WORKLOADS["c2"][0], "container_bytes": int(n2), "steps": a.steps, "value": n2 * a.steps / (c2["ms_dev"] / 1e3) / 1e6, "unit": "MB/s",
+                          "e2e": n2 * a.steps / (c2["ms_e2e"] / 1e3) / 1e6, "ms_per_step": c2["ms_dev"] / a.steps, "streams": len(c2["records"])}
         if cpu is not None:
             line["cpu_baseline"] = cpu
             line.update(par)

@@ -1,5 +1,6 @@
-"""Seeded synthetic deflate-bearing containers (SURVEY.md 8d), built with the reference's own zlib 1.2.8
-(oracle/_ref/libz128.so).  TEST / BENCH INFRASTRUCTURE ONLY."""
+"""Seeded synthetic deflate-bearing containers (SURVEY.md 8d), built with zref.zlib_lib(): the reference's own zlib 1.2.8 where it
+has been built, else the host's zlib and, at level 0, the oracle: the same bytes (Z_FIXED aside, where zlib 1.2.12 changed).
+TEST / BENCH INFRASTRUCTURE ONLY."""
 import random
 import numpy as np
 import zref

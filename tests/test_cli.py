@@ -1,17 +1,17 @@
 """The `uncomp` host program's argument handling and ATZ1 reader errors (no GPU needed for these paths)."""
+import json
 import os
 import struct
 import subprocess
 import tempfile
-
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 UNCOMP = os.path.join(ROOT, "antiz_b200", "uncomp")
 
 
 def run(*a):
-    return subprocess.run([UNCOMP] + list(a), capture_output=True, text=True)
+    # started as `uncomp` (argv[0]) wherever the checkout lies: TCLAP wraps the usage text relative to the program name
+    return subprocess.run(["uncomp"] + list(a), executable=UNCOMP, capture_output=True, text=True)
 
 
 def test_missing_input_is_a_parse_error():
@@ -50,23 +50,37 @@ CLI_CASES = ["", "--bogus", "--version", "-i", "--input", "-r", "-i x --recomp-t
              "-i x extra", "-i x --notest --notest", "-i nosuchfile -- foo bar", "-o y", "-i x -o", "--shortcut-len 5 --shortcut-len 6 -i x"]
 
 
-@pytest.mark.skipif(not os.path.exists(REF), reason="oracle/_ref/uncomp_ref not built")
+GOLDEN_CLI = os.path.join(ROOT, "tests", "golden", "cli_reference.json")
+EXTENSIONS = "antiz_b200 extensions: "
+
+
+def cli_texts(exe, tmp):
+    """{args: [exit code, stdout, stderr]} of `./uncomp args` for CLI_CASES and --help, with `exe` started as ./uncomp (the usage
+    line is wrapped relative to the program name).  This project's --help goes on after the reference's text with its extensions:
+    only the reference's part is kept."""
+    d = os.path.join(tmp, os.path.basename(exe) + "_dir")
+    os.mkdir(d); os.symlink(exe, os.path.join(d, "uncomp"))
+    out = {}
+    for args in CLI_CASES + ["--help"]:
+        p = subprocess.run(["./uncomp"] + args.split(), cwd=d, capture_output=True, text=True)
+        out[args] = [p.returncode, p.stdout.split(EXTENSIONS)[0] if args == "--help" else p.stdout, p.stderr]
+    return out
+
+
 def test_cli_texts_equal_the_reference_binary():
-    """usage, help, version and parse-error texts (stdout, stderr, exit code) against the reference's TCLAP front end, both
-    programs started under the same argv[0] (the usage line is wrapped relative to the program name)"""
+    """usage, help, version and parse-error texts (stdout, stderr, exit code) against the reference's TCLAP front end: the
+    reference binary where it has been built, else the stored record of its texts"""
     with tempfile.TemporaryDirectory() as tmp:
-        for d, exe in (("a", REF), ("b", UNCOMP)):
-            os.mkdir(os.path.join(tmp, d)); os.symlink(exe, os.path.join(tmp, d, "uncomp"))
-        def both(args):
-            return [subprocess.run(["./uncomp"] + args.split(), cwd=os.path.join(tmp, d), capture_output=True, text=True) for d in ("a", "b")]
+        want = cli_texts(REF, tmp) if os.path.exists(REF) else json.load(open(GOLDEN_CLI))
         for args in CLI_CASES:
-            r, u = both(args)
-            assert (r.returncode, r.stdout, r.stderr) == (u.returncode, u.stdout, u.stderr), args
+            p = subprocess.run(["./uncomp"] + args.split(), cwd=tmp, executable=UNCOMP, capture_output=True, text=True)
+            assert [p.returncode, p.stdout, p.stderr] == want[args], args
         # --help: the reference's text, then the extensions of this implementation
-        r, u = both("--help")
-        assert r.returncode == u.returncode == 0 and u.stdout.startswith(r.stdout) and r.stderr == u.stderr
-        rest = u.stdout[len(r.stdout):]
-        assert rest.startswith("antiz_b200 extensions: ") and all(f in rest for f in ("--gpus <integer>", "--device <integer>", "--exact-records", "--stats"))
+        r = want["--help"]
+        u = subprocess.run(["./uncomp", "--help"], cwd=tmp, executable=UNCOMP, capture_output=True, text=True)
+        assert r[0] == u.returncode == 0 and u.stdout.startswith(r[1]) and r[2] == u.stderr
+        rest = u.stdout[len(r[1]):]
+        assert rest.startswith(EXTENSIONS) and all(f in rest for f in ("--gpus <integer>", "--device <integer>", "--exact-records", "--stats"))
 
 
 def test_cli_layout_without_the_reference():
@@ -75,8 +89,8 @@ def test_cli_layout_without_the_reference():
     assert p.returncode == 1 and p.stdout == "AntiZ 0.1.6-git\n"
     lines = p.stderr.split("\n")
     assert lines[0] == "PARSE ERROR: Argument: --bogus" and lines[1] == "             Couldn't find match for argument" and lines[3] == "Brief USAGE: "
-    assert all(len(l) <= 75 for l in lines) and lines[4].startswith("   " + UNCOMP + "  [--brute-window] [--notest] [-r]")
-    assert p.stderr.endswith("For complete USAGE and HELP type: \n   " + UNCOMP + " --help\n\n")
+    assert all(len(l) <= 75 for l in lines) and lines[4].startswith("   uncomp  [--brute-window] [--notest] [-r]")
+    assert p.stderr.endswith("For complete USAGE and HELP type: \n   uncomp --help\n\n")
     assert run().stderr.startswith("PARSE ERROR:  \n             Required argument missing: input\n")
     assert run("-i").stderr.startswith("PARSE ERROR: Argument: -i (--input)\n             Missing a value for this argument!\n")
     assert run("-i", "x", "--mismatch-tol", "q").stderr.startswith("PARSE ERROR: Argument: (--mismatch-tol)\n             Couldn't read argument value from string 'q'\n")

@@ -1,5 +1,9 @@
 """-m gpu: whole-path parity.  The emitted ATZ1 file must be byte-identical to the reference binary's
-(oracle/_ref/uncomp_ref, the unmodified main.cpp + zlib 1.2.8) for the same flags, and reconstruction must be bit-exact."""
+(oracle/_ref/uncomp_ref, the unmodified main.cpp + zlib 1.2.8) for the same flags, and reconstruction must be bit-exact.
+Where the reference has not been built, its .atz files are known by their sha256 and summary lines, stored for every input of
+this module in tests/golden/atz_reference.json (tests/golden/make_atz_golden.py)."""
+import hashlib
+import json
 import os
 import subprocess
 import tempfile
@@ -14,6 +18,8 @@ from test_host_logic import _magic_positions
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 UNCOMP = os.path.join(ROOT, "antiz_b200", "uncomp")
+GOLDEN_ATZ = os.path.join(ROOT, "tests", "golden", "atz_reference.json")
+KEEP = ("Total zlib headers found", "recompressed:", "Total bytes written")
 
 CASES = [
     ("c1_single_1MiB_text", lambda: corpus.c1(), []),
@@ -42,45 +48,8 @@ CASES = [
 ]
 
 
-@pytest.mark.skipif(not os.path.exists(zref.REF_BIN), reason="oracle/_ref/uncomp_ref not built")
-@pytest.mark.parametrize("name,make,flags", CASES, ids=[c[0] for c in CASES])
-def test_atz_identical_to_reference_binary(name, make, flags):
-    data = make()
-    with tempfile.TemporaryDirectory(dir="/dev/shm" if os.path.isdir("/dev/shm") else None) as tmp:
-        f = os.path.join(tmp, "in.bin")
-        open(f, "wb").write(data)
-        ref = subprocess.run([zref.REF_BIN, "-i", f, "-o", f + ".ref.atz", "--notest"] + flags, capture_output=True, text=True)
-        assert ref.returncode == 0, ref.stdout
-        gpu = subprocess.run([UNCOMP, "-i", f, "-o", f + ".gpu.atz"] + flags, capture_output=True, text=True)
-        assert gpu.returncode == 0, gpu.stdout + gpu.stderr
-        assert "OK! Restoration is bit by bit identical" in gpu.stdout
-        a = open(f + ".ref.atz", "rb").read(); b = open(f + ".gpu.atz", "rb").read()
-        assert a == b, f"{name}: ATZ differs (sizes {len(a)} {len(b)})"
-        keep = ("Total zlib headers found", "recompressed:", "Total bytes written")
-        assert [l for l in ref.stdout.splitlines() if l.startswith(keep)] == [l for l in gpu.stdout.splitlines() if l.startswith(keep)]
-        # our reconstructor on the reference's ATZ, and the reference's reconstructor on ours
-        r1 = subprocess.run([UNCOMP, "-r", "-i", f + ".ref.atz", "-o", f + ".rec1"], capture_output=True, text=True)
-        assert r1.returncode == 0 and open(f + ".rec1", "rb").read() == data
-        r2 = subprocess.run([zref.REF_BIN, "-r", "-i", f + ".gpu.atz", "-o", f + ".rec2"], capture_output=True, text=True)
-        assert r2.returncode == 0 and open(f + ".rec2", "rb").read() == data
-
-
-@pytest.mark.skipif(not os.path.exists(zref.REF_BIN), reason="oracle/_ref/uncomp_ref not built")
-def test_batched_probe_equals_reference():
-    """more candidates than slots (forced with ATZ_SLOT_BATCH): probed in batches, accepted streams inflated again"""
-    data = corpus.c4(400, 45) + corpus.c2(6, 46)
-    with tempfile.TemporaryDirectory(dir="/dev/shm" if os.path.isdir("/dev/shm") else None) as tmp:
-        f = os.path.join(tmp, "in.bin"); open(f, "wb").write(data)
-        ref = subprocess.run([zref.REF_BIN, "-i", f, "-o", f + ".ref.atz", "--notest"], capture_output=True, text=True)
-        gpu = subprocess.run([UNCOMP, "-i", f, "-o", f + ".gpu.atz"], capture_output=True, text=True, env=dict(os.environ, ATZ_SLOT_BATCH="97"))
-        assert ref.returncode == 0 and gpu.returncode == 0, gpu.stdout + gpu.stderr
-        assert open(f + ".ref.atz", "rb").read() == open(f + ".gpu.atz", "rb").read()
-
-
-@pytest.mark.skipif(not os.path.exists(zref.REF_BIN), reason="oracle/_ref/uncomp_ref not built")
-def test_strategies_extension_recompresses_what_the_reference_cannot():
-    """--strategies (SURVEY.md 8 f4): streams made with Z_FILTERED / Z_FIXED / Z_RLE / Z_HUFFMAN_ONLY, which no candidate of the
-    reference reproduces, are recompressed and reconstruct bit-exactly; without the flag the ATZ file stays the reference's"""
+def _strategies_data():
+    """streams made with Z_FILTERED / Z_FIXED / Z_RLE / Z_HUFFMAN_ONLY, which no candidate of the reference reproduces"""
     import random
     r = random.Random(77)
     ss = []
@@ -89,14 +58,78 @@ def test_strategies_extension_recompresses_what_the_reference_cannot():
         strat = [1, 2, 3, 4][i % 4]
         lvl = r.randint(4, 9) if strat == 1 else r.randint(1, 9)
         ss.append(zref.ref_deflate(d, lvl, r.choice([12, 15]), r.choice([8, 9, 4]), strat))
-    data = corpus.container(ss, 78)[0]
+    return corpus.container(ss, 78)[0]
+
+
+def reference_inputs():
+    """key -> (input maker, flags) of every comparison with the reference binary in this module"""
+    d = {name: (make, flags) for name, make, flags in CASES}
+    d["batched_probe"] = (lambda: corpus.c4(400, 45) + corpus.c2(6, 46), [])
+    d["strategies"] = (_strategies_data, [])
+    d["gpus_mixed_brute_window"] = (lambda: corpus.mixed(2500000, 91), ["--brute-window"])
+    d["gpus_c2_chunks"] = (lambda: corpus.c2(60, 92, 1 << 10, 128 << 10), ["--chunksize", "100000"])
+    return d
+
+
+def sha256(path):
+    return hashlib.sha256(open(path, "rb").read()).hexdigest()
+
+
+def reference_atz(key, f, flags):
+    """(sha256 of the reference binary's .atz, its summary lines) for input file f: from the binary where it has been built (its
+    .atz is left at f + ".ref.atz"), else from the stored record, which must be for the same input bytes"""
+    if os.path.exists(zref.REF_BIN):
+        ref = subprocess.run([zref.REF_BIN, "-i", f, "-o", f + ".ref.atz", "--notest"] + flags, capture_output=True, text=True)
+        assert ref.returncode == 0, ref.stdout
+        return sha256(f + ".ref.atz"), [l for l in ref.stdout.splitlines() if l.startswith(KEEP)]
+    g = json.load(open(GOLDEN_ATZ))[key]
+    assert g["flags"] == flags and g["input_sha256"] == sha256(f), f"{key}: the input is not the one the stored record was made for"
+    return g["atz_sha256"], g["lines"]
+
+
+@pytest.mark.parametrize("name,make,flags", CASES, ids=[c[0] for c in CASES])
+def test_atz_identical_to_reference_binary(name, make, flags):
+    data = make()
+    with tempfile.TemporaryDirectory(dir="/dev/shm" if os.path.isdir("/dev/shm") else None) as tmp:
+        f = os.path.join(tmp, "in.bin")
+        open(f, "wb").write(data)
+        want, lines = reference_atz(name, f, flags)
+        gpu = subprocess.run([UNCOMP, "-i", f, "-o", f + ".gpu.atz"] + flags, capture_output=True, text=True)
+        assert gpu.returncode == 0, gpu.stdout + gpu.stderr
+        assert "OK! Restoration is bit by bit identical" in gpu.stdout
+        assert sha256(f + ".gpu.atz") == want, f"{name}: ATZ differs"
+        assert lines == [l for l in gpu.stdout.splitlines() if l.startswith(KEEP)]
+        # our reconstructor on the reference's ATZ (the same bytes as ours), and the reference's reconstructor on ours
+        r1 = subprocess.run([UNCOMP, "-r", "-i", f + ".gpu.atz", "-o", f + ".rec1"], capture_output=True, text=True)
+        assert r1.returncode == 0 and open(f + ".rec1", "rb").read() == data
+        if os.path.exists(zref.REF_BIN):
+            r2 = subprocess.run([zref.REF_BIN, "-r", "-i", f + ".gpu.atz", "-o", f + ".rec2"], capture_output=True, text=True)
+            assert r2.returncode == 0 and open(f + ".rec2", "rb").read() == data
+
+
+def test_batched_probe_equals_reference():
+    """more candidates than slots (forced with ATZ_SLOT_BATCH): probed in batches, accepted streams inflated again"""
+    make, flags = reference_inputs()["batched_probe"]
+    data = make()
     with tempfile.TemporaryDirectory(dir="/dev/shm" if os.path.isdir("/dev/shm") else None) as tmp:
         f = os.path.join(tmp, "in.bin"); open(f, "wb").write(data)
-        ref = subprocess.run([zref.REF_BIN, "-i", f, "-o", f + ".ref.atz", "--notest"], capture_output=True, text=True)
+        want, _ = reference_atz("batched_probe", f, flags)
+        gpu = subprocess.run([UNCOMP, "-i", f, "-o", f + ".gpu.atz"] + flags, capture_output=True, text=True, env=dict(os.environ, ATZ_SLOT_BATCH="97"))
+        assert gpu.returncode == 0, gpu.stdout + gpu.stderr
+        assert sha256(f + ".gpu.atz") == want
+
+
+def test_strategies_extension_recompresses_what_the_reference_cannot():
+    """--strategies (SURVEY.md 8 f4): streams made with Z_FILTERED / Z_FIXED / Z_RLE / Z_HUFFMAN_ONLY, which no candidate of the
+    reference reproduces, are recompressed and reconstruct bit-exactly; without the flag the ATZ file stays the reference's"""
+    data = _strategies_data()
+    with tempfile.TemporaryDirectory(dir="/dev/shm" if os.path.isdir("/dev/shm") else None) as tmp:
+        f = os.path.join(tmp, "in.bin"); open(f, "wb").write(data)
+        want, _ = reference_atz("strategies", f, [])
         plain = subprocess.run([UNCOMP, "-i", f, "-o", f + ".gpu.atz", "--notest"], capture_output=True, text=True)
         ext = subprocess.run([UNCOMP, "-i", f, "-o", f + ".ext.atz", "--strategies"], capture_output=True, text=True)
-        assert ref.returncode == 0 and plain.returncode == 0 and ext.returncode == 0, ext.stdout + ext.stderr
-        assert open(f + ".ref.atz", "rb").read() == open(f + ".gpu.atz", "rb").read()
+        assert plain.returncode == 0 and ext.returncode == 0, ext.stdout + ext.stderr
+        assert sha256(f + ".gpu.atz") == want
         assert "OK! Restoration is bit by bit identical" in ext.stdout
         count = lambda out: [int(x) for x in [l for l in out.splitlines() if l.startswith("recompressed:")][0].split(":")[1].split("/")]
         got, found = count(ext.stdout)       # (a stream that crosses the 524,288-byte chunk boundary is not detected, as in the reference)
@@ -187,7 +220,6 @@ def test_sharded_scan_and_search_equal_single(nsh, chunksize):
         c.close()
 
 
-@pytest.mark.skipif(not os.path.exists(zref.REF_BIN), reason="oracle/_ref/uncomp_ref not built")
 @pytest.mark.parametrize("gpus", [2, 4, 8])
 def test_uncomp_gpus_equals_reference(gpus):
     """`uncomp --gpus N`: one container sharded over N contexts in one process, .atz byte-identical to --gpus 1 and to uncomp_ref.
@@ -198,16 +230,16 @@ def test_uncomp_gpus_equals_reference(gpus):
     env = dict(os.environ)
     if ndev < gpus:
         env["ATZ_TEST_ONE_DEVICE"] = "1"
-    for data, flags in ((corpus.mixed(2500000, 91), ["--brute-window"]), (corpus.c2(60, 92, 1 << 10, 128 << 10), ["--chunksize", "100000"])):
+    for key in ("gpus_mixed_brute_window", "gpus_c2_chunks"):
+        make, flags = reference_inputs()[key]
         with tempfile.TemporaryDirectory(dir="/dev/shm" if os.path.isdir("/dev/shm") else None) as tmp:
-            f = os.path.join(tmp, "in.bin"); open(f, "wb").write(data)
-            ref = subprocess.run([zref.REF_BIN, "-i", f, "-o", f + ".ref.atz", "--notest"] + flags, capture_output=True, text=True)
+            f = os.path.join(tmp, "in.bin"); open(f, "wb").write(make())
+            want, _ = reference_atz(key, f, flags)
             one = subprocess.run([UNCOMP, "-i", f, "-o", f + ".g1.atz", "--notest"] + flags, capture_output=True, text=True)
             many = subprocess.run([UNCOMP, "-i", f, "-o", f + ".gn.atz", "--gpus", str(gpus)] + flags, capture_output=True, text=True, env=env)
-            assert ref.returncode == 0 and one.returncode == 0 and many.returncode == 0, many.stdout + many.stderr
+            assert one.returncode == 0 and many.returncode == 0, many.stdout + many.stderr
             assert "OK! Restoration is bit by bit identical" in many.stdout
-            a = open(f + ".ref.atz", "rb").read()
-            assert a == open(f + ".g1.atz", "rb").read() == open(f + ".gn.atz", "rb").read()
+            assert want == sha256(f + ".g1.atz") == sha256(f + ".gn.atz")
 
 
 def test_small_budget_batches_and_deferrals_do_not_change_records():

@@ -16,8 +16,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.fixture(scope="module")
-def scanner():
-    exe = os.path.join(tempfile.gettempdir(), "atz_zlibwrapper_scan")
+def scanner(tmp_path_factory):
+    exe = str(tmp_path_factory.mktemp("scanner") / "atz_zlibwrapper_scan")
     subprocess.check_call(["g++", "-std=c++17", "-O2", "-Wall", "-I", os.path.join(ROOT, "include"), "-I", os.path.join(ROOT, "antiz_b200", "host"),
                            os.path.join(ROOT, "tests", "zlibwrapper_scan.cpp"), "-o", exe, "-L", os.path.join(ROOT, "antiz_b200"), "-lantiz_b200",
                            "-Wl,-rpath," + os.path.join(ROOT, "antiz_b200")])

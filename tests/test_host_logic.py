@@ -1,7 +1,10 @@
 """Host logic of the product pinned on the CPU: the reference's candidate order (SURVEY.md A.2), chunk list and the
 ZBuffSearcher accept logic (A.1).  The accept logic is driven with probe records from the CPU oracle and compared with
-what the reference binary (oracle/_ref/uncomp_ref) finds on the same file."""
+what the reference binary (oracle/_ref/uncomp_ref) finds on the same file - or, where it has not been built, with the stored
+record of what it finds (tests/golden/atz_reference.json)."""
 import ctypes as C
+import hashlib
+import json
 import os
 import random
 import struct
@@ -150,10 +153,14 @@ def _fold_with_oracle(data, S):
     return [(out[3 * i], out[3 * i + 1], out[3 * i + 2]) for i in range(k)]
 
 
-def _reference_streams(data, S, tmp):
+GOLDEN_ATZ = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "atz_reference.json")
+
+
+def atz_streams(exe, data, S, tmp):
+    """(headers found, [(offset, streamLength, inflatedLength) of every recompressed stream]) of `exe -i file --notest --chunksize S`"""
     f = os.path.join(tmp, "in.bin")
     open(f, "wb").write(data)
-    out = subprocess.check_output([zref.REF_BIN, "-i", f, "--notest", "--chunksize", str(S)]).decode()
+    out = subprocess.check_output([exe, "-i", f, "--notest", "--chunksize", str(S)]).decode()
     found = int([l for l in out.splitlines() if l.startswith("Total zlib headers found")][0].split(":")[1])
     atz = open(f + ".atz", "rb").read()
     nrec = struct.unpack_from("<Q", atz, 20)[0]
@@ -164,29 +171,50 @@ def _reference_streams(data, S, tmp):
     return found, recs
 
 
-@pytest.mark.skipif(not os.path.exists(zref.REF_BIN), reason="oracle/_ref/uncomp_ref not built")
-@pytest.mark.parametrize("S", [524288, 40000, 4099, 1000])
-def test_scan_fold_matches_reference_binary(S):
+def _reference_streams(key, data, S, tmp):
+    if os.path.exists(zref.REF_BIN):
+        return atz_streams(zref.REF_BIN, data, S, tmp)
+    g = json.load(open(GOLDEN_ATZ))[key]
+    assert g["chunksize"] == S and g["input_sha256"] == hashlib.sha256(data).hexdigest(), f"{key}: not the input the stored record was made for"
+    return g["found"], [tuple(r) for r in g["records"]]
+
+
+FOLD_SIZES = [524288, 40000, 4099, 1000]
+QUIRK_CASES = [(5000, 91), (3000, 92), (20000, 93), (4099, 94)]
+
+
+def fold_input(S):
     R = random.Random(S)
     streams = [zref.ref_deflate(corpus.text(R.randint(300, 30000), 100 + i, 400), R.randint(0, 9), 15, 8) for i in range(40)]
     streams += [zref.ref_deflate(b"tiny", 6, 15, 8), zref.ref_deflate(bytes(R.randint(1, 20000)), 9, 15, 8)]
     data, _ = corpus.container(streams, S)
-    data += b"\x78\x9c" + R.randbytes(300)   # false candidates, one of them at the very end
+    return data + b"\x78\x9c" + R.randbytes(300)   # false candidates, one of them at the very end
+
+
+def fold_inputs():
+    """key -> (input, chunk size) of every comparison with the reference binary in this module"""
+    d = {f"scan_fold_{S}": (fold_input(S), S) for S in FOLD_SIZES}
+    d.update({f"overlap_quirk_{S}_{seed}": (corpus.at_chunk_starts(S, seed), S) for S, seed in QUIRK_CASES})
+    return d
+
+
+@pytest.mark.parametrize("S", FOLD_SIZES)
+def test_scan_fold_matches_reference_binary(S):
+    data = fold_input(S)
     with tempfile.TemporaryDirectory() as tmp:
-        found, recs = _reference_streams(data, S, tmp)
+        found, recs = _reference_streams(f"scan_fold_{S}", data, S, tmp)
     got = _fold_with_oracle(data, S)
     assert len(got) == found
     assert [g for g in got if g in set(recs)] == recs   # every stream the reference recompressed, in order
     assert found < 42 or S == 524288                     # small chunks really lose boundary-crossing streams (A.1)
 
 
-@pytest.mark.skipif(not os.path.exists(zref.REF_BIN), reason="oracle/_ref/uncomp_ref not built")
-@pytest.mark.parametrize("S,seed", [(5000, 91), (3000, 92), (20000, 93), (4099, 94)])
+@pytest.mark.parametrize("S,seed", QUIRK_CASES)
 def test_scan_fold_reproduces_the_overlap_byte_quirk(S, seed):
     """streams that start exactly on a chunk start k(S-1), k >= 2 (found at full size: one of configs[3]'s 50,000 streams)"""
     data = corpus.at_chunk_starts(S, seed)
     with tempfile.TemporaryDirectory() as tmp:
-        found, recs = _reference_streams(data, S, tmp)
+        found, recs = _reference_streams(f"overlap_quirk_{S}_{seed}", data, S, tmp)
     got = _fold_with_oracle(data, S)
     assert len(got) == found and [g for g in got if g in set(recs)] == recs
     # the quirk really decides something here: the plain "repeat the last byte" model finds a different number of streams

@@ -1,9 +1,10 @@
-"""ctypes access to the *reference's own* zlib 1.2.8 (oracle/_ref/libz128.so, built
-from /root/reference by oracle/build_ref.sh) and to the CPU oracle (oracle/liboracle.so).
+"""ctypes access to zlib - the *reference's own* zlib 1.2.8 (oracle/_ref/libz128.so, built by oracle/build_ref.sh where the
+reference sources are present), else the host's zlib - and to the CPU oracle (oracle/liboracle.so).
 
 TEST INFRASTRUCTURE ONLY - nothing under antiz_b200/ imports this module.
 """
 import ctypes as C
+import ctypes.util
 import os
 import subprocess
 
@@ -27,6 +28,7 @@ class ZStream(C.Structure):
 
 
 _ref = None
+_host = None
 _oracle = None
 
 
@@ -41,6 +43,24 @@ def ref():
         _ref.zlibVersion.restype = C.c_char_p
         assert _ref.zlibVersion() == b"1.2.8", _ref.zlibVersion()
     return _ref
+
+
+def host_zlib():
+    """the host's zlib (the library Python's zlib module uses).  Its deflate output equals zlib 1.2.8's at levels 1-9 with the
+    default and Z_FILTERED strategies (test_oracle_deflate checks that against the committed 1.2.8 digests), and on the inputs of
+    test_deflate_strategies_bit_exact with every strategy; level 0 differs (stored blocks, rewritten in zlib 1.2.11), and Z_FIXED
+    can (block choice changed in 1.2.12).  Its inflate accounting agrees with the oracle's (test_oracle_inflate)."""
+    global _host
+    if _host is None:
+        _host = C.CDLL(ctypes.util.find_library("z") or "libz.so.1")
+        _host.zlibVersion.restype = C.c_char_p
+    return _host
+
+
+def zlib_lib():
+    """what the ref_* helpers call: zlib 1.2.8 where the reference has been built, the host's zlib everywhere else (ref_deflate
+    then takes level 0 from the oracle, which lays out stored blocks as 1.2.8 does)"""
+    return ref() if have_ref() else host_zlib()
 
 
 def build_oracle():
@@ -62,9 +82,11 @@ def oracle():
     return _oracle
 
 
-def ref_deflate(data: bytes, level: int, wbits: int, memlevel: int, strategy: int = 0) -> bytes:
-    """deflateInit2(level, 8, wbits, memlevel, strategy) + deflate(Z_FINISH) with zlib 1.2.8 (strategy 1 = Z_FILTERED)."""
-    z = ref()
+def ref_deflate(data: bytes, level: int, wbits: int, memlevel: int, strategy: int = 0, z=None) -> bytes:
+    """deflateInit2(level, 8, wbits, memlevel, strategy) + deflate(Z_FINISH) with `z` or zlib_lib() (strategy 1 = Z_FILTERED)."""
+    if z is None and not have_ref() and level == 0 and strategy == 0:
+        return oracle_deflate(data, level, wbits, memlevel)
+    z = z or zlib_lib()
     s = ZStream()
     rc = z.deflateInit2_(C.byref(s), level, 8, wbits, memlevel, strategy, b"1.2.8", C.sizeof(ZStream))
     assert rc == Z_OK, rc
@@ -82,11 +104,11 @@ def ref_deflate(data: bytes, level: int, wbits: int, memlevel: int, strategy: in
 
 
 def ref_deflate_ex(data: bytes, level: int, wbits: int, memlevel: int, strategy: int = 0, flushes=(), tune=None) -> bytes:
-    """zlib 1.2.8 driven the way other encoders drive it: `flushes` = [(input offset, flush mode)] (1 Z_PARTIAL_FLUSH, 2 Z_SYNC_FLUSH,
+    """zlib_lib() driven the way other encoders drive it: `flushes` = [(input offset, flush mode)] (1 Z_PARTIAL_FLUSH, 2 Z_SYNC_FLUSH,
     3 Z_FULL_FLUSH, 5 Z_BLOCK) applied once the input up to that offset has been fed, then Z_FINISH; `tune` = deflateTune's
     (good_length, max_lazy, nice_length, max_chain).  Streams made like this inflate to `data` but are not what any plain
     deflateInit2 + deflate(Z_FINISH) produces: the search finds an imperfect winner or none."""
-    z = ref()
+    z = zlib_lib()
     s = ZStream()
     rc = z.deflateInit2_(C.byref(s), level, 8, wbits, memlevel, strategy, b"1.2.8", C.sizeof(ZStream))
     assert rc == Z_OK, rc
@@ -124,7 +146,7 @@ def ref_inflate_scan(buf: bytes, start: int, outcap: int, segments=None):
     inflate(Z_SYNC_FLUSH) with avail_in = len(buf)-start, avail_out = outcap, then drain
     while avail_out == 0.  Returns (first_total_in, ret, total_in, total_out, avail_in).
     """
-    z = ref()
+    z = zlib_lib()
     s = ZStream()
     rc = z.inflateInit_(C.byref(s), b"1.2.8", C.sizeof(ZStream))
     assert rc == Z_OK
@@ -144,7 +166,7 @@ def ref_inflate_scan(buf: bytes, start: int, outcap: int, segments=None):
 
 def ref_inflate(data: bytes, outlen: int):
     """doInflate (main.cpp:461-486): one-shot inflate(Z_FINISH)."""
-    z = ref()
+    z = zlib_lib()
     s = ZStream()
     assert z.inflateInit_(C.byref(s), b"1.2.8", C.sizeof(ZStream)) == Z_OK
     src = C.create_string_buffer(data, len(data) + 1)

@@ -22,7 +22,7 @@ struct AdlerJob { const uint8_t *in; uint32_t n; uint32_t *out; };
 struct RowTask { const uint8_t *in; uint32_t n; const uint32_t *list, *idx; const uint16_t *lsth; const uint8_t *tmap; uint32_t *rows; uint32_t rlen, budget, chunk0, level, pbegin, visited_only; };
 struct CopyJob { const uint8_t *src; uint8_t *dst; uint64_t n; };
 struct DiffJob { const uint8_t *out; const uint8_t *orig; uint32_t cprime, c; uint32_t *pos; uint8_t *val; uint32_t cap; uint32_t *count; };
-cudaError_t launch_deflate_trials(const TrialDesc *, TrialResult *, uint32_t, uint32_t *, const TrialOpts &, uint32_t *, uint8_t *, uint64_t, int, int, bool, cudaStream_t);
+cudaError_t launch_deflate_trials(const TrialDesc *, TrialResult *, uint32_t, uint32_t *, const TrialOpts &, uint32_t *, uint8_t *, uint64_t, int, bool, cudaStream_t);
 cudaError_t launch_build_chains(const ChainTask *, uint32_t, uint32_t, uint32_t *, uint32_t *, bool, cudaStream_t);
 uint32_t chain_chunk_size();
 cudaError_t launch_adler(const AdlerJob *, uint32_t, cudaStream_t);
@@ -34,7 +34,7 @@ cudaError_t launch_diff(const DiffJob *, uint32_t, cudaStream_t);
 uint32_t scan_tiles_for(uint64_t lo, uint64_t hi);
 cudaError_t launch_scan_count(const uint8_t *, uint64_t, uint64_t, uint64_t, uint32_t *, uint16_t *, uint32_t *, cudaStream_t);
 cudaError_t launch_scan_write(const uint8_t *, uint64_t, uint64_t, const uint16_t *, const uint32_t *, uint32_t *, uint8_t *, uint32_t, cudaStream_t);
-cudaError_t launch_inflate(const uint8_t *, const InflateJob *, InflateResult *, InflateResult *, uint32_t, uint32_t *, uint8_t *, uint64_t, uint64_t, int, int, bool, cudaStream_t);
+cudaError_t launch_inflate(const uint8_t *, const InflateJob *, InflateResult *, InflateResult *, uint32_t, uint32_t *, uint8_t *, uint64_t, uint64_t, int, int, cudaStream_t);
 } // namespace atz
 using namespace atz;
 
@@ -387,19 +387,9 @@ int launch_trials(atz_ctx *ctx, Lane &L, TrialSlot &X, const std::vector<PlainVi
         cost[i] = bytes * per;
     }
     // Queue order: by expected cost, most expensive first (the length of a launch is at least that of its longest trial).
-    // ATZ_TRIAL_ORDER=1 runs a launch stream by stream instead (longest plaintext first, each stream's trials by cost), so that the
-    // trials in flight share a few streams' bucket lists and row tables in L2.
     std::vector<uint32_t> order(sel.size());
     for (uint32_t i = 0; i < order.size(); i++) order[i] = i;
-    const int order_env = getenv("ATZ_TRIAL_ORDER") ? atoi(getenv("ATZ_TRIAL_ORDER")) : -1;   // test hook: 0 = by cost, 1 = by stream
-    const bool by_stream = order_env > 0;    // measured on B200 (c5, 128 MB): 1253 ms per step by stream, 1189 by cost - the tail of the last big streams outweighs the L2 hits; off
-    if (by_stream) {
-        std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) {
-            const uint32_t va = reqs[sel[a]].view, vb = reqs[sel[b]].view;
-            if (va != vb) { const uint32_t na = views[va].n, nb = views[vb].n; return na != nb ? na > nb : va < vb; }
-            return cost[a] > cost[b];
-        });
-    } else std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return cost[a] > cost[b]; });
+    std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return cost[a] > cost[b]; });
     ln.idx.resize(sel.size()); ln.descs.resize(sel.size());
     uint32_t max_fast_n = 0;
     for (size_t k = 0; k < order.size(); k++) {
@@ -420,28 +410,23 @@ int launch_trials(atz_ctx *ctx, Lane &L, TrialSlot &X, const std::vector<PlainVi
     }
     const uint32_t nt = (uint32_t)ln.descs.size();
     uint64_t stride = align_up((uint64_t)max_fast_n / 8 + 64, 256);     // inserted map: one bit per plaintext position
-    static const int force_dense = getenv("ATZ_DENSE") ? atoi(getenv("ATZ_DENSE")) : -1;
-    const bool dense = force_dense >= 0 ? force_dense != 0 : dense_mode >= 0 ? dense_mode != 0 : (int)nt > ctx->sms * 16;
+    const bool dense = dense_mode >= 0 ? dense_mode != 0 : (int)nt > ctx->sms * 16;
     int slots = dense ? ctx->sms * 24 : ctx->sms * 16;     // (64 registers / 32 warps per SM was measured: 763 vs 665 ms per step on the 128 MB mixed corpus)
     if (max_fast_n) {   // bound the inserted-map scratch
         uint64_t lim = std::max<uint64_t>((uint64_t)8 << 30, L.budget / 8);
         while (slots > 64 && (uint64_t)slots * stride > lim) slots /= 2;
     }
-    // one warp per CTA: a warp that finds the queue empty gives its registers and shared memory back at once, so the tail of this
-    // launch (a few long trials) leaves room for the kernels launched next to it
-    static const int wpc_env = getenv("ATZ_TRIAL_WPC") ? std::max(1, std::min(8, atoi(getenv("ATZ_TRIAL_WPC")))) : 1;
-    const int wpc = (int)nt <= ctx->sms * 4 ? 1 : wpc_env;
-    const int ctas = (int)std::min<uint32_t>((uint32_t)(slots / wpc), (nt + wpc - 1) / wpc);
+    const int ctas = (int)std::min<uint32_t>((uint32_t)slots, nt);     // one warp per CTA (launch_deflate_trials)
     CK(X.queue.ensure(64));
-    CK(X.symbuf.ensure((size_t)ctas * wpc * 32768 * 4));
-    if (max_fast_n) CK(X.insmap.ensure((size_t)ctas * wpc * stride));
+    CK(X.symbuf.ensure((size_t)ctas * 32768 * 4));
+    if (max_fast_n) CK(X.insmap.ensure((size_t)ctas * stride));
     CK(X.descs.ensure(nt * sizeof(TrialDesc)));
     CK(X.tres.ensure(nt * sizeof(TrialResult)));
     CK(cudaMemcpyAsync(X.descs.p, ln.descs.data(), nt * sizeof(TrialDesc), cudaMemcpyHostToDevice, X.stream));
     CK(cudaMemsetAsync(X.queue.p, 0, 4, X.stream));
     CK(cudaEventRecord(X.ev0, X.stream));
     CK(launch_deflate_trials(X.descs.as<TrialDesc>(), X.tres.as<TrialResult>(), nt, X.queue.as<uint32_t>(), opts, X.symbuf.as<uint32_t>(),
-                             X.insmap.as<uint8_t>(), stride, ctas, wpc, dense, X.stream));
+                             X.insmap.as<uint8_t>(), stride, ctas, dense, X.stream));
     CK(cudaEventRecord(X.ev1, X.stream));
     ln.tmp.resize(nt);     // (copied back by collect_trials: a device-to-pageable copy queued here would block the host until the kernel is done)
     ln.dense = dense; ln.pending = true;
@@ -828,23 +813,18 @@ static int ensure_range(atz_ctx *ctx, uint64_t a, uint64_t b) {
 // accept logic over them (scan_fold: cheap, deterministic, replicated), partitions the accepted streams (atz_host_partition) and
 // makes sure the plaintext of the streams it owns is resident.  SURVEY.md 8(e); main.cpp:392-420, 205-246.
 static int run_inflate(atz_ctx *ctx, const uint8_t *base, std::vector<InflateJob> &jv, std::vector<InflateResult> &rv, std::vector<InflateResult> &cv, uint8_t *arena,
-                       uint64_t S, double *acc, bool pair) {
+                       uint64_t S, double *acc) {
     if (jv.empty()) return ATZ_OK;
-    const int iwpc = 4; const int islots = ctx->sms * (getenv("ATZ_INFLATE_WARPS") ? atoi(getenv("ATZ_INFLATE_WARPS")) : 16);
-    // pair = two warps per stream (decoder + writer, inflate.cu): for the launches whose length is that of their longest stream
-    // (measured: 35.6 vs 39.0 ms on the PNG-like corpus, 26.2 vs 23.8 ms on configs[1], where fewer streams fit at once: off by default)
-    const bool pair_ok = getenv("ATZ_INFLATE_PAIR") && atoi(getenv("ATZ_INFLATE_PAIR")) != 0;
+    const int iwpc = 4; const int islots = ctx->sms * 16;
     uint32_t nj = (uint32_t)jv.size();
     int wpc = iwpc, ctas;
-    pair = pair && pair_ok;
-    if (pair) { wpc = 4; ctas = (int)std::min<uint32_t>((uint32_t)(islots / wpc), (nj + 1) / 2); }
-    else if ((int)nj <= ctx->sms * 4) { wpc = 1; ctas = (int)nj; } else ctas = (int)std::min<uint32_t>((uint32_t)(islots / wpc), (nj + wpc - 1) / wpc);
+    if ((int)nj <= ctx->sms * 4) { wpc = 1; ctas = (int)nj; } else ctas = (int)std::min<uint32_t>((uint32_t)(islots / wpc), (nj + wpc - 1) / wpc);
     CK(ctx->jobs.ensure(nj * sizeof(InflateJob))); CK(ctx->jres.ensure(nj * sizeof(InflateResult))); CK(ctx->jres2.ensure(nj * sizeof(InflateResult)));
     CK(cudaMemcpyAsync(ctx->jobs.p, jv.data(), nj * sizeof(InflateJob), cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaMemsetAsync(ctx->queue.p, 0, 4, ctx->stream));
     Phase ph(ctx, acc);
     CK(launch_inflate(base, ctx->jobs.as<InflateJob>(), ctx->jres.as<InflateResult>(), ctx->jres2.as<InflateResult>(), nj, ctx->queue.as<uint32_t>(), arena,
-                      S, S, ctas, wpc, pair, ctx->stream));
+                      S, S, ctas, wpc, ctx->stream));
     ph.stop(); ctx->st.kernel_launches++;
     CK(cudaGetLastError());
     rv.resize(nj); cv.resize(nj);
@@ -965,11 +945,11 @@ int atz_scan_shard(atz_ctx *ctx, uint64_t chunksize, uint32_t shard, uint32_t ns
             for (uint64_t b0 = 0; b0 < ncand; b0 += nslot) {
                 const uint64_t b1 = std::min<uint64_t>(ncand, b0 + nslot);
                 CK(cudaMemsetAsync(ctx->plain.p, 0, (b1 - b0) * SLOT + ATZ_PAD, ctx->stream));
-                if (resident) { int rc = run_inflate(ctx, ctx->d_file, jobs, res, cres, ctx->plain.as<uint8_t>(), S, &ctx->st.ms_inflate_probe, false); if (rc) return rc; }
+                if (resident) { int rc = run_inflate(ctx, ctx->d_file, jobs, res, cres, ctx->plain.as<uint8_t>(), S, &ctx->st.ms_inflate_probe); if (rc) return rc; }
                 else {
                     std::vector<InflateJob> bj(jobs.begin() + b0, jobs.begin() + b1); std::vector<InflateResult> br, bc;
                     for (size_t i = 0; i < bj.size(); i++) { bj[i].out_off = (uint64_t)i * SLOT; bj[i].tmap_off = (uint64_t)i * SLOT + QS; }
-                    int rc = run_inflate(ctx, ctx->d_file, bj, br, bc, ctx->plain.as<uint8_t>(), S, &ctx->st.ms_inflate_probe, false); if (rc) return rc;
+                    int rc = run_inflate(ctx, ctx->d_file, bj, br, bc, ctx->plain.as<uint8_t>(), S, &ctx->st.ms_inflate_probe); if (rc) return rc;
                     std::copy(br.begin(), br.end(), res.begin() + b0); std::copy(bc.begin(), bc.end(), cres.begin() + b0);
                 }
             }
@@ -1012,7 +992,7 @@ int atz_scan_shard(atz_ctx *ctx, uint64_t chunksize, uint32_t shard, uint32_t ns
                 uint8_t *base;
                 if (round == 0) { CK(ctx->plain2.ensure(arena + ATZ_PAD)); base = ctx->plain2.as<uint8_t>(); }
                 else { void *q = nullptr; CK(cudaMalloc(&q, arena + ATZ_PAD)); ctx->plain_extra.push_back(q); base = (uint8_t *)q; }
-                { int rc = run_inflate(ctx, ctx->d_file, bj, br, bc, base, S, &ctx->st.ms_inflate, true); if (rc) return rc; }
+                { int rc = run_inflate(ctx, ctx->d_file, bj, br, bc, base, S, &ctx->st.ms_inflate); if (rc) return rc; }
                 if (getenv("ATZ_DEBUG_SCAN")) {
                     std::vector<size_t> o(big.size()); for (size_t i = 0; i < o.size(); i++) o[i] = i;
                     auto tout = [&](size_t i) { return std::max(br[i].total_out, bc[i].status >= 0 ? bc[i].total_out : 0); };
@@ -1161,7 +1141,7 @@ int atz_scan_finish(atz_ctx *ctx, uint64_t *n_streams) {
         }
         void *q = nullptr; CK(cudaMalloc(&q, arena + ATZ_PAD)); ctx->plain_extra.push_back(q);
         CK(cudaMemsetAsync(q, 0, arena + ATZ_PAD, ctx->stream));
-        { int rc = run_inflate(ctx, base, vj, vr, vc, (uint8_t *)q, S, &ctx->st.ms_inflate, true); if (rc) return rc; }
+        { int rc = run_inflate(ctx, base, vj, vr, vc, (uint8_t *)q, S, &ctx->st.ms_inflate); if (rc) return rc; }
         for (size_t i = 0; i < recheck.size(); i++) {
             if (vr[i].status != INF_END || vr[i].total_out != acc[recheck[i]].tout) { ctx->err = "inflate() failed on an accepted stream (reference would abort, main.cpp:451)"; return ATZ_E_DATA; }
             StreamRec &r = ctx->streams[recheck[i]];
@@ -1707,7 +1687,7 @@ int atz_inflate_stream(atz_ctx *ctx, const uint8_t *in, uint64_t n, uint8_t *out
     {
         Phase ph(ctx, &ctx->st.ms_inflate);
         CK(launch_inflate(ctx->op_orig.as<uint8_t>(), ctx->jobs.as<InflateJob>(), ctx->jres.as<InflateResult>(), ctx->jres2.as<InflateResult>(), 1, ctx->queue.as<uint32_t>(),
-                          ctx->op_out.as<uint8_t>(), cap, 2, 1, 1, false, ctx->stream));
+                          ctx->op_out.as<uint8_t>(), cap, 2, 1, 1, ctx->stream));
         ph.stop(); ctx->st.kernel_launches++;
     }
     CK(cudaMemcpyAsync(&r, ctx->jres.p, sizeof r, cudaMemcpyDeviceToHost, ctx->stream));

@@ -20,7 +20,6 @@
 // Search trials never store their output: flushed words are compared with the original stream in flight
 // (the --shortcut-len prefix test, the ident count, the size gate and the mismatch cut are warp reductions).
 #include "common.cuh"
-#include <atomic>
 #include <cstdlib>
 
 namespace atz {
@@ -1136,10 +1135,9 @@ __global__ void __launch_bounds__(256, MINB) deflate_trials_kernel(const TrialDe
                                                              uint32_t *queue, TrialOpts opts, uint32_t *symbuf_all,
                                                              uint8_t *insmap_all, uint64_t insmap_stride) {
     extern __shared__ __align__(16) uint8_t smem[];
-    const uint32_t lane = lane_id(), warp = threadIdx.x >> 5, wpc = blockDim.x >> 5;
-    const uint32_t slot = blockIdx.x * wpc + warp;
+    const uint32_t lane = lane_id(), slot = blockIdx.x;
     Trial t;
-    t.sm = smem + warp * WARP_SMEM;
+    t.sm = smem;
     t.symbuf = symbuf_all + (size_t)slot * 32768u;
     t.insmap = (uint32_t *)(insmap_all + (size_t)slot * insmap_stride);
     for (;;) {
@@ -1348,26 +1346,14 @@ cudaError_t launch_resolve_rows(const ResTask *tasks, uint32_t ntasks, uint32_t 
     return cudaGetLastError();
 }
 
-size_t deflate_warp_smem() { return WARP_SMEM; }
-
+// one warp per CTA: a warp that finds the queue empty gives its registers and shared memory back at once, so the tail of a launch
+// (a few long trials) leaves room for the kernels launched next to it
 cudaError_t launch_deflate_trials(const TrialDesc *descs, TrialResult *results, uint32_t ntrials, uint32_t *queue, const TrialOpts &opts,
-                                  uint32_t *symbuf_all, uint8_t *insmap_all, uint64_t insmap_stride, int ctas, int warps_per_cta,
-                                  bool dense, cudaStream_t stream) {
-    size_t smem = (size_t)warps_per_cta * WARP_SMEM;
-    // 8 warps x WARP_SMEM exceeds the 48 KB default; the attribute belongs to the (function, device) pair, and contexts of several
-    // devices launch from their own host threads (uncomp --gpus N)
-    static std::atomic<uint64_t> attr_set{0};
-    int dev = 0; cudaGetDevice(&dev);
-    const uint64_t bit = 1ull << (dev & 63);
-    if (!(attr_set.load(std::memory_order_acquire) & bit)) {
-        cudaFuncSetAttribute(deflate_trials_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 8 * WARP_SMEM);
-        cudaFuncSetAttribute(deflate_trials_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 8 * WARP_SMEM);
-        attr_set.fetch_or(bit, std::memory_order_release);
-    }
+                                  uint32_t *symbuf_all, uint8_t *insmap_all, uint64_t insmap_stride, int ctas, bool dense, cudaStream_t stream) {
     // dense launches (more trials than 16 warps/SM can hold) use the 80-register build: more resident warps hide the
     // latency of the serial parse better than the extra registers do
-    if (dense) deflate_trials_kernel<3><<<ctas, warps_per_cta * 32, smem, stream>>>(descs, results, ntrials, queue, opts, symbuf_all, insmap_all, insmap_stride);
-    else deflate_trials_kernel<2><<<ctas, warps_per_cta * 32, smem, stream>>>(descs, results, ntrials, queue, opts, symbuf_all, insmap_all, insmap_stride);
+    if (dense) deflate_trials_kernel<3><<<ctas, 32, WARP_SMEM, stream>>>(descs, results, ntrials, queue, opts, symbuf_all, insmap_all, insmap_stride);
+    else deflate_trials_kernel<2><<<ctas, 32, WARP_SMEM, stream>>>(descs, results, ntrials, queue, opts, symbuf_all, insmap_all, insmap_stride);
     return cudaGetLastError();
 }
 

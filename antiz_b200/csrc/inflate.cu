@@ -37,8 +37,6 @@ namespace atz {
 #define I_CTAB 3816   /* u16[128] primary table of the code-length code */
 #define I_STAGE 4080  /* u8[STAGE_BYTES] output bytes of one token batch, then u8[STAGE_BYTES] their token-map codes (16 B aligned) */
 #define I_WARP (4080 + 2 * 2048)
-#define I_MAIL I_WARP /* pair mode: the decoder warp's mailbox to its writer warp (struct Mail) */
-#define I_PAIR (I_WARP + 304)
 // CTA-wide fixed tables
 #define F_LTAB 0
 #define F_DTAB 2048
@@ -56,16 +54,6 @@ struct Code { const uint16_t *tab; const uint16_t *sym; const uint16_t *cnt; uin
 __device__ __noinline__ void write_probe(InflateResult *r, uint32_t adler, uint64_t avail, uint64_t nout, uint64_t in_at_cap) {
     if (lane_id() == 0) { r->status = INF_NEED_INPUT; r->adler = adler; r->total_in = avail; r->total_out = nout; r->in_at_outcap = in_at_cap; }
 }
-
-// Pair mode (stage-2 launches, where every phase is as long as the longest stream): two warps per stream.  The decoder warp
-// runs the whole inflate state machine; the bytes of a token batch are produced by its partner, which it feeds through a
-// two-slot mailbox in shared memory, so the Huffman decode of batch i+1 overlaps the copies of batch i.  Whenever the decoder
-// needs the output itself (tokens outside batches, stored blocks, adler32, the result) it waits for the mailbox to drain.
-struct Mail {
-    volatile uint32_t prod, cons; uint32_t pad[2];
-    struct Slot { uint32_t cmd, ntok, nout_lo, nout_hi; uint32_t tok[32]; } slot[2];   // cmd: 0 = batch, 1 = new job (tok[0..3] = out, tmap), 2 = exit
-};
-#define TOK_LIT 0x02000000u   /* tok = len | dist << 9, or 1 | literal << 9 | TOK_LIT */
 
 struct Writer {
     uint8_t *out, *tmap, *sm;
@@ -153,29 +141,6 @@ struct Writer {
             __syncwarp();
         }
     }
-    // the partner warp of pair mode: serves the mailbox until told to exit
-    __device__ void serve(Mail *mail) {
-        const uint32_t lane = lane_id();
-        uint32_t cons = 0;
-        for (;;) {
-            if (lane == 0) while (mail->prod == cons) __nanosleep(40);
-            __syncwarp();
-            volatile Mail::Slot *sl = &mail->slot[cons & 1];
-            const uint32_t cmd = sl->cmd;
-            if (cmd == 0) {
-                const uint32_t ntok = sl->ntok, tok = sl->tok[lane]; const uint64_t nout = ((uint64_t)sl->nout_hi << 32) | sl->nout_lo;
-                const bool lit = (tok & TOK_LIT) != 0;
-                produce(tok & 0x1ffu, lit ? 0u : (tok >> 9) & 0xffffu, lit ? (tok >> 9) & 0xffu : 0u, ntok, nout);
-            } else if (cmd == 1) {
-                out = (uint8_t *)(((uint64_t)sl->tok[1] << 32) | sl->tok[0]); tmap = (uint8_t *)(((uint64_t)sl->tok[3] << 32) | sl->tok[2]);
-            }
-            __threadfence_block();
-            __syncwarp();
-            cons++;
-            if (lane == 0) mail->cons = cons;
-            if (cmd == 2) break;
-        }
-    }
 };
 
 struct Inflater {
@@ -189,26 +154,6 @@ struct Inflater {
     uint64_t first_cap, in_at_cap; bool cap_seen;
     uint32_t a, b;
     uint8_t *sm;
-    Mail *mail; uint32_t prod;   // pair mode: mailbox to the writer warp (nullptr: this warp produces its own output)
-
-    __device__ __forceinline__ void mail_post(uint32_t cmd, uint32_t ntok, uint64_t at, uint32_t tok) {
-        const uint32_t lane = lane_id();
-        if (lane == 0) while (prod - mail->cons >= 2) __nanosleep(40);
-        __syncwarp();
-        Mail::Slot *sl = &mail->slot[prod & 1];
-        sl->tok[lane] = tok;
-        if (lane == 0) { sl->cmd = cmd; sl->ntok = ntok; sl->nout_lo = (uint32_t)at; sl->nout_hi = (uint32_t)(at >> 32); }
-        __threadfence_block();
-        __syncwarp();
-        prod++;
-        if (lane == 0) mail->prod = prod;
-    }
-    // everything handed to the writer warp is in memory
-    __device__ __forceinline__ void drain() {
-        if (!mail) return;
-        if (lane_id() == 0) while (mail->cons != prod) __nanosleep(40);
-        __syncwarp();
-    }
 
     __device__ __forceinline__ uint32_t in_byte(uint64_t v) {
         uint64_t fp = off + v;
@@ -338,7 +283,6 @@ struct Inflater {
 
     __device__ __forceinline__ uint8_t *optr(uint64_t pos) { return out + pos; }
     __device__ __forceinline__ void put_literal(uint32_t v) {
-        drain();
         if (lane_id() == 0) { *optr(nout) = (uint8_t)v; if (tmap) tmap[nout] = 1; }
         nout++;
     }
@@ -346,7 +290,6 @@ struct Inflater {
     __device__ __forceinline__ void put_match(uint32_t len, uint32_t dist) {
         const uint32_t lane = lane_id();
         const uint32_t tin = TM_INNER + (len <= 4 ? 3u : len == 5 ? 2u : len == 6 ? 1u : 0u), tst = len < TM_LONG ? len : TM_LONG;
-        drain();
         __syncwarp();
         for (uint32_t i = lane; i < len; i += 32) {
             const uint32_t r = i < dist ? i : i % dist;
@@ -360,7 +303,6 @@ struct Inflater {
     // slice, the slices are combined in order (b_total += b_k + len_k * a_running).
     __device__ void adler_of_output() {
         const uint32_t lane = lane_id();
-        drain();
         const uint64_t per = (nout + 31) / 32;
         uint64_t beg = (uint64_t)lane * per, end = beg + per; if (beg > nout) beg = nout; if (end > nout) end = nout;
         uint32_t sa = 0, sb = 0; const uint32_t slen = (uint32_t)((end - beg) % 65521u);
@@ -419,8 +361,7 @@ struct Inflater {
 #undef BATCH_REFILL
         const uint32_t ntok = k;
         if (ntok == 0) return ev;
-        if (mail) mail_post(0, ntok, nout, lane < ntok ? (my_dist ? (my_len | (my_dist << 9)) : (1u | (my_lit << 9) | TOK_LIT)) : 0u);
-        else { Writer w{out, tmap, sm}; w.produce(my_len, my_dist, my_lit, ntok, nout); }
+        Writer{out, tmap, sm}.produce(my_len, my_dist, my_lit, ntok, nout);
         nout = vout;
         return ev;
     }
@@ -456,7 +397,6 @@ struct Inflater {
                     uint64_t can = avail - bp; uint32_t take = left < can ? left : (uint32_t)can;
                     if (!cap_seen && nout + take > first_cap) { cap_seen = true; in_at_cap = bp + (first_cap - nout); }
                     if (nout + take > out_cap) { status = INF_OUT_FULL; goto done; }
-                    drain();
                     __syncwarp();
                     for (uint32_t i = lane; i < take; i += 32) { *optr(nout + i) = (uint8_t)in_byte(bp + i); if (tmap) tmap[nout + i] = 0; }   // stored: no tokens known
                     __syncwarp();
@@ -547,7 +487,6 @@ struct Inflater {
     done:
 #undef NEED
 #undef FAILD
-        drain();
         if (lane == 0) {
             InflateResult *r = switched ? cont : res;
             r->status = status; r->adler = (b << 16) | a; r->total_in = bytes_used(); r->total_out = nout;
@@ -558,15 +497,12 @@ struct Inflater {
     }
 };
 
-template <bool PAIR>
 __global__ void __launch_bounds__(128) inflate_kernel(const uint8_t *file, const InflateJob *jobs, InflateResult *results, InflateResult *cont, uint32_t njobs,
                                                       uint32_t *queue, uint8_t *arena, uint64_t first_cap, uint64_t chunk) {
     extern __shared__ __align__(16) uint8_t smem_all[];
     const uint32_t lane = lane_id(), warp = threadIdx.x >> 5;
     Inflater inf;
-    inf.sm = smem_all + F_SIZE + (PAIR ? (warp >> 1) * I_PAIR : warp * I_WARP);
-    inf.mail = PAIR ? (Mail *)(inf.sm + I_MAIL) : nullptr; inf.prod = 0;
-    if (PAIR && (warp & 1) == 0 && lane == 0) { inf.mail->prod = 0; inf.mail->cons = 0; }
+    inf.sm = smem_all + F_SIZE + warp * I_WARP;
     // fixed Huffman tables once per CTA (Z/inffixed.h is what zlib uses; here they are rebuilt from the RFC lengths)
     {
         uint8_t *lens = inf.sm + I_LENS; uint32_t mx;
@@ -579,11 +515,6 @@ __global__ void __launch_bounds__(128) inflate_kernel(const uint8_t *file, const
             inf.build(lens, 32, (uint16_t *)(smem_all + F_DCNT), (uint16_t *)(smem_all + F_DSYM), (uint16_t *)(smem_all + F_DTAB), DPB, false, mx);
         }
         __syncthreads();
-    }
-    if (PAIR && (warp & 1)) {   // the writer warp of the pair
-        Writer w{nullptr, nullptr, inf.sm};
-        w.serve(inf.mail);
-        return;
     }
     for (;;) {
         uint32_t ji = 0;
@@ -600,26 +531,15 @@ __global__ void __launch_bounds__(128) inflate_kernel(const uint8_t *file, const
         inf.tmap = j.tmap_off != ~0ull ? arena + j.tmap_off : nullptr;
         inf.first_cap = first_cap ? first_cap : ~0ull; inf.in_at_cap = 0; inf.cap_seen = false;
         inf.a = 1; inf.b = 0;
-        if (PAIR) {
-            const uint64_t po = (uint64_t)inf.out, pt = (uint64_t)inf.tmap;
-            inf.mail_post(1, 0, 0, lane == 0 ? (uint32_t)po : lane == 1 ? (uint32_t)(po >> 32) : lane == 2 ? (uint32_t)pt : lane == 3 ? (uint32_t)(pt >> 32) : 0u);
-        }
         inf.run(&results[ji], &cont[ji]);
         __syncwarp();
     }
-    if (PAIR) inf.mail_post(2, 0, 0, 0u);
 }
 
-// pair = true: warps_per_cta must be even; every two warps serve one stream at a time (decoder + writer)
 cudaError_t launch_inflate(const uint8_t *file, const InflateJob *jobs, InflateResult *results, InflateResult *cont, uint32_t njobs, uint32_t *queue,
-                           uint8_t *arena, uint64_t first_cap, uint64_t chunk, int ctas, int warps_per_cta, bool pair, cudaStream_t s) {
-    if (pair) {
-        const size_t smem = F_SIZE + (size_t)(warps_per_cta / 2) * I_PAIR;
-        inflate_kernel<true><<<ctas, warps_per_cta * 32, smem, s>>>(file, jobs, results, cont, njobs, queue, arena, first_cap, chunk);
-    } else {
-        const size_t smem = F_SIZE + (size_t)warps_per_cta * I_WARP;
-        inflate_kernel<false><<<ctas, warps_per_cta * 32, smem, s>>>(file, jobs, results, cont, njobs, queue, arena, first_cap, chunk);
-    }
+                           uint8_t *arena, uint64_t first_cap, uint64_t chunk, int ctas, int warps_per_cta, cudaStream_t s) {
+    const size_t smem = F_SIZE + (size_t)warps_per_cta * I_WARP;
+    inflate_kernel<<<ctas, warps_per_cta * 32, smem, s>>>(file, jobs, results, cont, njobs, queue, arena, first_cap, chunk);
     return cudaGetLastError();
 }
 

@@ -300,9 +300,9 @@ def _records(data, opt, **env):
 
 def test_search_schedule_does_not_change_records():
     """the burst parse (speculation on the original's token boundaries), the
-    lane partition, phase B in the background, the queue order of a launch, rows at every position and the two-warp inflate are
-    scheduling choices: every per-stream record, including those of streams that are not recompressed, equals the one of the plain
-    serial single-lane foreground search (exact-records mode: no early cut)"""
+    lane partition, phase B in the background and rows at every position are scheduling choices: every per-stream record,
+    including those of streams that are not recompressed, equals the one of the plain serial single-lane foreground search
+    (exact-records mode: no early cut)"""
     exact = az.ATZ_F_EXACT_RECORDS
     cases = [
         (corpus.fast_mix(36, 62) + corpus.c2(24, 63, 1 << 10, 96 << 10), az.Options(flags=exact)),
@@ -311,10 +311,10 @@ def test_search_schedule_does_not_change_records():
         (corpus.mixed(900000, 66), az.Options(bruteforceWindow=True)),     # default mode: the early cut only ever hides records that are not written
     ]
     for data, opt in cases:
-        base = _records(data, opt, ATZ_BURST=0, ATZ_LANES=1, ATZ_BG_B=0, ATZ_TRIAL_ORDER=0)
+        base = _records(data, opt, ATZ_BURST=0, ATZ_LANES=1, ATZ_BG_B=0)
         assert any(r[7] for r in base[0]) or not base[0]
-        for env in (dict(ATZ_BURST=1, ATZ_LANES=1, ATZ_BG_B=0), dict(ATZ_BURST=1, ATZ_LANES=3, ATZ_BG_B=1, ATZ_TRIAL_ORDER=1),
-                    dict(ATZ_BURST=0, ATZ_LANES=1, ATZ_BG_B=1, ATZ_ALL_ROWS=1), dict(ATZ_BURST=1, ATZ_LANES=2, ATZ_BG_B=1, ATZ_INFLATE_PAIR=1 ),
+        for env in (dict(ATZ_BURST=1, ATZ_LANES=1, ATZ_BG_B=0), dict(ATZ_BURST=1, ATZ_LANES=3, ATZ_BG_B=1),
+                    dict(ATZ_BURST=0, ATZ_LANES=1, ATZ_BG_B=1, ATZ_ALL_ROWS=1), dict(ATZ_BURST=1, ATZ_LANES=2, ATZ_BG_B=1),
                     dict(ATZ_BURST=1, ATZ_LANES=1, ATZ_WAVE_GROWTH=16, ATZ_BATCH_SETS=1)):
             got = _records(data, opt, **env)
             if opt.flags & exact:

@@ -14,6 +14,7 @@ ATZ_OK, ATZ_E_NO_DEVICE, ATZ_E_CUDA, ATZ_E_ARG, ATZ_E_TOO_LARGE = 0, -1, -2, -3,
 ATZ_E_NOMEM, ATZ_E_DATA, ATZ_E_SMALL, ATZ_E_TRUNCATED, ATZ_E_STATE = -5, -6, -7, -8, -10
 ATZ_F_EXACT_RECORDS = 1
 ATZ_F_STRATEGIES = 2     # extension: also try Z_FILTERED / Z_FIXED / Z_RLE / Z_HUFFMAN_ONLY (include/antiz_b200.h)
+ATZ_SCAN_SMALL_WINDOWS = 1   # extension: the scan also accepts CINFO 0 and 1 headers (offsetType 24..31, searched at window 9)
 
 
 def clevel(level, strategy=0):
@@ -73,6 +74,7 @@ def lib():
         L.atz_ctx_create.argtypes = [C.c_int, C.POINTER(C.c_void_p)]
         L.atz_ctx_destroy.argtypes = [C.c_void_p]
         L.atz_ctx_set_budget.argtypes = [C.c_void_p, C.c_uint64]
+        L.atz_ctx_set_scan_flags.argtypes = [C.c_void_p, C.c_uint32]
         L.atz_load.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64]
         L.atz_load_device.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64]
         L.atz_scan.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
@@ -102,7 +104,7 @@ def lib():
     return _lib
 
 
-EXPORTS = ["atz_version", "atz_last_error", "atz_ctx_create", "atz_ctx_destroy", "atz_ctx_set_budget", "atz_load", "atz_load_device",
+EXPORTS = ["atz_version", "atz_last_error", "atz_ctx_create", "atz_ctx_destroy", "atz_ctx_set_budget", "atz_ctx_set_scan_flags", "atz_load", "atz_load_device",
            "atz_scan", "atz_attach", "atz_scan_shard", "atz_probe_export", "atz_probe_import", "atz_scan_finish", "atz_host_partition", "atz_search", "atz_search_shard", "atz_get_streams", "atz_get_owners", "atz_get_diffs", "atz_get_inflated", "atz_get_inflated_recomp", "atz_get_inflated_list", "atz_get_stats", "atz_timer_start", "atz_timer_stop",
            "atz_inflate_stream", "atz_deflate_stream", "atz_deflate_batch", "atz_trial"]
 
@@ -144,6 +146,10 @@ class Context:
 
     def set_budget(self, nbytes):
         self._ck(lib().atz_ctx_set_budget(self._h, nbytes))
+
+    def set_scan_flags(self, flags):
+        """the header set of the scan (ATZ_SCAN_* bits); only before the first load() / load_device() / attach()"""
+        self._ck(lib().atz_ctx_set_scan_flags(self._h, flags))
 
     def load(self, data):
         addr, n, keep = _buf(data)

@@ -32,7 +32,7 @@ cudaError_t launch_resolve_rows(const ResTask *, uint32_t, uint32_t, cudaStream_
 cudaError_t launch_gather(const CopyJob *, uint32_t, cudaStream_t);
 cudaError_t launch_diff(const DiffJob *, uint32_t, cudaStream_t);
 uint32_t scan_tiles_for(uint64_t lo, uint64_t hi);
-cudaError_t launch_scan_count(const uint8_t *, uint64_t, uint64_t, uint64_t, uint32_t *, uint16_t *, uint32_t *, cudaStream_t);
+cudaError_t launch_scan_count(const uint8_t *, uint64_t, uint64_t, uint64_t, uint32_t, uint32_t *, uint16_t *, uint32_t *, cudaStream_t);
 cudaError_t launch_scan_write(const uint8_t *, uint64_t, uint64_t, const uint16_t *, const uint32_t *, uint32_t *, uint8_t *, uint32_t, cudaStream_t);
 cudaError_t launch_inflate(const uint8_t *, const InflateJob *, InflateResult *, InflateResult *, uint32_t, uint32_t *, uint8_t *, uint64_t, uint64_t, int, int, cudaStream_t);
 } // namespace atz
@@ -112,6 +112,7 @@ struct atz_ctx {
     int sms = 148; size_t budget = 0;
     std::string err;
     int state = 0;   // 0 nothing, 1 loaded, 2 scanned, 3 searched
+    uint32_t scan_flags = 0; bool scan_flags_fixed = false;   // ATZ_SCAN_*: the header set of the scan (atz_ctx_set_scan_flags, fixed by the first load)
     HostDbg dbg;
     // input: the file image.  d_file is the device address of file offset 0; bytes [r0, r1) are mapped there (everything after atz_load /
     // atz_load_device; after atz_attach only what this shard's scan and its owned streams need, uploaded from h_file on demand)
@@ -162,12 +163,17 @@ struct Phase {   // CUDA-event timing of a phase on the context stream / on a la
 
 int trial_slots(atz_ctx *ctx) { return ctx->sms * 24; }   // 3 CTAs x 8 warps per SM (80-register build); sparse launches use 2 x 8 at ~116 registers
 
+// windowBits of a header type: the header's own for 0..23 (the reference's), 9 for CINFO 0 and 1 (ATZ_SCAN_SMALL_WINDOWS: zlib turns
+// windowBits 8 into 9, and a CINFO 0 header is written over a window-9 stream)
+inline int type_window(int offsetType) { return offsetType >= 24 ? 9 : 10 + offsetType / 4; }
+#define ATZ_NTYPES 32
+
 // ---- candidate order of the reference (main.cpp:487-602, 732-756) ----
 void push_range(std::vector<Params> &v, int cmin, int cmax, int wmin, int wmax, int mmin, int mmax) {
     for (int w = wmax; w >= wmin; w--) for (int m = mmax; m >= mmin; m--) for (int c = cmax; c >= cmin; c--) v.push_back({(uint8_t)c, (uint8_t)w, (uint8_t)m});
 }
 void class_sequence(int offsetType, std::vector<Params> &v) {
-    int w = 10 + offsetType / 4;
+    int w = type_window(offsetType);
     switch (offsetType % 4) {
     case 0: v.push_back({0, (uint8_t)w, 8}); v.push_back({1, (uint8_t)w, 8}); v.push_back({1, (uint8_t)w, 9});
             push_range(v, 1, 1, w, w, 1, 7); push_range(v, 2, 9, w, w, 1, 9); break;
@@ -179,8 +185,9 @@ void class_sequence(int offsetType, std::vector<Params> &v) {
              push_range(v, 1, 6, w, w, 1, 9); break;
     }
 }
+// (window 9, types 24..31: the whole grid 15..10, window 9 is not in it)
 void brute_sequence(int offsetType, std::vector<Params> &v) {
-    int w = 10 + offsetType / 4;
+    int w = type_window(offsetType);
     if (w == 10) push_range(v, 1, 9, 11, 15, 1, 9);
     else if (w == 15) push_range(v, 1, 9, 10, 14, 1, 9);
     else { push_range(v, 1, 9, 10, w - 1, 1, 9); push_range(v, 1, 9, w + 1, 15, 1, 9); }
@@ -191,7 +198,7 @@ void brute_sequence(int offsetType, std::vector<Params> &v) {
 // Z_FILTERED (1) only where it differs from the default (deflate_slow levels), Z_FIXED (4) everywhere, Z_RLE (3) and
 // Z_HUFFMAN_ONLY (2) once per memLevel (their output does not depend on the level)
 void strategy_sequence(int offsetType, std::vector<Params> &v) {
-    const int w = 10 + offsetType / 4;
+    const int w = type_window(offsetType);
     for (int m = 9; m >= 1; m--) for (int c = 9; c >= 4; c--) v.push_back({(uint8_t)c, (uint8_t)w, (uint8_t)m, 1});
     for (int m = 9; m >= 1; m--) for (int c = 9; c >= 1; c--) v.push_back({(uint8_t)c, (uint8_t)w, (uint8_t)m, 4});
     for (int m = 9; m >= 1; m--) v.push_back({1, (uint8_t)w, (uint8_t)m, 3});
@@ -201,12 +208,6 @@ void strategy_sequence(int offsetType, std::vector<Params> &v) {
 // ---- host-side scan logic (pure functions; also exported for CPU tests as atz_host_*) ----
 struct ProbeRec { int32_t status; uint64_t total_in, total_out, in_at_outcap; };
 struct Acc { uint64_t off, tin, tout; uint32_t cand; bool via_cont; };
-
-// parseOffsetType (main.cpp:168-203) in closed form (the same as csrc/scan.cu): type 0..23, or -1
-inline int header_type(uint32_t b0, uint32_t b1) {
-    if ((b0 & 0x8f) != 0x08 || b0 < 0x28 || (b1 & 0x20) || ((b0 << 8) | b1) % 31) return -1;
-    return 4 * ((int)(b0 >> 4) - 2) + (int)(b1 >> 6);
-}
 
 // chunk list of searchInfile (main.cpp:405-415): first read S bytes, then S-1 new bytes behind the kept last byte;
 // the loop runs until a read comes up short, so a file of exactly S + k(S-1) bytes gets a trailing 1-byte chunk.
@@ -764,9 +765,15 @@ void atz_ctx_destroy(atz_ctx *ctx) {
     delete ctx;
 }
 int atz_ctx_set_budget(atz_ctx *ctx, uint64_t bytes) { if (!ctx || bytes < (1u << 20)) return ATZ_E_ARG; ctx->budget = bytes; return ATZ_OK; }
+int atz_ctx_set_scan_flags(atz_ctx *ctx, uint32_t flags) {
+    if (!ctx || (flags & ~(uint32_t)ATZ_SCAN_SMALL_WINDOWS)) return ATZ_E_ARG;
+    if (ctx->scan_flags_fixed) { ctx->set_err("atz_ctx_set_scan_flags: the context has already loaded a file"); return ATZ_E_STATE; }
+    ctx->scan_flags = flags;
+    return ATZ_OK;
+}
 
 static void reset_scan(atz_ctx *ctx) {
-    ctx->st = atz_stats{}; ctx->streams.clear(); ctx->state = 0; ctx->sc = ScanState{};
+    ctx->st = atz_stats{}; ctx->streams.clear(); ctx->state = 0; ctx->sc = ScanState{}; ctx->scan_flags_fixed = true;
 }
 static int load_common(atz_ctx *ctx, const void *src, uint64_t n, cudaMemcpyKind kind) {
     if (!ctx || !src || n == 0) return ATZ_E_ARG;
@@ -870,7 +877,7 @@ int atz_scan_shard(atz_ctx *ctx, uint64_t chunksize, uint32_t shard, uint32_t ns
         uint32_t ncand = 0;
         {
             Phase ph(ctx, &ctx->st.ms_scan);
-            CK(launch_scan_count(ctx->d_file, f0, f1, N, ctx->tile_counts.as<uint32_t>(), ctx->scan_masks.as<uint16_t>(), ctx->total.as<uint32_t>(), ctx->stream));
+            CK(launch_scan_count(ctx->d_file, f0, f1, N, ctx->scan_flags, ctx->tile_counts.as<uint32_t>(), ctx->scan_masks.as<uint16_t>(), ctx->total.as<uint32_t>(), ctx->stream));
             CK(cudaMemcpyAsync(&ncand, ctx->total.p, 4, cudaMemcpyDeviceToHost, ctx->stream));
             CK(cudaStreamSynchronize(ctx->stream));
             ctx->st.kernel_launches += 2;
@@ -910,7 +917,7 @@ int atz_scan_shard(atz_ctx *ctx, uint64_t chunksize, uint32_t shard, uint32_t ns
                     const uint64_t p = cstart[k0 + i];
                     while (ci < cand.size() && cand[ci] < p) { c2.push_back(cand[ci]); t2.push_back(ctype[ci]); s2.push_back(0); ci++; }
                     if (ci < cand.size() && cand[ci] == p) ci++;                       // what K1 saw there were the file's own bytes
-                    const int ty = p + 1 < N ? header_type(edge[4 * i], edge[4 * i + 2]) : -1;
+                    const int ty = p + 1 < N ? zlib_header_type(edge[4 * i], edge[4 * i + 2], ctx->scan_flags) : -1;
                     if (ty >= 0) { c2.push_back((uint32_t)p); t2.push_back((uint8_t)ty); s2.push_back(1); }
                 }
                 while (ci < cand.size()) { c2.push_back(cand[ci]); t2.push_back(ctype[ci]); s2.push_back(0); ci++; }
@@ -1039,22 +1046,29 @@ int atz_scan_shard(atz_ctx *ctx, uint64_t chunksize, uint32_t shard, uint32_t ns
     return ATZ_OK;
 }
 
+// the export: the exporting context's scan flags (8 bytes; the records were found with that header set), then the records
 int atz_probe_export(atz_ctx *ctx, void *buf, uint64_t cap, uint64_t *nbytes) {
     if (!ctx || !nbytes) return ATZ_E_ARG;
     if (!ctx->sc.probed) return ATZ_E_STATE;
     const std::vector<ProbeX> &v = ctx->sc.px[ctx->sc.shard];
-    *nbytes = v.size() * sizeof(ProbeX);
+    const uint64_t flags = ctx->scan_flags;
+    *nbytes = sizeof flags + v.size() * sizeof(ProbeX);
     if (!buf || cap < *nbytes) return ATZ_E_SMALL;
-    if (*nbytes) memcpy(buf, v.data(), *nbytes);
+    memcpy(buf, &flags, sizeof flags);
+    if (!v.empty()) memcpy((uint8_t *)buf + sizeof flags, v.data(), v.size() * sizeof(ProbeX));
     return ATZ_OK;
 }
 int atz_probe_import(atz_ctx *ctx, uint32_t shard, const void *buf, uint64_t nbytes) {
-    if (!ctx || (!buf && nbytes) || nbytes % sizeof(ProbeX)) return ATZ_E_ARG;
+    uint64_t flags = 0;
+    if (!ctx || !buf || nbytes < sizeof flags || (nbytes - sizeof flags) % sizeof(ProbeX)) return ATZ_E_ARG;
     if (!ctx->sc.probed) return ATZ_E_STATE;
     if (shard >= ctx->sc.nshards || shard == ctx->sc.shard) return ATZ_E_ARG;
+    memcpy(&flags, buf, sizeof flags);
+    if (flags != ctx->scan_flags) { ctx->set_err("atz_probe_import: the shard scanned with other scan flags (atz_ctx_set_scan_flags)"); return ATZ_E_STATE; }
+    nbytes -= sizeof flags;
     std::vector<ProbeX> &v = ctx->sc.px[shard];
     v.resize(nbytes / sizeof(ProbeX));
-    if (nbytes) memcpy(v.data(), buf, nbytes);
+    if (nbytes) memcpy(v.data(), (const uint8_t *)buf + sizeof flags, nbytes);
     for (size_t i = 0; i < v.size(); i++) if (v[i].off >= ctx->n || (i && v[i].off <= v[i - 1].off)) return ATZ_E_ARG;
     ctx->sc.have[shard] = 1;
     return ATZ_OK;
@@ -1432,9 +1446,9 @@ int atz_search_shard(atz_ctx *ctx, const atz_options *opt, uint32_t shard, uint3
     ctx->dbg = HostDbg{}; for (int l = 0; l < ATZ_LANES; l++) ctx->lane[l].dbg = &ctx->dbg;
     ctx->dbg.lanes = getenv("ATZ_DEBUG_LANES") != nullptr; ctx->dbg.t0 = ctx->dbg.t = std::chrono::steady_clock::now(); host_mark(ctx->lane[0], -1);
     // the candidate sequences depend on the header type only: built once per type, shared by the streams
-    static std::vector<Params> seq_class[24], seq_brute[24], seq_strat[24];
+    static std::vector<Params> seq_class[ATZ_NTYPES], seq_brute[ATZ_NTYPES], seq_strat[ATZ_NTYPES];
     static std::once_flag seq_once;
-    std::call_once(seq_once, [] { for (int ty = 0; ty < 24; ty++) { class_sequence(ty, seq_class[ty]); brute_sequence(ty, seq_brute[ty]); strategy_sequence(ty, seq_strat[ty]); } });
+    std::call_once(seq_once, [] { for (int ty = 0; ty < ATZ_NTYPES; ty++) { class_sequence(ty, seq_class[ty]); brute_sequence(ty, seq_brute[ty]); strategy_sequence(ty, seq_strat[ty]); } });
     // which streams this call searches: after a sharded scan the ones this context owns (it holds no other plaintext); after a
     // plain atz_scan any partition can be asked for (every stream is resident) and is computed the same way (atz_host_partition)
     if (ctx->sc.nshards > 1 && (nshards != ctx->sc.nshards || shard != ctx->sc.shard)) { ctx->set_err("atz_search_shard: shard does not match the sharded scan"); return ATZ_E_ARG; }
@@ -1731,8 +1745,9 @@ int atz_trial(atz_ctx *ctx, const uint8_t *in, uint64_t n, const uint8_t *orig, 
 }
 
 // ---- host-logic test hooks: pure host code, usable without a CUDA device (tests/test_host_logic.py) ----
+int atz_host_header_type(uint32_t scan_flags, uint32_t b0, uint32_t b1) { return zlib_header_type(b0 & 0xff, b1 & 0xff, scan_flags); }
 int atz_host_candidate_sequence(int offsetType, int brute, uint8_t *clevel, uint8_t *window, uint8_t *memlevel, uint32_t cap) {
-    if (offsetType < 0 || offsetType > 23) return ATZ_E_ARG;
+    if (offsetType < 0 || offsetType >= ATZ_NTYPES) return ATZ_E_ARG;
     std::vector<Params> v;
     if (brute == 2) strategy_sequence(offsetType, v); else if (brute) brute_sequence(offsetType, v); else class_sequence(offsetType, v);
     for (size_t i = 0; i < v.size() && i < cap; i++) { clevel[i] = (uint8_t)(v[i].c | (v[i].s << 4)); window[i] = v[i].w; memlevel[i] = v[i].m; }

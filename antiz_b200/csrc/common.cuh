@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "../../include/antiz_b200.h"
 
 #define FULL 0xffffffffu
 #define ATZ_PAD 512u /* every device buffer that kernels read with unaligned word loads has >= this much zeroed slack */
@@ -80,6 +81,24 @@ struct InflateResult {
     int32_t status; uint32_t adler;
     uint64_t total_in, total_out, in_at_outcap;
 };
+
+// ---------------------------------------------------------------------------------------------
+// The zlib headers the scan accepts (K1 in scan.cu, the chunk-start fix-up in api.cu).  `scan_flags` is the context's
+// ATZ_SCAN_* set (include/antiz_b200.h).  The reference's 24 (ZBuffSearcher::parseOffsetType main.cpp:168-203): CM = 8,
+// CINFO 2..7, FDICT = 0, (CMF*256 + FLG) % 31 == 0.  ATZ_SCAN_SMALL_WINDOWS adds CINFO 0 and 1 (CMF 0x08, 0x18): 8 more pairs.
+// ---------------------------------------------------------------------------------------------
+__host__ __device__ __forceinline__ bool zlib_header_ok(uint32_t b0, uint32_t b1, uint32_t scan_flags) {
+    return (b0 & 0x8fu) == 0x08u && b0 >= ((scan_flags & ATZ_SCAN_SMALL_WINDOWS) ? 0x08u : 0x28u) && (b1 & 0x20u) == 0 && ((b0 << 8) | b1) % 31u == 0;
+}
+// offsetType of an accepted header: 4 * (CINFO - 2) + FLEVEL = 0..23 for the reference's set, 24 + 4 * CINFO + FLEVEL = 24..31 for
+// CINFO 0 and 1
+__host__ __device__ __forceinline__ int zlib_header_type_of(uint32_t b0, uint32_t b1) {
+    return b0 >= 0x28u ? 4 * ((int)(b0 >> 4) - 2) + (int)(b1 >> 6) : 24 + 4 * (int)(b0 >> 4) + (int)(b1 >> 6);
+}
+// the same, -1 if the header is not in the set
+__host__ __device__ __forceinline__ int zlib_header_type(uint32_t b0, uint32_t b1, uint32_t scan_flags) {
+    return zlib_header_ok(b0, b1, scan_flags) ? zlib_header_type_of(b0, b1) : -1;
+}
 
 // ---------------------------------------------------------------------------------------------
 // Device helpers

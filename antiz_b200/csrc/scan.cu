@@ -1,5 +1,6 @@
-// K1 - candidate scan: find every offset i with (file[i], file[i+1]) one of the 24 zlib headers AntiZ accepts
-// (ZBuffSearcher::parseOffsetType main.cpp:168-203: CM=8, CINFO 2..7, FDICT=0, (CMF*256+FLG) % 31 == 0).
+// K1 - candidate scan: find every offset i with (file[i], file[i+1]) one of the zlib headers of the context's scan set: the 24 AntiZ
+// accepts (ZBuffSearcher::parseOffsetType main.cpp:168-203: CM=8, CINFO 2..7, FDICT=0, (CMF*256+FLG) % 31 == 0), or those and the 8
+// of CINFO 0 and 1 (ATZ_SCAN_SMALL_WINDOWS; common.cuh zlib_header_ok).
 // HBM-bound by design: the file is read ONCE, with 16-byte vector loads; a word-at-a-time filter on the first header byte (low nibble 8,
 // top bit clear: three integer instructions per four bytes) leaves the per-position test to the few bytes that can start a header.
 // Pass 1 (scan_count_kernel) stores the 16-bit hit mask of every 16-byte group (N/8 bytes) and the hit count of every 64 KiB tile;
@@ -13,11 +14,7 @@ namespace atz {
 #define SCAN_THREADS 256
 #define SCAN_TILE (SCAN_THREADS * 16 * 16) /* 64 KiB per CTA */
 
-__device__ __forceinline__ bool is_magic(uint32_t b0, uint32_t b1) {
-    // closed form of the 24-way switch (checked exhaustively against it in tests/test_host_logic.py)
-    return (b0 & 0x8fu) == 0x08u && b0 >= 0x28u && (b1 & 0x20u) == 0 && ((b0 << 8) | b1) % 31u == 0;
-}
-// bytes of w whose low nibble is 8 and whose top bit is clear (0x08, 0x18, ... 0x78) -> 0x80 in that byte.  The zero-byte trick may
+// bytes of w whose low nibble is 8 and whose top bit is clear (0x08, 0x18, ... 0x78: every CMF of either set) -> 0x80 in that byte.  The zero-byte trick may
 // also flag the byte above a true hit (borrow); never misses one - the exact test follows.
 __device__ __forceinline__ uint32_t maybe_cmf(uint32_t w) {
     const uint32_t t = (w & 0x8f8f8f8fu) ^ 0x08080808u;
@@ -25,7 +22,7 @@ __device__ __forceinline__ uint32_t maybe_cmf(uint32_t w) {
 }
 // 16 consecutive positions starting at byte `pos` (a multiple of 16); bit k set <=> (pos+k, pos+k+1) is a header, pos+k is in
 // [lo, hi) (the part of the file this launch scans: a shard's chunk range, api.cu atz_scan_shard) and pos+k+1 < n
-__device__ __forceinline__ uint32_t magic_mask16(const uint8_t *file, uint64_t pos, uint64_t lo, uint64_t hi, uint64_t n) {
+__device__ __forceinline__ uint32_t magic_mask16(const uint8_t *file, uint64_t pos, uint64_t lo, uint64_t hi, uint64_t n, uint32_t flags) {
     if (pos >= hi || pos + 16 <= lo) return 0;
     const uint4 v = __ldg((const uint4 *)(file + pos));          // buffer is padded: always in bounds
     const uint32_t z0 = maybe_cmf(v.x), z1 = maybe_cmf(v.y), z2 = maybe_cmf(v.z), z3 = maybe_cmf(v.w);
@@ -41,20 +38,20 @@ __device__ __forceinline__ uint32_t magic_mask16(const uint8_t *file, uint64_t p
         const uint32_t k = (uint32_t)__ffs((int)q) - 1; q &= q - 1;
         const uint32_t b0 = (uint32_t)((k < 8 ? A >> (8 * k) : B >> (8 * (k - 8))) & 0xff);
         const uint32_t b1 = k == 15 ? nxt : (uint32_t)((k < 7 ? A >> (8 * (k + 1)) : B >> (8 * (k - 7))) & 0xff);
-        if (is_magic(b0, b1) && (inside || (pos + k + 1 < n && pos + k >= lo && pos + k < hi))) m |= 1u << k;
+        if (zlib_header_ok(b0, b1, flags) && (inside || (pos + k + 1 < n && pos + k >= lo && pos + k < hi))) m |= 1u << k;
     }
     return m;
 }
 
 // pass 1: masks[g] = hit mask of group g (g counts 16-byte groups from the tile base of this launch), tile_counts[t] = hits of tile t
-__global__ void __launch_bounds__(SCAN_THREADS) scan_count_kernel(const uint8_t *file, uint64_t lo, uint64_t hi, uint64_t n, uint32_t *tile_counts, uint16_t *masks) {
+__global__ void __launch_bounds__(SCAN_THREADS) scan_count_kernel(const uint8_t *file, uint64_t lo, uint64_t hi, uint64_t n, uint32_t flags, uint32_t *tile_counts, uint16_t *masks) {
     const uint64_t tile0 = (lo & ~(uint64_t)15) + (uint64_t)blockIdx.x * SCAN_TILE;
     uint16_t *tm = masks + (size_t)blockIdx.x * (SCAN_TILE / 16);
     uint32_t c = 0;
 #pragma unroll 4
     for (int it = 0; it < 16; it++) {
         const uint32_t g = (uint32_t)it * SCAN_THREADS + threadIdx.x;
-        const uint32_t m = magic_mask16(file, tile0 + (uint64_t)g * 16, lo, hi, n);
+        const uint32_t m = magic_mask16(file, tile0 + (uint64_t)g * 16, lo, hi, n, flags);
         tm[g] = (uint16_t)m; c += __popc(m);
     }
     c = __reduce_add_sync(FULL, c);
@@ -108,7 +105,7 @@ __global__ void __launch_bounds__(SCAN_THREADS) scan_write_kernel(const uint8_t 
         while (m) {
             const uint32_t k = __ffs((int)m) - 1; m &= m - 1;
             const uint64_t p = base + 32u * j + k;
-            if (o < cap) { cand[o] = (uint32_t)p; const uint32_t b0 = __ldg(file + p), b1 = __ldg(file + p + 1); ctype[o] = (uint8_t)(4 * ((b0 >> 4) - 2) + (b1 >> 6)); }
+            if (o < cap) { cand[o] = (uint32_t)p; const uint32_t b0 = __ldg(file + p), b1 = __ldg(file + p + 1); ctype[o] = (uint8_t)zlib_header_type_of(b0, b1); }
             o++;
         }
     }
@@ -117,9 +114,9 @@ __global__ void __launch_bounds__(SCAN_THREADS) scan_write_kernel(const uint8_t 
 // `file` is the address of file offset 0 (16 B aligned; only [lo & ~15, hi + 16) has to be mapped), positions lo <= i < hi are scanned
 uint32_t scan_tiles_for(uint64_t lo, uint64_t hi) { return hi > lo ? (uint32_t)((hi - (lo & ~(uint64_t)15) + SCAN_TILE - 1) / SCAN_TILE) : 0u; }
 // masks: scan_tiles_for(lo, hi) * 8 KiB (2 bytes per 16-byte group)
-cudaError_t launch_scan_count(const uint8_t *file, uint64_t lo, uint64_t hi, uint64_t n, uint32_t *tile_counts, uint16_t *masks, uint32_t *total, cudaStream_t s) {
+cudaError_t launch_scan_count(const uint8_t *file, uint64_t lo, uint64_t hi, uint64_t n, uint32_t flags, uint32_t *tile_counts, uint16_t *masks, uint32_t *total, cudaStream_t s) {
     uint32_t nt = scan_tiles_for(lo, hi);
-    if (nt) scan_count_kernel<<<nt, SCAN_THREADS, 0, s>>>(file, lo, hi, n, tile_counts, masks);
+    if (nt) scan_count_kernel<<<nt, SCAN_THREADS, 0, s>>>(file, lo, hi, n, flags, tile_counts, masks);
     scan_tiles_kernel<<<1, 1024, 0, s>>>(tile_counts, nt, total);
     return cudaGetLastError();
 }

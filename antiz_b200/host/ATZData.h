@@ -26,6 +26,7 @@ struct programOptions {
     bool exactRecords = false;           // ATZ_F_EXACT_RECORDS
     bool stats = false;                  // print per-phase timings
     bool strategies = false;             // ATZ_F_STRATEGIES: also try zlib's other strategies (changes the ATZ file vs the reference)
+    bool smallWindows = false;           // ATZ_SCAN_SMALL_WINDOWS: also accept CINFO 0 and 1 headers (the reference can still reconstruct)
 };
 
 struct zlibParamPack {

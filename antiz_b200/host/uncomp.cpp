@@ -101,6 +101,10 @@ class ATZcreator {
             mk(0);
             for (auto &t : th) t.join();
             for (int g = 0; g < ng; g++) if (crc[g] != ATZ_OK) { std::cout << "error: no usable CUDA device " << (options.device + g) << " (antiz_b200 has no CPU path)" << std::endl; std::exit(1); }
+            for (int g = 0; g < ng && options.smallWindows; g++) {   // before any load: every shard scans with the same header set
+                const int rc = atz_ctx_set_scan_flags(ctxs[g], ATZ_SCAN_SMALL_WINDOWS);
+                if (rc != ATZ_OK) { std::cout << atz_err(ctxs[g], rc) << std::endl; abort(); }
+            }
         }
         // one container over ng GPUs (SURVEY.md 8e): every context probes its own range of chunks, the host hands each shard's probe
         // records to the others, every context replays the accept logic and keeps the plaintext of the streams it owns
@@ -412,6 +416,7 @@ static const CliArg kExtArgs[] = {   // antiz_b200 only: listed after the refere
     {"", "exact-records", nullptr, false, "Disable the early cut of hopeless trials (the per-stream records of streams that are not recompressed stay exact; the ATZ file is the same either way)"},
     {"", "stats", nullptr, false, "Print per-phase timings to stderr"},
     {"", "strategies", nullptr, false, "For streams that no plain parameter set reproduces, also try zlib's other strategies (Z_FILTERED, Z_FIXED, Z_RLE, Z_HUFFMAN_ONLY). More streams are recompressed, but the ATZ file then differs from the reference's and only this program can reconstruct from it. Default: disabled"},
+    {"", "small-windows", nullptr, false, "Also look for zlib streams with 256- and 512-byte windows (header bytes 0x08 and 0x18). More streams are found and recompressed, so the ATZ file differs from the reference's, but the reference can still reconstruct from it. Default: disabled"},
 };
 static std::string cli_short_id(const CliArg &a) {
     std::string id = a.flag[0] ? std::string("-") + a.flag : std::string("--") + a.name;
@@ -520,6 +525,7 @@ static void parseCLI(int argc, char *argv[], std::string &infile_name, std::stri
         else if (n == "exact-records") options.exactRecords = true;
         else if (n == "stats") { options.stats = true; g_print_stats = true; }
         else if (n == "strategies") options.strategies = true;
+        else if (n == "small-windows") options.smallWindows = true;
         else if (n == "help") { usage(argv[0]); std::exit(0); }
         else if (n == "version") { std::cout << std::endl << argv[0] << "  version: " << antiz_ver << std::endl << std::endl; std::exit(0); }
     }

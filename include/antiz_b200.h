@@ -68,7 +68,8 @@ typedef struct {
     int64_t  firstDiffByte;   /* -1 = none */
     uint64_t ndiff;           /* diffByteOffsets.size() (only filled for recomp streams) */
     uint64_t diff_index;      /* first entry of this stream in the arrays returned by atz_get_diffs() */
-    int32_t  offsetType;      /* 0..23, parseOffsetType (main.cpp:168-203) */
+    int32_t  offsetType;      /* 0..23, parseOffsetType (main.cpp:168-203) = 4 * (CINFO - 2) + FLEVEL; with ATZ_SCAN_SMALL_WINDOWS
+                                 also 24..31 = 24 + 4 * CINFO + FLEVEL (CINFO 0 and 1) */
     uint8_t  clevel, window, memlevel; /* zlibParamPack; ctor defaults 9/15/9 (ATZData.h:50-52) */
     uint8_t  recomp;
 } atz_stream;
@@ -94,6 +95,16 @@ int  atz_ctx_create(int device, atz_ctx **out);
 void atz_ctx_destroy(atz_ctx *ctx);
 /* Upper bound of device memory the search may use for hash-chain structures (default: 60% of free memory). */
 int  atz_ctx_set_budget(atz_ctx *ctx, uint64_t bytes);
+/* Which zlib headers the scan accepts (ATZ_SCAN_* bits; default 0: the reference's 24).  Valid before the first atz_load /
+ * atz_load_device / atz_attach; ATZ_E_STATE after that, ATZ_E_ARG for an unknown bit.  Every shard of a sharded run must use the
+ * same set: atz_probe_import refuses the records of a shard that scanned with another one (ATZ_E_STATE). */
+int  atz_ctx_set_scan_flags(atz_ctx *ctx, uint32_t flags);
+/* Extension (SURVEY.md 8 f4; not in the reference, whose scan stops at CINFO 2): also accept the 8 headers with CINFO 0 and 1
+ * (CMF 0x08 and 0x18; windows of 256 and 512 bytes).  zlib writes CINFO 1 for deflateInit2(windowBits 8 or 9); CINFO 0 comes from
+ * encoders that rewrite the header of a small stream.  Both are searched at windowBits 9 (offsetType 24..31); a CINFO 0 stream that
+ * zlib reproduces differs from its winner in the two header bytes, which go into its diff list.  The ATZ layout does not change, so
+ * the reference's reconstructor still reads the file; it differs from the reference's own output because more streams are found. */
+#define ATZ_SCAN_SMALL_WINDOWS 1
 
 /* ---- precompress path ------------------------------------------------------------------------------ */
 
@@ -187,9 +198,13 @@ int atz_trial(atz_ctx *ctx, const uint8_t *in, uint64_t n, const uint8_t *orig, 
 
 /* ---- host-logic hooks (pure host code, no device needed): the reference's candidate order (main.cpp:487-602), chunk list
  * (main.cpp:405-415) and ZBuffSearcher accept logic (main.cpp:205-246), exported so CPU tests can pin them. ---- */
-/* brute: 0 = the header class's sequence (81 candidates), 1 = the --brute-window grid (405), 2 = the ATZ_F_STRATEGIES extension
- * (153; strategy in the high nibble of clevel).  Returns the length of the sequence. */
+/* brute: 0 = the header class's sequence (81 candidates), 1 = the --brute-window grid (405; 486 for offsetType 24..31, whose
+ * header window 9 is not part of the grid), 2 = the ATZ_F_STRATEGIES extension (153; strategy in the high nibble of clevel).
+ * offsetType 0..31 (24..31: ATZ_SCAN_SMALL_WINDOWS, searched at window 9).  Returns the length of the sequence. */
 int atz_host_candidate_sequence(int offsetType, int brute, uint8_t *clevel, uint8_t *window, uint8_t *memlevel, uint32_t cap);
+/* The header test of the scan (the same function K1 runs): offsetType of the zlib header (b0, b1) under the ATZ_SCAN_* set
+ * scan_flags, or -1 if the set does not accept it. */
+int atz_host_header_type(uint32_t scan_flags, uint32_t b0, uint32_t b1);
 /* owner[k] = shard that searches the k-th accepted stream of a scan, given the streams' inflated lengths.  probed_by == NULL: longest
  * first, each to the least loaded shard (what atz_search_shard uses after a plain atz_scan).  probed_by[k] = shard whose chunk range
  * stream k starts in (what atz_scan_finish uses): a stream stays where its plaintext already is unless that shard holds more than 2 %

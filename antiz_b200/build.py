@@ -9,7 +9,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libantiz_b200.so")
 UNCOMP = os.path.join(HERE, "uncomp")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-CU = ["api.cu", "scan.cu", "inflate.cu", "chains.cu", "deflate.cu"]
+CU = ["api.cu", "scan.cu", "inflate.cu", "chains.cu", "deflate.cu", "png.cu"]
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC,-O2,-Wall"]
 
 

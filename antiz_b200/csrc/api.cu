@@ -35,6 +35,8 @@ uint32_t scan_tiles_for(uint64_t lo, uint64_t hi);
 cudaError_t launch_scan_count(const uint8_t *, uint64_t, uint64_t, uint64_t, uint32_t, uint32_t *, uint16_t *, uint32_t *, cudaStream_t);
 cudaError_t launch_scan_write(const uint8_t *, uint64_t, uint64_t, const uint16_t *, const uint32_t *, uint32_t *, uint8_t *, uint32_t, cudaStream_t);
 cudaError_t launch_inflate(const uint8_t *, const InflateJob *, InflateResult *, InflateResult *, uint32_t, uint32_t *, uint8_t *, uint64_t, uint64_t, int, int, cudaStream_t);
+cudaError_t launch_idat_count(const uint8_t *, uint64_t, uint64_t, uint64_t, const uint32_t *, uint32_t, uint32_t *, cudaStream_t);
+cudaError_t launch_idat_write(const uint8_t *, uint64_t, uint64_t, uint64_t, const uint32_t *, const uint32_t *, const uint32_t *, const uint64_t *, uint32_t, uint32_t *, cudaStream_t);
 } // namespace atz
 using namespace atz;
 
@@ -64,6 +66,8 @@ struct StreamRec {
     uint32_t owner = 0;                 // shard that searches this stream (atz_host_partition)
     uint32_t adler = 0;
     std::vector<uint64_t> diff_off; std::vector<uint8_t> diff_val;
+    std::vector<uint32_t> pieces;       // ATZ_SCAN_PNG_IDAT: the piece lengths of a split stream (empty: an ordinary stream)
+    uint64_t span() const { return s.streamLength + (pieces.empty() ? 0 : 12 * (pieces.size() - 1)); }   // bytes from s.offset to the stream's end in the file
 };
 
 struct Params { uint8_t c, w, m, s = 0; };   // level, windowBits, memLevel, strategy (0 = Z_DEFAULT_STRATEGY: all the reference ever uses)
@@ -74,12 +78,20 @@ struct ProbeX {
     uint64_t off, avail, p_in, p_out, p_cap, c_in, c_out, c_cap;
     int32_t p_status, c_status; uint32_t p_adler, c_adler, local, type;
 };
+// A split stream (ATZ_SCAN_PNG_IDAT) as a shard found it: the header offset, C and U of the de-chunked stream, its adler32 and header
+// type, and its piece lengths (the run's IDAT data lengths up to the one that holds the stream's last byte, that one cut at C)
+struct SplitX {
+    uint64_t off, c, u; uint32_t adler, type; std::vector<uint32_t> pieces;
+    uint64_t span() const { return c + 12 * (pieces.size() - 1); }
+};
+struct SplitDev { const uint8_t *comp, *plain, *tmap; };   // where the probing shard keeps a split stream's bytes
 // State of a (possibly sharded) scan between atz_scan_shard and atz_scan_finish
 struct ScanState {
     bool probed = false, resident = false; uint64_t S = 0, SLOT = 0, QS = 0; uint32_t shard = 0, nshards = 1;
     std::vector<uint32_t> cand; std::vector<uint8_t> ctype; std::vector<InflateJob> jobs; std::vector<InflateResult> res, cres;
     std::vector<const uint8_t *> big_plain, big_tmap;
     std::vector<std::vector<ProbeX>> px; std::vector<uint8_t> have;
+    std::vector<std::vector<SplitX>> split; std::vector<SplitDev> split_dev;   // split streams of every shard; device bytes of this shard's
 };
 
 // coarse host-side stopwatch buckets (ATZ_DEBUG_HOST=1 prints them at the end of a search): per context, written by lane 0's thread only
@@ -119,7 +131,7 @@ struct atz_ctx {
     Buf file; const uint8_t *d_file = nullptr; uint64_t n = 0;
     const uint8_t *h_file = nullptr; uint64_t r0 = 0, r1 = 0; Buf comp_extra;
     // scan
-    Buf tile_counts, scan_masks, cand, ctype, jobs, jres, jres2, queue, total;
+    Buf tile_counts, scan_masks, cand, ctype, jobs, jres, jres2, queue, total, idat_counts, idat_runs, idat_lens;
     ScanState sc;
     // streams
     std::vector<StreamRec> streams; Buf plain, plain2; std::vector<void *> plain_extra;   // stage-1 slots, stage-2 regions, retry rounds
@@ -750,7 +762,7 @@ void atz_ctx_destroy(atz_ctx *ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
-    Buf *all[] = {&ctx->file, &ctx->tile_counts, &ctx->scan_masks, &ctx->cand, &ctx->ctype, &ctx->jobs, &ctx->jres, &ctx->queue, &ctx->jres2, &ctx->total, &ctx->plain, &ctx->plain2,
+    Buf *all[] = {&ctx->file, &ctx->tile_counts, &ctx->scan_masks, &ctx->cand, &ctx->ctype, &ctx->jobs, &ctx->jres, &ctx->queue, &ctx->jres2, &ctx->total, &ctx->idat_counts, &ctx->idat_runs, &ctx->idat_lens, &ctx->plain, &ctx->plain2,
                   &ctx->gather, &ctx->cjobs, &ctx->comp_extra, &ctx->op_in, &ctx->op_orig, &ctx->op_out, &ctx->op_misc};
     for (Buf *b : all) b->release();
     for (void *q : ctx->plain_extra) cudaFree(q);
@@ -766,7 +778,7 @@ void atz_ctx_destroy(atz_ctx *ctx) {
 }
 int atz_ctx_set_budget(atz_ctx *ctx, uint64_t bytes) { if (!ctx || bytes < (1u << 20)) return ATZ_E_ARG; ctx->budget = bytes; return ATZ_OK; }
 int atz_ctx_set_scan_flags(atz_ctx *ctx, uint32_t flags) {
-    if (!ctx || (flags & ~(uint32_t)ATZ_SCAN_SMALL_WINDOWS)) return ATZ_E_ARG;
+    if (!ctx || (flags & ~(uint32_t)(ATZ_SCAN_SMALL_WINDOWS | ATZ_SCAN_PNG_IDAT))) return ATZ_E_ARG;
     if (ctx->scan_flags_fixed) { ctx->set_err("atz_ctx_set_scan_flags: the context has already loaded a file"); return ATZ_E_STATE; }
     ctx->scan_flags = flags;
     return ATZ_OK;
@@ -841,6 +853,125 @@ static int run_inflate(atz_ctx *ctx, const uint8_t *base, std::vector<InflateJob
     return ATZ_OK;
 }
 
+// ---- ATZ_SCAN_PNG_IDAT ----
+struct RunBytes { uint64_t off; const uint32_t *len; size_t npieces; uint64_t total; };   // a run's pieces in the file: piece k+1 starts 12 bytes after piece k
+// The pieces of every run put together in one new device buffer (freed with plain_extra at the next scan), each run at at[i] with ATZ_PAD
+// zeroed bytes behind it: one gather launch over the file image for the runs inside the mapped range, host copies from the attached file
+// for the others.
+static int dechunk(atz_ctx *ctx, const std::vector<RunBytes> &runs, uint8_t *&base, std::vector<uint64_t> &at) {
+    at.resize(runs.size()); uint64_t tot = 0;
+    for (size_t i = 0; i < runs.size(); i++) { at[i] = tot; tot = align_up(tot + runs[i].total + ATZ_PAD, 256); }
+    void *q = nullptr; CK(cudaMalloc(&q, tot + ATZ_PAD)); ctx->plain_extra.push_back(q); base = (uint8_t *)q;
+    CK(cudaMemsetAsync(q, 0, tot + ATZ_PAD, ctx->stream));
+    std::vector<CopyJob> cj; std::vector<uint8_t> stage;
+    for (size_t i = 0; i < runs.size(); i++) {
+        const RunBytes &r = runs[i];
+        const bool mapped = ctx->d_file && r.off >= ctx->r0 && r.off + r.total + 12 * (r.npieces - 1) <= ctx->r1;
+        if (!mapped && !ctx->h_file) { ctx->set_err("IDAT run outside the resident file range"); return ATZ_E_STATE; }
+        if (!mapped) stage.resize(r.total);
+        uint64_t src = r.off, dst = 0;
+        for (size_t k = 0; k < r.npieces; k++) {
+            if (mapped) cj.push_back(CopyJob{ctx->d_file + src, base + at[i] + dst, r.len[k]});
+            else memcpy(stage.data() + dst, ctx->h_file + src, r.len[k]);
+            dst += r.len[k]; src += r.len[k] + 12;
+        }
+        if (!mapped && r.total) { CK(cudaMemcpyAsync(base + at[i], stage.data(), r.total, cudaMemcpyHostToDevice, ctx->stream)); CK(cudaStreamSynchronize(ctx->stream)); }
+    }
+    if (!cj.empty()) {
+        CK(ctx->cjobs.ensure(cj.size() * sizeof(CopyJob)));
+        CK(cudaMemcpyAsync(ctx->cjobs.p, cj.data(), cj.size() * sizeof(CopyJob), cudaMemcpyHostToDevice, ctx->stream));
+        CK(launch_gather(ctx->cjobs.as<CopyJob>(), (uint32_t)cj.size(), ctx->stream)); ctx->st.kernel_launches++;
+        CK(cudaStreamSynchronize(ctx->stream));
+    }
+    return ATZ_OK;
+}
+
+// The split streams of this shard: the K1 candidates (cand, type: K1's own list) that start an IDAT run (png.cu), each inflated by K2
+// over its run's data put together; a stream that ends there beyond its first piece and is longer than 16 bytes is recorded (SplitX)
+// with its plaintext and token map left resident, like a probed ordinary stream's.
+static int probe_idat_runs(atz_ctx *ctx, const std::vector<uint32_t> &cand, const std::vector<uint8_t> &type) {
+    ScanState &sc = ctx->sc; const uint64_t N = ctx->n;
+    const uint32_t nc = (uint32_t)cand.size();
+    std::vector<uint32_t> which, cnt; std::vector<uint64_t> at; std::vector<uint32_t> lens;   // run i: candidate which[i], cnt[i] lengths at lens[at[i]]
+    if (nc) {
+        std::vector<uint32_t> counts(nc);
+        Phase ph(ctx, &ctx->st.ms_scan);
+        CK(ctx->idat_counts.ensure((size_t)nc * 4));
+        CK(launch_idat_count(ctx->d_file, N, ctx->r0, ctx->r1, ctx->cand.as<uint32_t>(), nc, ctx->idat_counts.as<uint32_t>(), ctx->stream)); ctx->st.kernel_launches++;
+        CK(cudaMemcpyAsync(counts.data(), ctx->idat_counts.p, (size_t)nc * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        std::vector<uint32_t> dw; std::vector<uint64_t> dat; uint64_t tot = 0;
+        for (uint32_t k = 0; k < nc; k++) if (counts[k] && counts[k] != IDAT_FAR) { dw.push_back(k); dat.push_back(tot); tot += counts[k]; }
+        lens.resize(tot);
+        if (!dw.empty()) {
+            CK(ctx->idat_runs.ensure(dw.size() * 12)); CK(ctx->idat_lens.ensure(tot * 4));
+            uint64_t *d_at = ctx->idat_runs.as<uint64_t>(); uint32_t *d_which = (uint32_t *)(d_at + dw.size());   // (the 8-byte offsets first: aligned)
+            CK(cudaMemcpyAsync(d_at, dat.data(), dw.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
+            CK(cudaMemcpyAsync(d_which, dw.data(), dw.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+            CK(launch_idat_write(ctx->d_file, N, ctx->r0, ctx->r1, ctx->cand.as<uint32_t>(), ctx->idat_counts.as<uint32_t>(), d_which, d_at, (uint32_t)dw.size(),
+                                 ctx->idat_lens.as<uint32_t>(), ctx->stream));
+            ctx->st.kernel_launches++;
+            CK(cudaMemcpyAsync(lens.data(), ctx->idat_lens.p, tot * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        }
+        ph.stop();
+        // runs that leave the resident range (atz_attach): walked again over the whole attached file
+        size_t j = 0;
+        for (uint32_t k = 0; k < nc; k++) {
+            if (counts[k] == IDAT_FAR) {
+                if (!ctx->h_file) { ctx->set_err("IDAT run outside the resident file range"); return ATZ_E_STATE; }
+                const uint32_t m = idat_run(ctx->h_file, N, 0, N, cand[k], nullptr, 0);
+                if (!m) continue;
+                which.push_back(k); cnt.push_back(m); at.push_back(lens.size()); lens.resize(lens.size() + m);
+                idat_run(ctx->h_file, N, 0, N, cand[k], lens.data() + at.back(), m);
+            } else if (j < dw.size() && dw[j] == k) { which.push_back(k); cnt.push_back(counts[k]); at.push_back(dat[j]); j++; }
+        }
+    }
+    const size_t nr = which.size();
+    std::vector<RunBytes> runs(nr);
+    for (size_t i = 0; i < nr; i++) {
+        RunBytes r{cand[which[i]], lens.data() + at[i], cnt[i], 0};
+        for (size_t k = 0; k < cnt[i]; k++) r.total += r.len[k];
+        runs[i] = r;
+    }
+    sc.split[sc.shard].clear(); sc.split_dev.clear();
+    if (!nr) return ATZ_OK;
+    uint8_t *comp = nullptr; std::vector<uint64_t> cat;
+    { int rc = dechunk(ctx, runs, comp, cat); if (rc) return rc; }
+    // K2 over the de-chunked runs: the plaintext length is not known, so a region that turns out too small is enlarged and the job rerun
+    std::vector<size_t> todo(nr); std::vector<uint64_t> cap(nr);
+    for (size_t i = 0; i < nr; i++) { todo[i] = i; cap[i] = align_up(std::max<uint64_t>(4 * 8192, 5 * runs[i].total) + 16384, 256); }
+    std::vector<InflateResult> fin(nr); std::vector<const uint8_t *> plain(nr), tmap(nr);
+    while (!todo.empty()) {
+        uint64_t arena = 0; std::vector<InflateJob> bj(todo.size()); std::vector<InflateResult> br, bc;
+        for (size_t t = 0; t < todo.size(); t++) {
+            const size_t i = todo[t];
+            bj[t] = InflateJob{cat[i], runs[i].total, runs[i].total, arena, cap[i], 0, 0};
+            arena = align_up(arena + cap[i] + ATZ_PAD, 256); bj[t].tmap_off = arena; arena = align_up(arena + cap[i] + 64, 256);
+        }
+        void *q = nullptr; CK(cudaMalloc(&q, arena + ATZ_PAD)); ctx->plain_extra.push_back(q);
+        CK(cudaMemsetAsync(q, 0, arena + ATZ_PAD, ctx->stream));
+        { int rc = run_inflate(ctx, comp, bj, br, bc, (uint8_t *)q, sc.S, &ctx->st.ms_inflate_probe); if (rc) return rc; }
+        std::vector<size_t> again;
+        for (size_t t = 0; t < todo.size(); t++) {
+            const size_t i = todo[t];
+            if (br[t].status == INF_OUT_FULL) {
+                const uint64_t lim = 1032 * runs[i].total + 65536;
+                if (cap[i] >= lim) { ctx->set_err("inflate output exceeds the deflate expansion bound"); return ATZ_E_CUDA; }
+                cap[i] = std::min<uint64_t>(align_up(cap[i] * 6, 256), align_up(lim, 256)); again.push_back(i);
+            } else { fin[i] = br[t]; plain[i] = (uint8_t *)q + bj[t].out_off; tmap[i] = (uint8_t *)q + bj[t].tmap_off; }
+        }
+        todo.swap(again);
+    }
+    for (size_t i = 0; i < nr; i++) {
+        const InflateResult &r = fin[i]; const uint64_t C = r.total_in;
+        if (r.status != INF_END || C <= runs[i].len[0] || C <= 16) continue;
+        SplitX x{runs[i].off, C, r.total_out, r.adler, type[which[i]], {}};
+        for (uint64_t k = 0, got = 0; got < C; k++) { const uint64_t l = std::min<uint64_t>(runs[i].len[k], C - got); x.pieces.push_back((uint32_t)l); got += l; }
+        sc.split[sc.shard].push_back(std::move(x)); sc.split_dev.push_back(SplitDev{comp + cat[i], plain[i], tmap[i]});
+    }
+    return ATZ_OK;
+}
+
 int atz_scan_shard(atz_ctx *ctx, uint64_t chunksize, uint32_t shard, uint32_t nshards) {
     if (!ctx || nshards == 0 || shard >= nshards) return ATZ_E_ARG;
     if (ctx->state < 1) return ATZ_E_STATE;
@@ -850,6 +981,7 @@ int atz_scan_shard(atz_ctx *ctx, uint64_t chunksize, uint32_t shard, uint32_t ns
     ctx->streams.clear(); ctx->state = 1;
     ScanState &sc = ctx->sc; sc = ScanState{};
     sc.S = S; sc.shard = shard; sc.nshards = nshards; sc.px.assign(nshards, std::vector<ProbeX>()); sc.have.assign(nshards, 0);
+    sc.split.assign(nshards, std::vector<SplitX>());
     std::vector<uint64_t> cstart, clen;
     chunk_list(N, S, cstart, clen);
     const size_t nch = cstart.size();
@@ -867,6 +999,7 @@ int atz_scan_shard(atz_ctx *ctx, uint64_t chunksize, uint32_t shard, uint32_t ns
     sc.QS = QS; sc.SLOT = SLOT;
     std::vector<uint32_t> &cand = sc.cand; std::vector<uint8_t> &ctype = sc.ctype;
     std::vector<InflateJob> &jobs = sc.jobs; std::vector<InflateResult> &res = sc.res, &cres = sc.cres;
+    std::vector<uint32_t> k1cand; std::vector<uint8_t> k1type;    // ATZ_SCAN_PNG_IDAT: K1's own candidates (the real file bytes, no chunk-start fix-up)
     // a continuation (a stream that runs over the end of its chunk) reads the following chunks: map `extra` of them behind the
     // shard's own; in the rare case that one needs more than that, the probe is repeated with four times as many
     for (size_t extra = 1;; extra *= 4) {
@@ -892,6 +1025,7 @@ int atz_scan_shard(atz_ctx *ctx, uint64_t chunksize, uint32_t shard, uint32_t ns
             }
             ph.stop();
             CK(cudaGetLastError());
+            if (ctx->scan_flags & ATZ_SCAN_PNG_IDAT) { k1cand = cand; k1type = ctype; }
         }
         // ---- the first position of every chunk k >= 2 holds file[start_k - 1] in the reference's buffer (see chunk_list): fix those up ----
         std::vector<uint8_t> special;    // per candidate: 1 = its first byte is file[off - 1]
@@ -1041,35 +1175,70 @@ int atz_scan_shard(atz_ctx *ctx, uint64_t chunksize, uint32_t shard, uint32_t ns
         if (res[k].status == INF_NEED_INPUT && cres[k].status >= 0) { x.c_status = cres[k].status; x.c_in = cres[k].total_in; x.c_out = cres[k].total_out; x.c_cap = cres[k].in_at_outcap; x.c_adler = cres[k].adler; }
         mine.push_back(x);
     }
+    if (ctx->scan_flags & ATZ_SCAN_PNG_IDAT) { int rc = probe_idat_runs(ctx, k1cand, k1type); if (rc) return rc; }
     sc.have[shard] = 1; sc.probed = true;
     ctx->st.algo_bytes += f1 - f0;
     return ATZ_OK;
 }
 
-// the export: the exporting context's scan flags (8 bytes; the records were found with that header set), then the records
+// the export: the exporting context's scan flags (8 bytes; the records were found with that header set), then the records; with
+// ATZ_SCAN_PNG_IDAT then the split streams (SPLIT_HEAD bytes each: off, C, U, adler, type, number of pieces; then the piece lengths)
+// and the size of that part (8 bytes)
+#define SPLIT_HEAD 36
 int atz_probe_export(atz_ctx *ctx, void *buf, uint64_t cap, uint64_t *nbytes) {
     if (!ctx || !nbytes) return ATZ_E_ARG;
     if (!ctx->sc.probed) return ATZ_E_STATE;
     const std::vector<ProbeX> &v = ctx->sc.px[ctx->sc.shard];
     const uint64_t flags = ctx->scan_flags;
-    *nbytes = sizeof flags + v.size() * sizeof(ProbeX);
+    std::vector<uint8_t> split;
+    if (flags & ATZ_SCAN_PNG_IDAT) {
+        for (const SplitX &x : ctx->sc.split[ctx->sc.shard]) {
+            uint8_t h[SPLIT_HEAD]; const uint32_t np = (uint32_t)x.pieces.size();
+            memcpy(h, &x.off, 8); memcpy(h + 8, &x.c, 8); memcpy(h + 16, &x.u, 8); memcpy(h + 24, &x.adler, 4); memcpy(h + 28, &x.type, 4); memcpy(h + 32, &np, 4);
+            split.insert(split.end(), h, h + SPLIT_HEAD);
+            split.insert(split.end(), (const uint8_t *)x.pieces.data(), (const uint8_t *)(x.pieces.data() + np));
+        }
+        const uint64_t sb = split.size(); split.insert(split.end(), (const uint8_t *)&sb, (const uint8_t *)&sb + 8);
+    }
+    *nbytes = sizeof flags + v.size() * sizeof(ProbeX) + split.size();
     if (!buf || cap < *nbytes) return ATZ_E_SMALL;
     memcpy(buf, &flags, sizeof flags);
     if (!v.empty()) memcpy((uint8_t *)buf + sizeof flags, v.data(), v.size() * sizeof(ProbeX));
+    if (!split.empty()) memcpy((uint8_t *)buf + sizeof flags + v.size() * sizeof(ProbeX), split.data(), split.size());
     return ATZ_OK;
 }
 int atz_probe_import(atz_ctx *ctx, uint32_t shard, const void *buf, uint64_t nbytes) {
-    uint64_t flags = 0;
-    if (!ctx || !buf || nbytes < sizeof flags || (nbytes - sizeof flags) % sizeof(ProbeX)) return ATZ_E_ARG;
+    uint64_t flags = 0, split_bytes = 0;
+    if (!ctx || !buf || nbytes < sizeof flags) return ATZ_E_ARG;
+    const uint8_t *b = (const uint8_t *)buf;
+    memcpy(&flags, b, sizeof flags);
+    if (flags & ATZ_SCAN_PNG_IDAT) {     // the split streams and their size behind the probe records
+        if (nbytes < 2 * sizeof flags) return ATZ_E_ARG;
+        memcpy(&split_bytes, b + nbytes - 8, 8);
+        if (split_bytes > nbytes - 16) return ATZ_E_ARG;
+        split_bytes += 8;
+    }
+    if ((nbytes - sizeof flags - split_bytes) % sizeof(ProbeX)) return ATZ_E_ARG;
     if (!ctx->sc.probed) return ATZ_E_STATE;
     if (shard >= ctx->sc.nshards || shard == ctx->sc.shard) return ATZ_E_ARG;
-    memcpy(&flags, buf, sizeof flags);
     if (flags != ctx->scan_flags) { ctx->set_err("atz_probe_import: the shard scanned with other scan flags (atz_ctx_set_scan_flags)"); return ATZ_E_STATE; }
-    nbytes -= sizeof flags;
+    nbytes -= sizeof flags + split_bytes;
     std::vector<ProbeX> &v = ctx->sc.px[shard];
     v.resize(nbytes / sizeof(ProbeX));
-    if (nbytes) memcpy(v.data(), (const uint8_t *)buf + sizeof flags, nbytes);
+    if (nbytes) memcpy(v.data(), b + sizeof flags, nbytes);
     for (size_t i = 0; i < v.size(); i++) if (v[i].off >= ctx->n || (i && v[i].off <= v[i - 1].off)) return ATZ_E_ARG;
+    std::vector<SplitX> &sv = ctx->sc.split[shard]; sv.clear();
+    for (const uint8_t *q = b + sizeof flags + nbytes, *e = q + (split_bytes ? split_bytes - 8 : 0); q < e;) {
+        if (e - q < SPLIT_HEAD) return ATZ_E_ARG;
+        SplitX x; uint32_t np = 0;
+        memcpy(&x.off, q, 8); memcpy(&x.c, q + 8, 8); memcpy(&x.u, q + 16, 8); memcpy(&x.adler, q + 24, 4); memcpy(&x.type, q + 28, 4); memcpy(&np, q + 32, 4);
+        q += SPLIT_HEAD;
+        if (np < 2 || (uint64_t)(e - q) / 4 < np) return ATZ_E_ARG;
+        x.pieces.resize(np); memcpy(x.pieces.data(), q, 4ull * np); q += 4ull * np;
+        uint64_t sum = 0; for (uint32_t l : x.pieces) sum += l;
+        if (sum != x.c || x.type >= ATZ_NTYPES || x.off >= ctx->n || x.span() > ctx->n - x.off || (!sv.empty() && x.off <= sv.back().off)) return ATZ_E_ARG;
+        sv.push_back(std::move(x));
+    }
     ctx->sc.have[shard] = 1;
     return ATZ_OK;
 }
@@ -1097,20 +1266,62 @@ int atz_scan_finish(atz_ctx *ctx, uint64_t *n_streams) {
         }
         scan_fold(cstart, clen, xc.data(), nx, pr.data(), avail.data(), cont_of.data(), cr.data(), acc);
     }
+    // ---- ATZ_SCAN_PNG_IDAT, after the fold and the same on every context: a split stream (file order) is dropped if an accepted stream
+    // or a split stream kept before it overlaps its span without lying inside it; otherwise it takes the place of the accepted streams
+    // inside its span (accidents of inflating compressed bytes) ----
+    struct SplitRef { const SplitX *x; uint32_t src, local; };
+    std::vector<SplitRef> spl; std::vector<int32_t> split_of;     // split_of[s]: stream s is spl[split_of[s]] (-1: an accepted stream of the fold)
+    for (uint32_t g = 0; g < sc.nshards; g++) for (uint32_t i = 0; i < (uint32_t)sc.split[g].size(); i++) spl.push_back(SplitRef{&sc.split[g][i], g, i});
+    if (!spl.empty()) {
+        std::vector<uint64_t> pmax(acc.size());   // largest end of acc[0 .. j]
+        for (size_t j = 0; j < acc.size(); j++) pmax[j] = std::max(j ? pmax[j - 1] : 0, acc[j].off + acc[j].tin);
+        std::vector<uint8_t> gone(acc.size(), 0); std::vector<uint32_t> kept; uint64_t last = 0;
+        for (uint32_t q = 0; q < (uint32_t)spl.size(); q++) {
+            const uint64_t a = spl[q].x->off, b = a + spl[q].x->span();
+            if (a < last) continue;
+            const size_t j0 = std::lower_bound(acc.begin(), acc.end(), a, [](const Acc &u, uint64_t v) { return u.off < v; }) - acc.begin();
+            if (j0 && pmax[j0 - 1] > a) continue;
+            size_t j1 = j0; bool inside = true;
+            for (; j1 < acc.size() && acc[j1].off < b; j1++) if (acc[j1].off + acc[j1].tin > b) { inside = false; break; }
+            if (!inside) continue;
+            for (size_t j = j0; j < j1; j++) gone[j] = 1;
+            kept.push_back(q); last = b;
+        }
+        std::vector<Acc> m; size_t k = 0;
+        for (size_t j = 0; j <= acc.size(); j++) {
+            for (; k < kept.size() && (j == acc.size() || spl[kept[k]].x->off < acc[j].off); k++) {
+                const SplitX &x = *spl[kept[k]].x;
+                m.push_back(Acc{x.off, x.c, x.u, kept[k], false}); split_of.push_back((int32_t)kept[k]);
+            }
+            if (j < acc.size() && !gone[j]) { m.push_back(acc[j]); split_of.push_back(-1); }
+        }
+        acc.swap(m);
+    }
+    split_of.resize(acc.size(), -1);
     // ---- accepted streams; the ones this shard owns get their plaintext (already resident where this context probed them) ----
     const size_t ns = acc.size();
     std::vector<uint64_t> ulen(ns); std::vector<uint32_t> owner(ns, 0);
     for (size_t s = 0; s < ns; s++) ulen[s] = acc[s].tout;
     std::vector<uint32_t> probed_by(ns);
-    for (size_t s = 0; s < ns; s++) probed_by[s] = src[acc[s].cand];
+    for (size_t s = 0; s < ns; s++) probed_by[s] = split_of[s] >= 0 ? spl[split_of[s]].src : src[acc[s].cand];
     stream_partition(ulen.data(), probed_by.data(), (uint32_t)ns, sc.nshards, owner.data());
     ctx->streams.assign(ns, StreamRec{});
-    std::vector<size_t> recheck; uint64_t far_bytes = 0;
+    std::vector<size_t> recheck, far_runs; uint64_t far_bytes = 0;
     for (size_t s = 0; s < ns; s++) {
         if (acc[s].tout >= 0xffffff00ull || acc[s].tin >= 0xffffff00ull) return ATZ_E_TOO_LARGE;
-        StreamRec &r = ctx->streams[s]; const ProbeX &x = *all[acc[s].cand];
+        StreamRec &r = ctx->streams[s];
         r.s = atz_stream{}; r.s.offset = acc[s].off; r.s.streamLength = acc[s].tin; r.s.inflatedLength = acc[s].tout;
         r.s.clevel = 9; r.s.window = 15; r.s.memlevel = 9; r.s.firstDiffByte = -1;
+        if (split_of[s] >= 0) {     // a split stream: its bytes are resident where it was probed; another owner puts its pieces together and inflates them again
+            const SplitRef &q = spl[split_of[s]];
+            r.s.offsetType = (int32_t)q.x->type; r.owner = owner[s]; r.adler = q.x->adler; r.pieces = q.x->pieces;
+            if (r.owner != sc.shard) continue;
+            if (q.src == sc.shard) { const SplitDev &d = sc.split_dev[q.local]; r.d_comp = d.comp; r.d_plain = d.plain; r.d_tmap = d.tmap; }
+            else { far_runs.push_back(s); recheck.push_back(s); }
+            ctx->st.algo_bytes += acc[s].tin + acc[s].tout;
+            continue;
+        }
+        const ProbeX &x = *all[acc[s].cand];
         r.s.offsetType = (int32_t)(x.type & 0xff); r.owner = owner[s];
         r.adler = acc[s].via_cont ? x.c_adler : x.p_adler;
         if (r.owner != sc.shard) continue;
@@ -1123,6 +1334,13 @@ int atz_scan_finish(atz_ctx *ctx, uint64_t *n_streams) {
         if (acc[s].off >= ctx->r0 && acc[s].off + acc[s].tin <= ctx->r1) r.d_comp = ctx->d_file + acc[s].off;
         else far_bytes += align_up(acc[s].tin + ATZ_PAD, 256);
         ctx->st.algo_bytes += acc[s].tin + acc[s].tout;
+    }
+    if (!far_runs.empty()) {   // (before the staging below, which takes every owned stream that has no compressed bytes yet)
+        std::vector<RunBytes> rb;
+        for (size_t s : far_runs) { const StreamRec &r = ctx->streams[s]; rb.push_back(RunBytes{r.s.offset, r.pieces.data(), r.pieces.size(), r.s.streamLength}); }
+        uint8_t *base = nullptr; std::vector<uint64_t> at;
+        { int rc = dechunk(ctx, rb, base, at); if (rc) return rc; }
+        for (size_t i = 0; i < far_runs.size(); i++) ctx->streams[far_runs[i]].d_comp = base + at[i];
     }
     if (far_bytes) {   // compressed bytes of owned streams outside the mapped range: staged (one pinned-free gather on the host side, one copy)
         if (!ctx->h_file) { ctx->set_err("owned stream outside the resident file range"); return ATZ_E_STATE; }
@@ -1159,6 +1377,7 @@ int atz_scan_finish(atz_ctx *ctx, uint64_t *n_streams) {
         for (size_t i = 0; i < recheck.size(); i++) {
             if (vr[i].status != INF_END || vr[i].total_out != acc[recheck[i]].tout) { ctx->err = "inflate() failed on an accepted stream (reference would abort, main.cpp:451)"; return ATZ_E_DATA; }
             StreamRec &r = ctx->streams[recheck[i]];
+            if (!r.pieces.empty() && (vr[i].total_in != r.s.streamLength || vr[i].adler != r.adler)) { ctx->set_err("a split stream inflates differently on its owner than where it was probed"); return ATZ_E_DATA; }
             r.d_plain = (uint8_t *)q + vj[i].out_off; r.d_tmap = (uint8_t *)q + vj[i].tmap_off; r.adler = vr[i].adler;
         }
     }
@@ -1483,10 +1702,10 @@ int atz_search_shard(atz_ctx *ctx, const atz_options *opt, uint32_t shard, uint3
     uint64_t di = 0, nrec = 0, atz = 28, lastend = 0;
     for (auto &r : ctx->streams) {
         r.s.diff_index = di; di += r.s.ndiff;
-        if (r.s.recomp) { nrec++; atz += 35 + (r.s.ndiff ? 8 + 9 * r.s.ndiff : 0) + r.s.inflatedLength; }
-        else atz += r.s.streamLength;
+        if (r.s.recomp) { nrec++; atz += 35 + (r.s.ndiff ? 8 + 9 * r.s.ndiff : 0) + r.s.inflatedLength + (r.pieces.empty() ? 0 : 8 + 16 * r.pieces.size() - 12); }
+        else atz += r.span();
         if (r.s.offset >= lastend) { atz += r.s.offset - lastend; }
-        lastend = r.s.offset + r.s.streamLength;
+        lastend = r.s.offset + r.span();
     }
     if (lastend < ctx->n) atz += ctx->n - lastend;
     ctx->st.n_recomp = nrec;
@@ -1509,6 +1728,16 @@ int atz_get_owners(atz_ctx *ctx, uint32_t *owner, uint64_t cap) {
     if (ctx->state < 2) return ATZ_E_STATE;
     if (cap < ctx->streams.size()) return ATZ_E_SMALL;
     for (size_t i = 0; i < ctx->streams.size(); i++) owner[i] = ctx->streams[i].owner;
+    return ATZ_OK;
+}
+int atz_get_pieces(atz_ctx *ctx, uint64_t i, uint32_t *len, uint64_t cap, uint64_t *npieces) {
+    if (!ctx || !npieces || (!len && cap)) return ATZ_E_ARG;
+    if (ctx->state < 2) return ATZ_E_STATE;
+    if (i >= ctx->streams.size()) return ATZ_E_ARG;
+    const std::vector<uint32_t> &p = ctx->streams[i].pieces;
+    *npieces = p.size();
+    if (cap < p.size()) return ATZ_E_SMALL;
+    if (!p.empty()) memcpy(len, p.data(), p.size() * 4);
     return ATZ_OK;
 }
 int atz_get_diffs(atz_ctx *ctx, uint64_t *offsets, uint8_t *values, uint64_t cap, uint64_t *n) {
@@ -1746,6 +1975,11 @@ int atz_trial(atz_ctx *ctx, const uint8_t *in, uint64_t n, const uint8_t *orig, 
 
 // ---- host-logic test hooks: pure host code, usable without a CUDA device (tests/test_host_logic.py) ----
 int atz_host_header_type(uint32_t scan_flags, uint32_t b0, uint32_t b1) { return zlib_header_type(b0 & 0xff, b1 & 0xff, scan_flags); }
+int atz_host_idat_run(const uint8_t *file, uint64_t n, uint64_t p, uint32_t *len, uint64_t cap, uint64_t *npieces) {
+    if (!file || !npieces || (!len && cap)) return ATZ_E_ARG;
+    *npieces = p < n ? idat_run(file, n, 0, n, p, len, (uint32_t)std::min<uint64_t>(cap, 0xffffffffull)) : 0;
+    return ATZ_OK;
+}
 int atz_host_candidate_sequence(int offsetType, int brute, uint8_t *clevel, uint8_t *window, uint8_t *memlevel, uint32_t cap) {
     if (offsetType < 0 || offsetType >= ATZ_NTYPES) return ATZ_E_ARG;
     std::vector<Params> v;

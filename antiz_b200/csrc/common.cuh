@@ -101,6 +101,38 @@ __host__ __device__ __forceinline__ int zlib_header_type(uint32_t b0, uint32_t b
 }
 
 // ---------------------------------------------------------------------------------------------
+// PNG IDAT runs (ATZ_SCAN_PNG_IDAT; png.cu, api.cu).  A header at p starts a run when p >= 8, file[p-4..p) == "IDAT", the chunk's
+// length L1 = BE32(file[p-8..p-4]) >= 2 and the chunk behind its CRC (header at p + L1 + 4) is an IDAT too.  The run goes on over
+// consecutive IDATs whose data and CRC lie inside the file [0, n) and ends at another chunk type or at one that would run past the
+// end.  Returns the number of chunks (0: p starts no run; a run has >= 2) and their data lengths in len[0 .. min(count, cap)).
+// Only [lo, lim) is read (the part of the file the caller can address); a walk that would need a byte outside returns IDAT_FAR,
+// and the caller walks again over the whole file.  One dependent 8-byte read per chunk.
+// ---------------------------------------------------------------------------------------------
+#define IDAT_FAR 0xffffffffu
+__host__ __device__ __forceinline__ uint32_t be32(const uint8_t *q) { return (uint32_t)q[0] << 24 | (uint32_t)q[1] << 16 | (uint32_t)q[2] << 8 | q[3]; }
+__host__ __device__ __forceinline__ bool is_idat(const uint8_t *q) { return q[0] == 'I' && q[1] == 'D' && q[2] == 'A' && q[3] == 'T'; }
+__host__ __device__ inline uint32_t idat_run(const uint8_t *file, uint64_t n, uint64_t lo, uint64_t lim, uint64_t p, uint32_t *len, uint32_t cap) {
+    if (p < 8) return 0;
+    if (p - 8 < lo || p > lim) return IDAT_FAR;
+    if (!is_idat(file + p - 4)) return 0;
+    uint64_t L = be32(file + p - 8), d = p;     // the current chunk: data at d, L bytes
+    if (L < 2) return 0;
+    uint32_t cnt = 0;
+    for (;;) {
+        if (d + L + 4 > n) break;                 // data or CRC past the end of the file: not part of the run
+        if (d + L + 4 > lim) return IDAT_FAR;
+        if (cnt < cap) len[cnt] = (uint32_t)L;
+        cnt++;
+        const uint64_t q = d + L + 4;             // the next chunk's header
+        if (q + 8 > n) break;
+        if (q + 8 > lim) return IDAT_FAR;
+        if (!is_idat(file + q + 4)) break;
+        L = be32(file + q); d = q + 8;
+    }
+    return cnt >= 2 ? cnt : 0;
+}
+
+// ---------------------------------------------------------------------------------------------
 // Device helpers
 // ---------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t lane_id() { return threadIdx.x & 31u; }

@@ -5,7 +5,8 @@
 // (writeATZfile/writeStreamdesc main.cpp:764-831), same reconstruction (reconstructATZ main.cpp:869-950) and the
 // same built-in self test (testATZfile main.cpp:1173-1203).  The host keeps what the reference's L1/L2 layers do
 // (CLI, file IO, ATZ1 layout, phase order); phases 1 and 3 and the per-stream deflate of the reconstructor run on
-// the GPU.  Extensions: --gpus N (static shard of the stream x parameter grid), --device D, --exact-records, --stats.
+// the GPU.  Extensions: --gpus N (static shard of the stream x parameter grid), --device D, --exact-records, --stats, --strategies,
+// --small-windows, --png.
 #include "ATZData.h"
 #include "antiz_b200.h"
 #include <chrono>
@@ -101,8 +102,9 @@ class ATZcreator {
             mk(0);
             for (auto &t : th) t.join();
             for (int g = 0; g < ng; g++) if (crc[g] != ATZ_OK) { std::cout << "error: no usable CUDA device " << (options.device + g) << " (antiz_b200 has no CPU path)" << std::endl; std::exit(1); }
-            for (int g = 0; g < ng && options.smallWindows; g++) {   // before any load: every shard scans with the same header set
-                const int rc = atz_ctx_set_scan_flags(ctxs[g], ATZ_SCAN_SMALL_WINDOWS);
+            const uint32_t scan_flags = (options.smallWindows ? ATZ_SCAN_SMALL_WINDOWS : 0) | (options.png ? ATZ_SCAN_PNG_IDAT : 0);
+            for (int g = 0; g < ng && scan_flags; g++) {   // before any load: every shard scans with the same header set
+                const int rc = atz_ctx_set_scan_flags(ctxs[g], scan_flags);
                 if (rc != ATZ_OK) { std::cout << atz_err(ctxs[g], rc) << std::endl; abort(); }
             }
         }
@@ -173,6 +175,11 @@ class ATZcreator {
             s.identBytes = a.identBytes; s.firstDiffByte = a.firstDiffByte; s.recomp = a.recomp != 0;
             s.diffByteOffsets.assign(doff[g].begin() + a.diff_index, doff[g].begin() + a.diff_index + a.ndiff);
             s.diffByteVal.assign(dval[g].begin() + a.diff_index, dval[g].begin() + a.diff_index + a.ndiff);
+            if (options.png) {
+                uint64_t np = 0; atz_get_pieces(ctxs[g], i, nullptr, 0, &np);
+                s.pieces.resize(np);
+                if (np && atz_get_pieces(ctxs[g], i, s.pieces.data(), np, &np) != ATZ_OK) { std::cout << atz_err(ctxs[g], -1) << std::endl; abort(); }
+            }
             streams.push_back(std::move(s));
         }
         std::cout << std::endl;
@@ -201,10 +208,12 @@ class ATZcreator {
 
     uint64_t countRecomp() { uint64_t n = 0; for (auto &s : streams) if (s.recomp) n++; return n; }
 
-    // ATZ1 layout (main.cpp:775-831): header, per recompressed stream {descriptor, diffs, inflated data}, residue.
+    // ATZ1 layout (main.cpp:775-831): header, per recompressed stream {descriptor, diffs, inflated data}, residue.  A stream split over
+    // PNG IDAT chunks (--png) has bit 7 of its window byte set and, behind the diffs, u64 npieces, npieces u32 piece lengths and the
+    // (npieces - 1) x 12 framing bytes between the pieces, copied from the input (its CRCs stay exact even where they are wrong).
     void writeATZfile() {
         uint64_t total = 28, nrec = countRecomp();
-        for (auto &s : streams) if (s.recomp) total += 35 + (s.diffByteOffsets.empty() ? 0 : 8 + 9 * s.diffByteOffsets.size()) + s.inflatedLength;
+        for (auto &s : streams) if (s.recomp) total += 35 + (s.diffByteOffsets.empty() ? 0 : 8 + 9 * s.diffByteOffsets.size()) + s.inflatedLength + (s.pieces.empty() ? 0 : 8 + 16 * s.pieces.size() - 12);
         std::vector<uint8_t> out; out.reserve(total + infileSize);
         out.insert(out.end(), {'A', 'T', 'Z', 1});
         put8(out, 0); put8(out, infileSize); put8(out, nrec);
@@ -230,7 +239,7 @@ class ATZcreator {
             auto &s = streams[i];
             if (!s.recomp) continue;
             put8(out, s.offset); put8(out, s.streamLength); put8(out, s.inflatedLength);
-            out.push_back(s.zlibparams.clevel); out.push_back(s.zlibparams.window); out.push_back(s.zlibparams.memlevel);
+            out.push_back(s.zlibparams.clevel); out.push_back(s.zlibparams.window | (s.pieces.empty() ? 0 : 0x80)); out.push_back(s.zlibparams.memlevel);
             uint64_t nd = s.diffByteOffsets.size();
             put8(out, nd);
             if (nd > 0) {
@@ -238,14 +247,20 @@ class ATZcreator {
                 for (uint64_t k = 0; k < nd; k++) put8(out, s.diffByteOffsets[k]);
                 for (uint64_t k = 0; k < nd; k++) out.push_back(s.diffByteVal[k]);
             }
+            if (!s.pieces.empty()) {
+                put8(out, s.pieces.size());
+                for (uint32_t l : s.pieces) for (int b = 0; b < 4; b++) out.push_back((uint8_t)(l >> (8 * b)));
+                uint64_t at = s.offset;
+                for (size_t k = 0; k + 1 < s.pieces.size(); k++) { at += s.pieces[k]; out.insert(out.end(), file.begin() + at, file.begin() + at + 12); at += 12; }
+            }
             const uint32_t g = owner[i];
             out.insert(out.end(), payload[g].begin() + pay_at[g], payload[g].begin() + pay_at[g] + s.inflatedLength); pay_at[g] += s.inflatedLength;
         }
         uint64_t lastos = 0, lastlen = 0;   // residue: gaps, non-recompressed streams, tail (main.cpp:784-796)
         for (auto &s : streams) {
             if ((lastos + lastlen) != s.offset) out.insert(out.end(), file.begin() + (lastos + lastlen), file.begin() + s.offset);
-            if (!s.recomp) out.insert(out.end(), file.begin() + s.offset, file.begin() + s.offset + s.streamLength);
-            lastos = s.offset; lastlen = s.streamLength;
+            if (!s.recomp) out.insert(out.end(), file.begin() + s.offset, file.begin() + s.offset + s.spanLength());
+            lastos = s.offset; lastlen = s.spanLength();
         }
         if ((lastos + lastlen) < infileSize) out.insert(out.end(), file.begin() + (lastos + lastlen), file.end());
         uint64_t atzlen = out.size();
@@ -288,7 +303,7 @@ class ATZreconstructor {
         }
         if (nstrms > (atzfileSize - 28) / 35) return invalid("stream count exceeds the ATZ file");
         std::vector<ATZdata::streamOffset> list;
-        uint64_t residueos = readStreamdesc_ALL(atz, list, nstrms);
+        uint64_t residueos = readStreamdesc_ALL(atz, list, nstrms, origlen);
         // every stream's doDeflate (main.cpp:914, 976-1003) in batched kernel launches
         atz_ctx *ctx = nullptr;
         if (atz_ctx_create(dev, &ctx) != ATZ_OK) { std::cout << "error: no usable CUDA device (antiz_b200 has no CPU path)" << std::endl; std::exit(1); }
@@ -298,8 +313,8 @@ class ATZreconstructor {
             uint64_t end = 0, gaps = 0;
             for (uint64_t j = 0; j < n; j++) {
                 const auto &s = list[j];
-                if (s.offset < end || s.offset > origlen || s.streamLength > origlen - s.offset) return invalid("stream descriptors out of order or outside the original file");
-                gaps += s.offset - end; end = s.offset + s.streamLength;
+                if (s.offset < end || s.offset > origlen || s.spanLength() > origlen - s.offset) return invalid("stream descriptors out of order or outside the original file");
+                gaps += s.offset - end; end = s.offset + s.spanLength();
                 if (s.streamLength >= 0xffff0000ull || s.inflatedLength >= 0xffffff00ull) return invalid("stream too large");
                 if ((s.zlibparams.clevel & 15) > 9 || (s.zlibparams.clevel >> 4) > 4 || s.zlibparams.window < 9 || s.zlibparams.window > 15 || s.zlibparams.memlevel < 1 || s.zlibparams.memlevel > 9) return invalid("bad zlib parameters");
             }
@@ -340,8 +355,15 @@ class ATZreconstructor {
                     sum += s.diffByteOffsets[i];
                 }
             }
-            recfile.write(reinterpret_cast<const char *>(cb), (std::streamsize)s.streamLength);
-            lastos = s.offset; lastlen = s.streamLength;
+            if (s.pieces.empty()) recfile.write(reinterpret_cast<const char *>(cb), (std::streamsize)s.streamLength);
+            else {   // piece 1, framing 1, piece 2, ...
+                uint64_t at = 0;
+                for (size_t k = 0; k < s.pieces.size(); k++) {
+                    recfile.write(reinterpret_cast<const char *>(cb + at), (std::streamsize)s.pieces[k]); at += s.pieces[k];
+                    if (k + 1 < s.pieces.size()) recfile.write(reinterpret_cast<const char *>(atz.data() + s.gapsAt + 12 * k), 12);
+                }
+            }
+            lastos = s.offset; lastlen = s.spanLength();
         }
         if ((lastos + lastlen) < origlen) recfile.write(reinterpret_cast<const char *>(atz.data() + residueos + gapsum), (std::streamsize)(origlen - (lastos + lastlen)));
         recfile.close();
@@ -359,9 +381,10 @@ class ATZreconstructor {
         origlen = get8(&atz[12]); nstrms = get8(&atz[20]);
         return 0;
     }
-    uint64_t readStreamdesc_ALL(const std::vector<uint8_t> &atz, std::vector<ATZdata::streamOffset> &list, uint64_t nstrms) {   // main.cpp:1031-1063
+    uint64_t readStreamdesc_ALL(const std::vector<uint8_t> &atz, std::vector<ATZdata::streamOffset> &list, uint64_t nstrms, uint64_t origlen) {   // main.cpp:1031-1063
         uint64_t lastos = 28;
         auto need = [&](uint64_t end) { if (end > atz.size()) { std::cout << "Invalid file: truncated stream description" << std::endl; std::exit(1); } };
+        auto invalid = [](const char *what) { std::cout << "Invalid file: " << what << std::endl; std::exit(1); };
         for (uint64_t j = 0; j < nstrms; j++) {
             need(lastos + 35);
             list.push_back(ATZdata::streamOffset(get8(&atz[lastos]), -1, get8(&atz[lastos + 8]), get8(&atz[lastos + 16])));
@@ -377,12 +400,26 @@ class ATZreconstructor {
                     s.diffByteVal.push_back(atz[43 + diffbytes * 8 + i + lastos]);
                 }
                 s.atzInfos = 43 + diffbytes * 9 + lastos;
-                lastos = lastos + 43 + diffbytes * 9 + s.inflatedLength;
             } else {
                 s.firstDiffByte = -1;
                 s.atzInfos = 35 + lastos;
-                lastos = lastos + 35 + s.inflatedLength;
             }
+            if (s.zlibparams.window & 0x80) {   // split over PNG IDAT chunks (--png): piece table and framing bytes, checked before any GPU work
+                s.zlibparams.window &= 0x7f;
+                if (s.zlibparams.window < 9 || s.zlibparams.window > 15) invalid("bad window of a split stream");
+                need(s.atzInfos + 8);
+                const uint64_t np = get8(&atz[s.atzInfos]);
+                if (np < 2) invalid("a split stream needs at least 2 pieces");
+                if (np > (atz.size() - s.atzInfos - 8) / 16 + 1) need(atz.size() + 1);   // (the sizes below cannot wrap)
+                need(s.atzInfos + 8 + 16 * np - 12);
+                uint64_t sum = 0;
+                for (uint64_t k = 0; k < np; k++) { uint32_t l; std::memcpy(&l, &atz[s.atzInfos + 8 + 4 * k], 4); s.pieces.push_back(l); sum += l; }
+                if (sum != s.streamLength) invalid("piece lengths of a split stream do not sum to its length");
+                if (s.offset > origlen || s.spanLength() > origlen - s.offset) invalid("split stream outside the original file");
+                s.gapsAt = s.atzInfos + 8 + 4 * np;
+                s.atzInfos += 8 + 16 * np - 12;
+            }
+            lastos = s.atzInfos + s.inflatedLength;
             if (s.inflatedLength > atz.size()) need(atz.size() + 1);
             need(lastos);
         }
@@ -417,6 +454,7 @@ static const CliArg kExtArgs[] = {   // antiz_b200 only: listed after the refere
     {"", "stats", nullptr, false, "Print per-phase timings to stderr"},
     {"", "strategies", nullptr, false, "For streams that no plain parameter set reproduces, also try zlib's other strategies (Z_FILTERED, Z_FIXED, Z_RLE, Z_HUFFMAN_ONLY). More streams are recompressed, but the ATZ file then differs from the reference's and only this program can reconstruct from it. Default: disabled"},
     {"", "small-windows", nullptr, false, "Also look for zlib streams with 256- and 512-byte windows (header bytes 0x08 and 0x18). More streams are found and recompressed, so the ATZ file differs from the reference's, but the reference can still reconstruct from it. Default: disabled"},
+    {"", "png", nullptr, false, "Also find zlib streams that PNG files split over consecutive IDAT chunks, and recompress them with the chunk framing between the pieces stored verbatim. The ATZ file then differs from the reference's and only this program can reconstruct from it. Default: disabled"},
 };
 static std::string cli_short_id(const CliArg &a) {
     std::string id = a.flag[0] ? std::string("-") + a.flag : std::string("--") + a.name;
@@ -526,6 +564,7 @@ static void parseCLI(int argc, char *argv[], std::string &infile_name, std::stri
         else if (n == "stats") { options.stats = true; g_print_stats = true; }
         else if (n == "strategies") options.strategies = true;
         else if (n == "small-windows") options.smallWindows = true;
+        else if (n == "png") options.png = true;
         else if (n == "help") { usage(argv[0]); std::exit(0); }
         else if (n == "version") { std::cout << std::endl << argv[0] << "  version: " << antiz_ver << std::endl << std::endl; std::exit(0); }
     }

@@ -105,6 +105,15 @@ int  atz_ctx_set_scan_flags(atz_ctx *ctx, uint32_t flags);
  * zlib reproduces differs from its winner in the two header bytes, which go into its diff list.  The ATZ layout does not change, so
  * the reference's reconstructor still reads the file; it differs from the reference's own output because more streams are found. */
 #define ATZ_SCAN_SMALL_WINDOWS 1
+/* Extension (SURVEY.md 8 f4; not in the reference): PNG encoders split an image's zlib stream over consecutive IDAT chunks, with 12 bytes
+ * of chunk framing (CRC, next length and type) between two pieces, so the scan's inflate fails at the end of the first piece.  With this
+ * flag a K1 candidate that starts an IDAT run (header right behind an "IDAT" tag whose chunk is followed by another IDAT; see
+ * atz_host_idat_run) is also inflated over the run's data, concatenated.  A stream that ends there (adler32 correct) beyond its first
+ * chunk and is longer than 16 bytes is a split stream: its record has offset = the header, streamLength = C, the de-chunked compressed
+ * length, and its span in the file is C + 12 * (pieces - 1) bytes (atz_get_pieces).  It replaces the accepted streams that lie inside
+ * that span and is dropped if an accepted stream overlaps the span without lying inside it.  May be ORed with ATZ_SCAN_SMALL_WINDOWS.
+ * The ATZ file of a run with split streams can only be read by this library's reconstructor. */
+#define ATZ_SCAN_PNG_IDAT 4
 
 /* ---- precompress path ------------------------------------------------------------------------------ */
 
@@ -156,6 +165,10 @@ int atz_get_streams(atz_ctx *ctx, atz_stream *streams, uint64_t cap);
 /* owner[i] = shard that owns stream i: set by atz_scan_finish (sharded scan) or by the last atz_search_shard (0 before that).  The
  * host gathers stream i's record, diff list and plaintext from that context; every context of a run reports the same list. */
 int atz_get_owners(atz_ctx *ctx, uint32_t *owner, uint64_t cap);
+/* The pieces of stream i in the file (ATZ_SCAN_PNG_IDAT): *npieces = 0 for an ordinary stream, >= 2 for a split one, whose piece
+ * lengths (summing to streamLength; piece k+1 starts 12 bytes after piece k ends) go to len[0 .. min(npieces, cap)).  ATZ_E_SMALL if
+ * cap < npieces.  Every context of a sharded run reports the same pieces. */
+int atz_get_pieces(atz_ctx *ctx, uint64_t stream_index, uint32_t *len, uint64_t cap, uint64_t *npieces);
 /* diffByteOffsets (delta-encoded, main.cpp:757-763) and diffByteVal of all recomp streams, concatenated. */
 int atz_get_diffs(atz_ctx *ctx, uint64_t *offsets, uint8_t *values, uint64_t cap, uint64_t *n);
 /* Inflated payload of stream i (what writeStreamdesc re-inflates, main.cpp:824-828). */
@@ -205,6 +218,9 @@ int atz_host_candidate_sequence(int offsetType, int brute, uint8_t *clevel, uint
 /* The header test of the scan (the same function K1 runs): offsetType of the zlib header (b0, b1) under the ATZ_SCAN_* set
  * scan_flags, or -1 if the set does not accept it. */
 int atz_host_header_type(uint32_t scan_flags, uint32_t b0, uint32_t b1);
+/* The IDAT run walker of ATZ_SCAN_PNG_IDAT (the same function the run-detection kernel runs) at file offset p: *npieces = number of
+ * IDAT chunks of the run (0: p starts none; a run has >= 2), their data lengths into len[0 .. min(*npieces, cap)). */
+int atz_host_idat_run(const uint8_t *file, uint64_t n, uint64_t p, uint32_t *len, uint64_t cap, uint64_t *npieces);
 /* owner[k] = shard that searches the k-th accepted stream of a scan, given the streams' inflated lengths.  probed_by == NULL: longest
  * first, each to the least loaded shard (what atz_search_shard uses after a plain atz_scan).  probed_by[k] = shard whose chunk range
  * stream k starts in (what atz_scan_finish uses): a stream stays where its plaintext already is unless that shard holds more than 2 %

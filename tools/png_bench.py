@@ -1,0 +1,105 @@
+"""PNG corpus measurement for ATZ_SCAN_PNG_IDAT (uncomp --png): configs[2]'s generator parameters (500 images, 20-200 KB of
+plaintext, half Z_FILTERED) written as PNGs with 8 KB IDAT chunks, scanned and searched with the flag off, with --png and with
+--png --strategies.  Value MB/s uses bench.py's definition: input bytes over device-resident load + scan + search (CUDA events).
+Prints one JSON line per mode and the card's name and power limit.
+
+--overhead: the default bench.py workload (configs[4], 1 GB, --brute-window) with the flag off and on, alternating, `--steps` timed runs
+each, each on a fresh context after one warm-up run; the records of the two must be identical.  Needs a B200."""
+import argparse
+import json
+import os
+import random
+import subprocess
+import sys
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
+import torch  # noqa: E402
+
+import antiz_b200 as az  # noqa: E402
+import corpus  # noqa: E402
+import zref  # noqa: E402
+from test_gpu_png_idat import idat_sizes, png_image  # noqa: E402
+
+
+def png_corpus(n=500, seed=3, umin=20_000, umax=200_000, filtered_frac=0.5):
+    r = random.Random(seed)
+    imgs = []
+    for i in range(n):       # corpus.c3's draws, in the same order
+        u = r.randint(umin, umax)
+        d = corpus.binaryish(u, seed * 100003 + i) if i % 2 else corpus.text(u, seed * 100003 + i)
+        lvl, w, m = r.randint(1, 9), r.randint(10, 15), r.randint(1, 9)
+        strat = 1 if (r.random() < filtered_frac and lvl >= 4) else 0
+        z = zref.ref_deflate(d, lvl, w, m, strat)
+        imgs.append(png_image(z, idat_sizes(len(z), 8192, r), i)[0])
+    return corpus.container(imgs, seed)[0]
+
+
+def measure(data, dev, flags, opt, steps=3):
+    ctx = az.Context(0)
+    if flags:
+        ctx.set_scan_flags(flags)
+    best = None
+    for _ in range(steps + 1):    # the first pass warms up
+        ctx.timer_start()
+        ctx.load_device(dev.data_ptr(), len(data)); ctx.scan(); ctx.search(opt)
+        ms = ctx.timer_stop()
+        best = ms if best is None else min(best, ms)
+    st = ctx.stats(); ss = ctx.streams()
+    atz = 28; last = 0
+    for i, s in enumerate(ss):
+        pc = ctx.pieces(i); span = s.streamLength + 12 * max(0, len(pc) - 1)
+        atz += s.offset - last if s.offset >= last else 0
+        atz += 35 + (8 + 9 * s.ndiff if s.ndiff else 0) + s.inflatedLength + (8 + 16 * len(pc) - 12 if pc else 0) if s.recomp else span
+        last = s.offset + span
+    atz += max(0, len(data) - last)
+    out = dict(streams=len(ss), split=sum(1 for i in range(len(ss)) if ctx.pieces(i)), recompressed=int(st.n_recomp), atz_bytes=atz,
+               value_MBps=round(len(data) / 1e6 / (best / 1e3), 2), ms_best=round(best, 1), ms_scan=round(st.ms_scan, 2), ms_probe=round(st.ms_inflate_probe, 2))
+    ctx.close()
+    return out
+
+
+def overhead(steps):
+    import bench
+    data = bench.make_container("c5", bench.C5_DEFAULT_MB, bench.SEED)
+    dev = torch.frombuffer(bytearray(data), dtype=torch.uint8).cuda()
+    opt = az.Options(bruteforceWindow=True)
+    ms = {"off": [], "png": []}
+    recs = {}
+    for i in range(steps):     # one context at a time (each takes 60 % of the free memory as its budget): a warm-up run, then a timed one
+        for k, flags in (("off", 0), ("png", az.ATZ_SCAN_PNG_IDAT)):
+            ctx = az.Context(0)
+            if flags:
+                ctx.set_scan_flags(flags)
+            for _ in range(2):     # the warm-up, then the timed run
+                ctx.timer_start()
+                ctx.load_device(dev.data_ptr(), len(data)); ctx.scan(bench.CHUNKSIZE); ctx.search(opt)
+                t = ctx.timer_stop()
+            ms[k].append(round(t, 1))
+            recs[k] = ctx.stream_table()
+            ctx.close()
+    same = recs["off"].tobytes() == recs["png"].tobytes() and len(recs["off"]) > 0
+    print(json.dumps(dict(workload="configs[4]", input_bytes=len(data), streams=len(recs["off"]), records_identical=same,
+                          ms_off=ms["off"], ms_png=ms["png"], value_MBps_off=[round(len(data) / 1e3 / t, 1) for t in ms["off"]],
+                          value_MBps_png=[round(len(data) / 1e3 / t, 1) for t in ms["png"]])), flush=True)
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--overhead", action="store_true")
+    ap.add_argument("--steps", type=int, default=3)
+    a = ap.parse_args()
+    smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True, text=True).stdout.strip().splitlines()
+    print(json.dumps(dict(card=smi[0] if smi else "unknown")))
+    if a.overhead:
+        return overhead(a.steps)
+    data = png_corpus()
+    dev = torch.frombuffer(bytearray(data), dtype=torch.uint8).cuda()
+    print(json.dumps(dict(input_bytes=len(data))))
+    for name, flags, opt in (("off", 0, az.Options()), ("png", az.ATZ_SCAN_PNG_IDAT, az.Options()),
+                             ("png+strategies", az.ATZ_SCAN_PNG_IDAT, az.Options(flags=az.ATZ_F_STRATEGIES))):
+        print(json.dumps(dict(mode=name, **measure(data, dev, flags, opt))), flush=True)
+
+
+if __name__ == "__main__":
+    main()

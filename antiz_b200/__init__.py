@@ -21,6 +21,11 @@ ATZ_SCAN_PNG_IDAT = 4        # extension: the scan also finds zlib streams split
 def clevel(level, strategy=0):
     """`clevel` byte with a zlib strategy in its high nibble (ATZ_CLEVEL)"""
     return level | (strategy << 4)
+
+
+def nested_depth(d):
+    """Options.flags bits asking the search to recompress zlib streams nested inside recompressed ones, d levels deep (ATZ_F_NESTED_DEPTH)"""
+    return d << 8
 TR_COMPARED, TR_BAILED, TR_SIZE, TR_CUT = 0, 1, 2, 3
 
 
@@ -44,6 +49,11 @@ class Stream(C.Structure):
     _fields_ = [("offset", C.c_uint64), ("streamLength", C.c_uint64), ("inflatedLength", C.c_uint64), ("identBytes", C.c_uint64),
                 ("firstDiffByte", C.c_int64), ("ndiff", C.c_uint64), ("diff_index", C.c_uint64), ("offsetType", C.c_int32),
                 ("clevel", C.c_uint8), ("window", C.c_uint8), ("memlevel", C.c_uint8), ("recomp", C.c_uint8)]
+
+
+class Nested(C.Structure):
+    """atz_nested: a stream inside the plaintext of `parent` (< n_streams: a top-level stream; else entry parent - n_streams of the same list)"""
+    _fields_ = [("parent", C.c_uint64), ("depth", C.c_uint32), ("reserved", C.c_uint32), ("s", Stream)]
 
 
 class Stats(C.Structure):
@@ -92,6 +102,7 @@ def lib():
         L.atz_search_shard.argtypes = [C.c_void_p, C.POINTER(Options), C.c_uint32, C.c_uint32]
         L.atz_get_streams.argtypes = [C.c_void_p, C.POINTER(Stream), C.c_uint64]
         L.atz_get_diffs.argtypes = [C.c_void_p, C.POINTER(C.c_uint64), C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
+        L.atz_get_nested.argtypes = [C.c_void_p, C.POINTER(Nested), C.c_uint64, C.POINTER(C.c_uint64)]
         L.atz_get_inflated.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64]
         L.atz_get_inflated_recomp.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
         L.atz_get_inflated_list.argtypes = [C.c_void_p, C.POINTER(C.c_uint64), C.c_uint64, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
@@ -108,7 +119,7 @@ def lib():
 
 
 EXPORTS = ["atz_version", "atz_last_error", "atz_ctx_create", "atz_ctx_destroy", "atz_ctx_set_budget", "atz_ctx_set_scan_flags", "atz_load", "atz_load_device",
-           "atz_scan", "atz_attach", "atz_scan_shard", "atz_probe_export", "atz_probe_import", "atz_scan_finish", "atz_host_partition", "atz_search", "atz_search_shard", "atz_get_streams", "atz_get_owners", "atz_get_pieces", "atz_get_diffs", "atz_get_inflated", "atz_get_inflated_recomp", "atz_get_inflated_list", "atz_get_stats", "atz_timer_start", "atz_timer_stop",
+           "atz_scan", "atz_attach", "atz_scan_shard", "atz_probe_export", "atz_probe_import", "atz_scan_finish", "atz_host_partition", "atz_search", "atz_search_shard", "atz_get_streams", "atz_get_owners", "atz_get_pieces", "atz_get_diffs", "atz_get_nested", "atz_get_inflated", "atz_get_inflated_recomp", "atz_get_inflated_list", "atz_get_stats", "atz_timer_start", "atz_timer_stop",
            "atz_inflate_stream", "atz_deflate_stream", "atz_deflate_batch", "atz_trial"]
 
 
@@ -265,6 +276,18 @@ class Context:
         vals = (C.c_uint8 * n.value)()
         self._ck(lib().atz_get_diffs(self._h, offs, vals, n.value, C.byref(n)))
         return list(offs), bytes(vals)
+
+    def nested(self):
+        """the nested streams of the last search (atz_get_nested): Nested records, level by level, then by parent, then by offset; the
+        payload of entry j is inflated(n_streams + j, ...)"""
+        n = C.c_uint64()
+        rc = lib().atz_get_nested(self._h, None, 0, C.byref(n))
+        if rc not in (ATZ_OK, ATZ_E_SMALL):
+            self._ck(rc)
+        arr = (Nested * max(n.value, 1))()
+        if n.value:
+            self._ck(lib().atz_get_nested(self._h, arr, n.value, C.byref(n)))
+        return [arr[i] for i in range(n.value)]
 
     def inflated(self, i, length):
         out = (C.c_uint8 * max(length, 1))()

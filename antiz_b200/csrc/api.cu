@@ -67,6 +67,7 @@ struct StreamRec {
     uint32_t adler = 0;
     std::vector<uint64_t> diff_off; std::vector<uint8_t> diff_val;
     std::vector<uint32_t> pieces;       // ATZ_SCAN_PNG_IDAT: the piece lengths of a split stream (empty: an ordinary stream)
+    uint64_t parent = 0; uint32_t depth = 0;   // a nested stream (ATZ_F_NESTED_DEPTH): atz_nested.parent and .depth; s.offset is relative to the parent's plaintext
     uint64_t span() const { return s.streamLength + (pieces.empty() ? 0 : 12 * (pieces.size() - 1)); }   // bytes from s.offset to the stream's end in the file
 };
 
@@ -135,6 +136,9 @@ struct atz_ctx {
     ScanState sc;
     // streams
     std::vector<StreamRec> streams; Buf plain, plain2; std::vector<void *> plain_extra;   // stage-1 slots, stage-2 regions, retry rounds
+    // nested streams of the last search (ATZ_F_NESTED_DEPTH), level by level; their plaintext and token maps live in nest_extra, the
+    // scan buffer of a level and the probe slots in nest_scan / nest_slots (never ctx->plain: parents may live in its stage-1 slots)
+    std::vector<StreamRec> nested; std::vector<void *> nest_extra; Buf nest_scan, nest_slots;
     // search
     Lane lane[ATZ_LANES];   // lane 0 runs on `stream` (the single-stream operators use it); 1.. have streams of lower priority
     Buf gather, cjobs;
@@ -179,6 +183,7 @@ int trial_slots(atz_ctx *ctx) { return ctx->sms * 24; }   // 3 CTAs x 8 warps pe
 // windowBits 8 into 9, and a CINFO 0 header is written over a window-9 stream)
 inline int type_window(int offsetType) { return offsetType >= 24 ? 9 : 10 + offsetType / 4; }
 #define ATZ_NTYPES 32
+#define ATZ_NESTED_MAX 8   // deepest ATZ_F_NESTED_DEPTH
 
 // ---- candidate order of the reference (main.cpp:487-602, 732-756) ----
 void push_range(std::vector<Params> &v, int cmin, int cmax, int wmin, int wmax, int mmin, int mmax) {
@@ -763,9 +768,10 @@ void atz_ctx_destroy(atz_ctx *ctx) {
     cudaSetDevice(ctx->device);
     cudaStreamSynchronize(ctx->stream);
     Buf *all[] = {&ctx->file, &ctx->tile_counts, &ctx->scan_masks, &ctx->cand, &ctx->ctype, &ctx->jobs, &ctx->jres, &ctx->queue, &ctx->jres2, &ctx->total, &ctx->idat_counts, &ctx->idat_runs, &ctx->idat_lens, &ctx->plain, &ctx->plain2,
-                  &ctx->gather, &ctx->cjobs, &ctx->comp_extra, &ctx->op_in, &ctx->op_orig, &ctx->op_out, &ctx->op_misc};
+                  &ctx->gather, &ctx->cjobs, &ctx->comp_extra, &ctx->op_in, &ctx->op_orig, &ctx->op_out, &ctx->op_misc, &ctx->nest_scan, &ctx->nest_slots};
     for (Buf *b : all) b->release();
     for (void *q : ctx->plain_extra) cudaFree(q);
+    for (void *q : ctx->nest_extra) cudaFree(q);
     for (int l = 0; l < ATZ_LANES; l++) {
         Lane &L = ctx->lane[l];
         if (L.ts[1].stream) { cudaStreamSynchronize(L.ts[1].stream); cudaStreamDestroy(L.ts[1].stream); }
@@ -784,7 +790,13 @@ int atz_ctx_set_scan_flags(atz_ctx *ctx, uint32_t flags) {
     return ATZ_OK;
 }
 
+static void drop_nested(atz_ctx *ctx) {
+    ctx->nested.clear();
+    for (void *q : ctx->nest_extra) cudaFree(q);
+    ctx->nest_extra.clear();
+}
 static void reset_scan(atz_ctx *ctx) {
+    drop_nested(ctx);
     ctx->st = atz_stats{}; ctx->streams.clear(); ctx->state = 0; ctx->sc = ScanState{}; ctx->scan_flags_fixed = true;
 }
 static int load_common(atz_ctx *ctx, const void *src, uint64_t n, cudaMemcpyKind kind) {
@@ -978,6 +990,7 @@ int atz_scan_shard(atz_ctx *ctx, uint64_t chunksize, uint32_t shard, uint32_t ns
     if (chunksize < 2) return ATZ_E_ARG;
     cudaSetDevice(ctx->device);
     const uint64_t N = ctx->n, S = chunksize;
+    drop_nested(ctx);     // (their bytes point into the plaintext freed below)
     ctx->streams.clear(); ctx->state = 1;
     ScanState &sc = ctx->sc; sc = ScanState{};
     sc.S = S; sc.shard = shard; sc.nshards = nshards; sc.px.assign(nshards, std::vector<ProbeX>()); sc.have.assign(nshards, 0);
@@ -1404,17 +1417,17 @@ static void merge_lane_stats(atz_ctx *ctx, Lane &L) {
     ctx->st.ms_trials_max_kernel = std::max(ctx->st.ms_trials_max_kernel, a.ms_trials_max_kernel);
 }
 
-// The search of one lane: the streams `sidx` (indices into ctx->streams), in batches whose chain structures fit the lane's budget.
-static int search_lane(atz_ctx *ctx, Lane &L, const atz_options *opt, const TrialOpts &topts, const std::vector<uint32_t> &sidx,
+// The search of one lane: the streams `sidx` (indices into R: ctx->streams, or ctx->nested), in batches whose chain structures fit the lane's budget.
+static int search_lane(atz_ctx *ctx, Lane &L, const atz_options *opt, const TrialOpts &topts, std::vector<StreamRec> &R, const std::vector<uint32_t> &sidx,
                        const std::vector<Params> *seq_class, const std::vector<Params> *seq_brute, const std::vector<Params> *seq_strat) {
     cudaSetDevice(ctx->device);
     const size_t ns = sidx.size();
     std::vector<PlainView> views(ns);
     for (size_t j = 0; j < ns; j++) {
-        const StreamRec &r = ctx->streams[sidx[j]];
+        const StreamRec &r = R[sidx[j]];
         views[j] = PlainView{r.d_plain, (uint32_t)r.s.inflatedLength, r.d_comp, (uint32_t)r.s.streamLength, r.adler, r.d_tmap};
     }
-    auto S = [&](size_t j) -> atz_stream & { return ctx->streams[sidx[j]].s; };
+    auto S = [&](size_t j) -> atz_stream & { return R[sidx[j]].s; };
     const size_t slots_share = std::max<size_t>(64, (size_t)trial_slots(ctx) / (size_t)std::max(1, ctx->nlanes_last));   // speculation depth as if the lanes shared one launch
     CK(L.queue.ensure(64));
     struct Prog { const std::vector<Params> *sq = nullptr; size_t next = 0; int phase = 0; bool done = false; };   // phase 0 = header class, 1 = brute window, 2 = other strategies (extension)
@@ -1588,7 +1601,7 @@ static int search_lane(atz_ctx *ctx, Lane &L, const atz_options *opt, const Tria
             std::vector<DiffJob> dj; uint64_t dpos = 0; std::vector<uint64_t> dstart;
             for (size_t q = 0; q < need.size(); q++) {
                 atz_stream &st = S(need[q]); uint32_t cap = (uint32_t)(st.streamLength - st.identBytes + 1);
-                dj.push_back(DiffJob{L.tmp_out.as<uint8_t>() + offs[q], ctx->streams[sidx[need[q]]].d_comp, tr[q].out_len, (uint32_t)st.streamLength,
+                dj.push_back(DiffJob{L.tmp_out.as<uint8_t>() + offs[q], R[sidx[need[q]]].d_comp, tr[q].out_len, (uint32_t)st.streamLength,
                                      L.tmp_pos.as<uint32_t>() + dpos, L.tmp_val.as<uint8_t>() + dpos, cap, L.tmp_cnt.as<uint32_t>() + q});
                 dstart.push_back(dpos); dpos += cap;
             }
@@ -1604,7 +1617,7 @@ static int search_lane(atz_ctx *ctx, Lane &L, const atz_options *opt, const Tria
             CK(cudaMemcpyAsync(hcnt.data(), L.tmp_cnt.p, need.size() * 4, cudaMemcpyDeviceToHost, L.stream));
             CK(cudaStreamSynchronize(L.stream));
             for (size_t q = 0; q < need.size(); q++) {
-                StreamRec &r = ctx->streams[sidx[need[q]]]; uint32_t nd = hcnt[q];
+                StreamRec &r = R[sidx[need[q]]]; uint32_t nd = hcnt[q];
                 if (nd != r.s.streamLength - r.s.identBytes) { ctx->set_err("diff pass disagrees with the trial's ident count"); return ATZ_E_CUDA; }
                 r.s.firstDiffByte = hpos[dstart[q]]; r.s.ndiff = nd;
                 r.diff_off.resize(nd); r.diff_val.resize(nd);
@@ -1656,10 +1669,172 @@ static int search_lane(atz_ctx *ctx, Lane &L, const atz_options *opt, const Tria
     return ATZ_OK;
 }
 
+// The streams `which` (indices into R) on the search lanes (lane_partition), one host thread each
+static int search_set(atz_ctx *ctx, const atz_options *opt, const TrialOpts &topts, std::vector<StreamRec> &R, const std::vector<uint32_t> &which,
+                      const std::vector<Params> *seq_class, const std::vector<Params> *seq_brute, const std::vector<Params> *seq_strat) {
+    std::vector<uint64_t> ulen(which.size());
+    for (size_t k = 0; k < which.size(); k++) ulen[k] = R[which[k]].s.inflatedLength;
+    std::vector<std::vector<uint32_t>> part;
+    const int nl = lane_partition(ulen.data(), (uint32_t)ulen.size(), getenv("ATZ_LANES") ? atoi(getenv("ATZ_LANES")) : 0, part);
+    for (auto &v : part) for (uint32_t &k : v) k = which[k];     // positions in `which` -> indices into R (ascending either way)
+    ctx->nlanes_last = nl;
+    for (int l = 0; l < nl; l++) { ctx->lane[l].st = atz_stats{}; ctx->lane[l].budget = ctx->budget / nl; }
+    std::vector<int> rcs(nl, ATZ_OK);
+    {
+        std::vector<std::thread> th;
+        for (int l = 1; l < nl; l++) th.emplace_back([&, l] { rcs[l] = search_lane(ctx, ctx->lane[l], opt, topts, R, part[l], seq_class, seq_brute, seq_strat); });
+        rcs[0] = search_lane(ctx, ctx->lane[0], opt, topts, R, part[0], seq_class, seq_brute, seq_strat);
+        for (auto &t : th) t.join();
+    }
+    for (int l = 0; l < nl; l++) merge_lane_stats(ctx, ctx->lane[l]);   // phase times are per-lane event times and overlap each other
+    for (int rc : rcs) if (rc) return rc;
+    return ATZ_OK;
+}
+
+// One level of the nested descent (ATZ_F_NESTED_DEPTH).  The plaintext P of every parent in `par` (ids as atz_nested.parent counts them)
+// is gathered into one scan buffer with ATZ_PAD zero bytes behind each, in batches of at most an eighth of the budget and of 2 GiB (K1's
+// candidate positions are 32 bits wide; a batch of one parent, < 0xffffff00 bytes, always fits).  K1 runs over the
+// buffer as it is: no accepted first byte is 0x00, and (b0, 0x00) is never a header (b0 * 256 % 31 == 0 only for multiples of 31, none
+// of which is accepted), so no hit starts in a gap or runs into one.  K2 inflates every candidate with its input cut at the end of its
+// parent (no token map, an output region grown on overflow).  Walking P ascending, a candidate that ends there with a correct adler32
+// after more than 16 bytes is a stream, and the walk goes on behind it; no chunking, no IDAT runs.  The streams found are inflated once
+// more into regions of their exact size with token maps, as top-level streams are.  Their compressed bytes stay in their parent's P.
+static int probe_nested(atz_ctx *ctx, const std::vector<uint64_t> &par, uint32_t depth) {
+    const uint64_t ns = ctx->streams.size();
+    struct Par { uint64_t id; const uint8_t *plain; uint64_t u; uint32_t owner; };
+    std::vector<Par> pv;
+    for (uint64_t id : par) { const StreamRec &r = id < ns ? ctx->streams[id] : ctx->nested[id - ns]; pv.push_back(Par{id, r.d_plain, r.s.inflatedLength, r.owner}); }
+    const uint32_t flags = ctx->scan_flags & ATZ_SCAN_SMALL_WINDOWS;
+    const uint64_t lim = getenv("ATZ_NEST_BATCH") ? (uint64_t)std::max(1, atoi(getenv("ATZ_NEST_BATCH")))     // test hook
+                                                  : std::min<uint64_t>(std::max<uint64_t>(ctx->budget / 8, 64ull << 20), 2ull << 30);
+    const uint64_t Q = 8192;
+    for (size_t b0 = 0; b0 < pv.size();) {
+        std::vector<uint64_t> at; uint64_t tot = 0; size_t b1 = b0;
+        for (; b1 < pv.size(); b1++) {
+            const uint64_t nt = align_up(tot + pv[b1].u + ATZ_PAD, 256);
+            if (b1 > b0 && nt > lim) break;
+            at.push_back(tot); tot = nt;
+        }
+        if (at.back() + pv[b1 - 1].u > 0xffffffffull) { ctx->set_err("nested scan buffer positions exceed 32 bits"); return ATZ_E_TOO_LARGE; }
+        CK(ctx->nest_scan.ensure(tot + ATZ_PAD));
+        uint8_t *buf = ctx->nest_scan.as<uint8_t>();
+        CK(cudaMemsetAsync(buf, 0, tot + ATZ_PAD, ctx->stream));
+        {
+            std::vector<CopyJob> cj;
+            for (size_t i = b0; i < b1; i++) if (pv[i].u) cj.push_back(CopyJob{pv[i].plain, buf + at[i - b0], pv[i].u});
+            if (!cj.empty()) {
+                CK(ctx->cjobs.ensure(cj.size() * sizeof(CopyJob)));
+                CK(cudaMemcpyAsync(ctx->cjobs.p, cj.data(), cj.size() * sizeof(CopyJob), cudaMemcpyHostToDevice, ctx->stream));
+                CK(launch_gather(ctx->cjobs.as<CopyJob>(), (uint32_t)cj.size(), ctx->stream)); ctx->st.kernel_launches++;
+            }
+        }
+        // ---- K1 over the scan buffer ----
+        std::vector<uint32_t> cand; std::vector<uint8_t> ctype;
+        {
+            Phase ph(ctx, &ctx->st.ms_scan);
+            CK(ctx->tile_counts.ensure((size_t)scan_tiles_for(0, tot) * 4 + 64)); CK(ctx->scan_masks.ensure((size_t)scan_tiles_for(0, tot) * 8192 + 64));
+            CK(ctx->total.ensure(64)); CK(ctx->queue.ensure(64));
+            uint32_t nc = 0;
+            CK(launch_scan_count(buf, 0, tot, tot, flags, ctx->tile_counts.as<uint32_t>(), ctx->scan_masks.as<uint16_t>(), ctx->total.as<uint32_t>(), ctx->stream));
+            CK(cudaMemcpyAsync(&nc, ctx->total.p, 4, cudaMemcpyDeviceToHost, ctx->stream));
+            CK(cudaStreamSynchronize(ctx->stream));
+            ctx->st.kernel_launches += 2;
+            if (nc) {
+                CK(ctx->cand.ensure((size_t)nc * 4)); CK(ctx->ctype.ensure(nc));
+                CK(launch_scan_write(buf, 0, tot, ctx->scan_masks.as<uint16_t>(), ctx->tile_counts.as<uint32_t>(), ctx->cand.as<uint32_t>(), ctx->ctype.as<uint8_t>(), nc, ctx->stream));
+                ctx->st.kernel_launches++;
+                cand.resize(nc); ctype.resize(nc);
+                CK(cudaMemcpyAsync(cand.data(), ctx->cand.p, (size_t)nc * 4, cudaMemcpyDeviceToHost, ctx->stream));
+                CK(cudaMemcpyAsync(ctype.data(), ctx->ctype.p, nc, cudaMemcpyDeviceToHost, ctx->stream));
+            }
+            ph.stop();
+            CK(cudaGetLastError());
+        }
+        ctx->st.algo_bytes += tot;
+        // ---- K2 probe: every candidate's input is the rest of its parent's P ----
+        const size_t nc = cand.size();
+        std::vector<uint32_t> pof(nc); std::vector<InflateJob> jobs(nc); std::vector<InflateResult> res(nc);
+        for (size_t k = 0, i = 0; k < nc; k++) {
+            while (i + 1 < at.size() && cand[k] >= at[i + 1]) i++;
+            pof[k] = (uint32_t)i;
+            const uint64_t end = at[i] + pv[b0 + i].u, avail = end > cand[k] ? end - cand[k] : 0;
+            jobs[k] = InflateJob{cand[k], avail, avail, 0, Q, ~0ull, 0};
+        }
+        {
+            std::vector<size_t> todo(nc); std::vector<uint64_t> cap(nc, Q);
+            for (size_t k = 0; k < nc; k++) todo[k] = k;
+            while (!todo.empty()) {
+                std::vector<size_t> again;
+                for (size_t t0 = 0; t0 < todo.size();) {     // launches whose output regions stay within `lim` (at least one job each)
+                    std::vector<InflateJob> bj; uint64_t arena = 0; size_t t1 = t0;
+                    for (; t1 < todo.size(); t1++) {
+                        const uint64_t sz = align_up(cap[todo[t1]] + ATZ_PAD, 256);
+                        if (t1 > t0 && arena + sz > lim) break;
+                        InflateJob j = jobs[todo[t1]]; j.out_off = arena; j.out_cap = cap[todo[t1]]; bj.push_back(j); arena += sz;
+                    }
+                    CK(ctx->nest_slots.ensure(arena + ATZ_PAD));
+                    CK(cudaMemsetAsync(ctx->nest_slots.p, 0, arena + ATZ_PAD, ctx->stream));
+                    std::vector<InflateResult> br, bc;
+                    { int rc = run_inflate(ctx, buf, bj, br, bc, ctx->nest_slots.as<uint8_t>(), ~0ull, &ctx->st.ms_inflate_probe); if (rc) return rc; }
+                    for (size_t t = t0; t < t1; t++) {
+                        const size_t k = todo[t]; res[k] = br[t - t0];
+                        // (the bound is deflate's 1032:1 expansion; a plaintext of 4 GiB or more could not be recorded)
+                        const uint64_t bound = std::min<uint64_t>(1032 * jobs[k].avail + 65536, 0xffffff00ull);
+                        if (res[k].status == INF_OUT_FULL && cap[k] < bound) { cap[k] = std::min<uint64_t>(cap[k] * 6, bound); again.push_back(k); }
+                    }
+                    t0 = t1;
+                }
+                todo.swap(again);
+            }
+        }
+        // ---- the walk over each parent's P ----
+        std::vector<size_t> acc; uint64_t next = 0;
+        for (size_t k = 0, cur = SIZE_MAX; k < nc; k++) {
+            if (pof[k] != cur) { cur = pof[k]; next = 0; }
+            const uint64_t p = cand[k] - at[pof[k]];
+            if (p < next) continue;
+            if (res[k].status == INF_END && res[k].total_in > 16 && res[k].total_out < 0xffffff00ull) { acc.push_back(k); next = p + res[k].total_in; }
+        }
+        // ---- produce mode: plaintext + token map of every stream found ----
+        if (!acc.empty()) {
+            std::vector<size_t> ord(acc.size());     // longest first (the jobs run off a queue)
+            for (size_t i = 0; i < ord.size(); i++) ord[i] = i;
+            std::stable_sort(ord.begin(), ord.end(), [&](size_t a, size_t b) { return res[acc[a]].total_out > res[acc[b]].total_out; });
+            uint64_t arena = 0; std::vector<InflateJob> vj(acc.size()); std::vector<InflateResult> vr, vc;
+            for (size_t i = 0; i < ord.size(); i++) {
+                const size_t k = acc[ord[i]]; const uint64_t u = res[k].total_out;
+                vj[i] = InflateJob{cand[k], jobs[k].avail, jobs[k].avail, arena, u, 0, 0}; arena = align_up(arena + u + ATZ_PAD, 256);
+                vj[i].tmap_off = arena; arena = align_up(arena + u + 64, 256);
+            }
+            void *q = nullptr; CK(cudaMalloc(&q, arena + ATZ_PAD)); ctx->nest_extra.push_back(q);
+            CK(cudaMemsetAsync(q, 0, arena + ATZ_PAD, ctx->stream));
+            { int rc = run_inflate(ctx, buf, vj, vr, vc, (uint8_t *)q, ~0ull, &ctx->st.ms_inflate); if (rc) return rc; }
+            std::vector<size_t> slot(acc.size());
+            for (size_t i = 0; i < ord.size(); i++) slot[ord[i]] = i;
+            for (size_t a = 0; a < acc.size(); a++) {
+                const size_t k = acc[a], i = slot[a]; const Par &pp = pv[b0 + pof[k]];
+                if (vr[i].status != INF_END || vr[i].total_out != res[k].total_out || vr[i].total_in != res[k].total_in) { ctx->set_err("a nested stream inflates differently the second time"); return ATZ_E_DATA; }
+                StreamRec r;
+                r.s = atz_stream{}; r.s.offset = cand[k] - at[pof[k]]; r.s.streamLength = res[k].total_in; r.s.inflatedLength = res[k].total_out;
+                r.s.offsetType = ctype[k]; r.s.clevel = 9; r.s.window = 15; r.s.memlevel = 9; r.s.firstDiffByte = -1;
+                r.d_plain = (uint8_t *)q + vj[i].out_off; r.d_tmap = (uint8_t *)q + vj[i].tmap_off; r.d_comp = pp.plain + r.s.offset;
+                r.owner = pp.owner; r.adler = vr[i].adler; r.parent = pp.id; r.depth = depth;
+                ctx->nested.push_back(std::move(r));
+                ctx->st.algo_bytes += res[k].total_in + res[k].total_out;
+            }
+        }
+        b0 = b1;
+    }
+    return ATZ_OK;
+}
+
 int atz_search_shard(atz_ctx *ctx, const atz_options *opt, uint32_t shard, uint32_t nshards) {
     if (!ctx || !opt || nshards == 0 || shard >= nshards) return ATZ_E_ARG;
+    const uint32_t depth = (uint32_t)opt->flags >> 8;     // (every bit from 8 up: a depth above 8 is refused, not wrapped)
+    if (depth > ATZ_NESTED_MAX) return ATZ_E_ARG;
     if (ctx->state < 2) return ATZ_E_STATE;
     cudaSetDevice(ctx->device);
+    drop_nested(ctx);
     const size_t ns = ctx->streams.size();
     const TrialOpts topts = make_opts(opt, true);
     ctx->dbg = HostDbg{}; for (int l = 0; l < ATZ_LANES; l++) ctx->lane[l].dbg = &ctx->dbg;
@@ -1683,22 +1858,24 @@ int atz_search_shard(atz_ctx *ctx, const atz_options *opt, uint32_t shard, uint3
         r.s.identBytes = 0; r.s.clevel = 9; r.s.window = 15; r.s.memlevel = 9; r.s.recomp = 0; r.s.firstDiffByte = -1; r.s.ndiff = 0; r.diff_off.clear(); r.diff_val.clear();
         if (r.owner == shard) mine.push_back((uint32_t)s);
     }
-    std::vector<uint64_t> ulen(mine.size());
-    for (size_t k = 0; k < mine.size(); k++) ulen[k] = ctx->streams[mine[k]].s.inflatedLength;
-    std::vector<std::vector<uint32_t>> part;
-    const int nl = lane_partition(ulen.data(), (uint32_t)ulen.size(), getenv("ATZ_LANES") ? atoi(getenv("ATZ_LANES")) : 0, part);
-    for (auto &v : part) for (uint32_t &k : v) k = mine[k];     // positions in `mine` -> stream indices (ascending either way)
-    ctx->nlanes_last = nl;
-    for (int l = 0; l < nl; l++) { ctx->lane[l].st = atz_stats{}; ctx->lane[l].budget = ctx->budget / nl; }
-    std::vector<int> rcs(nl, ATZ_OK);
-    {
-        std::vector<std::thread> th;
-        for (int l = 1; l < nl; l++) th.emplace_back([&, l] { rcs[l] = search_lane(ctx, ctx->lane[l], opt, topts, part[l], seq_class, seq_brute, seq_strat); });
-        rcs[0] = search_lane(ctx, ctx->lane[0], opt, topts, part[0], seq_class, seq_brute, seq_strat);
-        for (auto &t : th) t.join();
+    { int rc = search_set(ctx, opt, topts, ctx->streams, mine, seq_class, seq_brute, seq_strat); if (rc) return rc; }
+    // ATZ_F_NESTED_DEPTH: level by level, the plaintext of the recompressed streams of the level above that this context owns is scanned
+    // (probe_nested) and the streams found there are searched like top-level ones; they belong to their parent's owner
+    std::vector<uint64_t> par;
+    for (size_t s = 0; s < ns && depth; s++) if (ctx->streams[s].s.recomp && ctx->streams[s].owner == shard && ctx->streams[s].d_plain) par.push_back(s);
+    for (uint32_t d = 1; d <= depth && !par.empty(); d++) {
+        const size_t first = ctx->nested.size();
+        {   // the scan buffer and the probe slots are needed for the probe only
+            const int rc = probe_nested(ctx, par, d);
+            ctx->nest_scan.release(); ctx->nest_slots.release();
+            if (rc) return rc;
+        }
+        std::vector<uint32_t> lvl;
+        for (size_t j = first; j < ctx->nested.size(); j++) lvl.push_back((uint32_t)j);
+        { int rc = search_set(ctx, opt, topts, ctx->nested, lvl, seq_class, seq_brute, seq_strat); if (rc) return rc; }
+        par.clear();
+        for (uint32_t j : lvl) if (ctx->nested[j].s.recomp) par.push_back(ns + j);
     }
-    for (int l = 0; l < nl; l++) merge_lane_stats(ctx, ctx->lane[l]);   // phase times are per-lane event times and overlap each other
-    for (int rc : rcs) if (rc) return rc;
     uint64_t di = 0, nrec = 0, atz = 28, lastend = 0;
     for (auto &r : ctx->streams) {
         r.s.diff_index = di; di += r.s.ndiff;
@@ -1708,6 +1885,7 @@ int atz_search_shard(atz_ctx *ctx, const atz_options *opt, uint32_t shard, uint3
         lastend = r.s.offset + r.span();
     }
     if (lastend < ctx->n) atz += ctx->n - lastend;
+    for (auto &r : ctx->nested) { r.s.diff_index = di; di += r.s.ndiff; }
     ctx->st.n_recomp = nrec;
     ctx->st.algo_bytes += ctx->st.trial_algo_bytes + atz;
     host_mark(ctx->lane[0], 0);
@@ -1744,17 +1922,33 @@ int atz_get_diffs(atz_ctx *ctx, uint64_t *offsets, uint8_t *values, uint64_t cap
     if (!ctx) return ATZ_E_ARG;
     if (ctx->state < 3) return ATZ_E_STATE;
     uint64_t tot = 0; for (auto &r : ctx->streams) tot += r.s.ndiff;
+    for (auto &r : ctx->nested) tot += r.s.ndiff;
     if (n) *n = tot;
     if (cap < tot) return ATZ_E_SMALL;
     uint64_t o = 0;
-    for (auto &r : ctx->streams) for (uint64_t i = 0; i < r.s.ndiff; i++) { offsets[o] = r.diff_off[i]; values[o] = r.diff_val[i]; o++; }
+    for (auto *v : {&ctx->streams, &ctx->nested})
+        for (auto &r : *v) for (uint64_t i = 0; i < r.s.ndiff; i++) { offsets[o] = r.diff_off[i]; values[o] = r.diff_val[i]; o++; }
     return ATZ_OK;
+}
+int atz_get_nested(atz_ctx *ctx, atz_nested *out, uint64_t cap, uint64_t *n) {
+    if (!ctx || !n || (!out && cap)) return ATZ_E_ARG;
+    if (ctx->state < 3) return ATZ_E_STATE;
+    *n = ctx->nested.size();
+    if (cap < ctx->nested.size()) return ATZ_E_SMALL;
+    for (size_t j = 0; j < ctx->nested.size(); j++) { const StreamRec &r = ctx->nested[j]; out[j] = atz_nested{r.parent, r.depth, 0, r.s}; }
+    return ATZ_OK;
+}
+// stream i as atz_get_inflated counts: top-level streams, then the nested ones (nullptr: no such stream)
+static StreamRec *stream_at(atz_ctx *ctx, uint64_t i) {
+    const uint64_t ns = ctx->streams.size();
+    return i < ns ? &ctx->streams[i] : i - ns < ctx->nested.size() ? &ctx->nested[i - ns] : nullptr;
 }
 int atz_get_inflated(atz_ctx *ctx, uint64_t i, uint8_t *dst, uint64_t cap) {
     if (!ctx || !dst) return ATZ_E_ARG;
     if (ctx->state < 2) return ATZ_E_STATE;
-    if (i >= ctx->streams.size()) return ATZ_E_ARG;
-    StreamRec &r = ctx->streams[i];
+    StreamRec *rp = stream_at(ctx, i);
+    if (!rp) return ATZ_E_ARG;
+    StreamRec &r = *rp;
     if (cap < r.s.inflatedLength) return ATZ_E_SMALL;
     if (!r.d_plain) { ctx->set_err("stream is owned by another shard"); return ATZ_E_STATE; }
     cudaSetDevice(ctx->device);
@@ -1763,12 +1957,12 @@ int atz_get_inflated(atz_ctx *ctx, uint64_t i, uint8_t *dst, uint64_t cap) {
     ph.stop();
     return ATZ_OK;
 }
-static int gather_streams(atz_ctx *ctx, const std::vector<size_t> &which, uint8_t *dst, uint64_t tot) {
+static int gather_streams(atz_ctx *ctx, const std::vector<const StreamRec *> &which, uint8_t *dst, uint64_t tot) {
     // the payloads go into one contiguous device buffer (one kernel), then a single D2H copy
     CK(ctx->gather.ensure(tot + 64)); CK(ctx->cjobs.ensure(which.size() * sizeof(CopyJob)));
     std::vector<CopyJob> cj; cj.reserve(which.size());
     uint64_t o = 0;
-    for (size_t i : which) { const StreamRec &r = ctx->streams[i]; cj.push_back(CopyJob{r.d_plain, ctx->gather.as<uint8_t>() + o, r.s.inflatedLength}); o += r.s.inflatedLength; }
+    for (const StreamRec *p : which) { const StreamRec &r = *p; cj.push_back(CopyJob{r.d_plain, ctx->gather.as<uint8_t>() + o, r.s.inflatedLength}); o += r.s.inflatedLength; }
     CK(cudaMemcpyAsync(ctx->cjobs.p, cj.data(), cj.size() * sizeof(CopyJob), cudaMemcpyHostToDevice, ctx->stream));
     Phase ph(ctx, &ctx->st.ms_d2h);
     CK(launch_gather(ctx->cjobs.as<CopyJob>(), (uint32_t)cj.size(), ctx->stream)); ctx->st.kernel_launches++;
@@ -1779,8 +1973,8 @@ static int gather_streams(atz_ctx *ctx, const std::vector<size_t> &which, uint8_
 int atz_get_inflated_recomp(atz_ctx *ctx, uint8_t *dst, uint64_t cap, uint64_t *n) {
     if (!ctx) return ATZ_E_ARG;
     if (ctx->state < 3) return ATZ_E_STATE;
-    uint64_t tot = 0; std::vector<size_t> which;
-    for (size_t i = 0; i < ctx->streams.size(); i++) if (ctx->streams[i].s.recomp && ctx->streams[i].d_plain) { tot += ctx->streams[i].s.inflatedLength; which.push_back(i); }   // (of a sharded run: the ones this context owns)
+    uint64_t tot = 0; std::vector<const StreamRec *> which;
+    for (const StreamRec &r : ctx->streams) if (r.s.recomp && r.d_plain) { tot += r.s.inflatedLength; which.push_back(&r); }   // (of a sharded run: the ones this context owns)
     if (n) *n = tot;
     if (!dst || cap < tot) return ATZ_E_SMALL;
     if (!tot) return ATZ_OK;
@@ -1790,11 +1984,12 @@ int atz_get_inflated_recomp(atz_ctx *ctx, uint8_t *dst, uint64_t cap, uint64_t *
 int atz_get_inflated_list(atz_ctx *ctx, const uint64_t *indices, uint64_t count, uint8_t *dst, uint64_t cap, uint64_t *n) {
     if (!ctx || (!indices && count)) return ATZ_E_ARG;
     if (ctx->state < 2) return ATZ_E_STATE;
-    uint64_t tot = 0; std::vector<size_t> which;
+    uint64_t tot = 0; std::vector<const StreamRec *> which;
     for (uint64_t k = 0; k < count; k++) {
-        if (indices[k] >= ctx->streams.size()) return ATZ_E_ARG;
-        if (!ctx->streams[indices[k]].d_plain) { ctx->set_err("stream is owned by another shard"); return ATZ_E_STATE; }
-        tot += ctx->streams[indices[k]].s.inflatedLength; which.push_back((size_t)indices[k]);
+        const StreamRec *r = stream_at(ctx, indices[k]);
+        if (!r) return ATZ_E_ARG;
+        if (!r->d_plain) { ctx->set_err("stream is owned by another shard"); return ATZ_E_STATE; }
+        tot += r->s.inflatedLength; which.push_back(r);
     }
     if (n) *n = tot;
     if (!dst || cap < tot) return ATZ_E_SMALL;

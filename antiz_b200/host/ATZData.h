@@ -28,6 +28,7 @@ struct programOptions {
     bool strategies = false;             // ATZ_F_STRATEGIES: also try zlib's other strategies (changes the ATZ file vs the reference)
     bool smallWindows = false;           // ATZ_SCAN_SMALL_WINDOWS: also accept CINFO 0 and 1 headers (the reference can still reconstruct)
     bool png = false;                    // ATZ_SCAN_PNG_IDAT: also find zlib streams split over PNG IDAT chunks (changes the ATZ file vs the reference)
+    int nested = 0;                      // ATZ_F_NESTED_DEPTH: also recompress zlib streams inside recompressed ones, this many levels deep (changes the ATZ file vs the reference)
 };
 
 struct zlibParamPack {

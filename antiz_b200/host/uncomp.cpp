@@ -6,7 +6,7 @@
 // same built-in self test (testATZfile main.cpp:1173-1203).  The host keeps what the reference's L1/L2 layers do
 // (CLI, file IO, ATZ1 layout, phase order); phases 1 and 3 and the per-stream deflate of the reconstructor run on
 // the GPU.  Extensions: --gpus N (static shard of the stream x parameter grid), --device D, --exact-records, --stats, --strategies,
-// --small-windows, --png.
+// --small-windows, --png, --nested.
 #include "ATZData.h"
 #include "antiz_b200.h"
 #include <chrono>
@@ -148,6 +148,7 @@ class ATZcreator {
         atz_options o{};
         o.recompTresh = options.recompTresh; o.sizediffTresh = options.sizediffTresh; o.shortcutLength = options.shortcutLength;
         o.mismatchTol = options.mismatchTol; o.bruteforceWindow = options.bruteforceWindow; o.flags = (options.exactRecords ? ATZ_F_EXACT_RECORDS : 0) | (options.strategies ? ATZ_F_STRATEGIES : 0);
+        o.flags |= ATZ_F_NESTED_DEPTH(options.nested);
         int ng = (int)ctxs.size();
         std::vector<int> rcs(ng, 0);
         auto work = [&](int g) { rcs[g] = atz_search_shard(ctxs[g], &o, (uint32_t)g, (uint32_t)ng); };
@@ -182,8 +183,33 @@ class ATZcreator {
             }
             streams.push_back(std::move(s));
         }
+        // nested streams (--nested): each context lists the ones under the streams it owns; their parent indices are turned into the
+        // tree below (kids[i] for top-level stream i, nests[k].kids for nested stream k, in offset order)
+        kids.assign(nstreams, {}); nests.clear();
+        for (int g = 0; g < ng && options.nested; g++) {
+            uint64_t nn = 0; atz_get_nested(ctxs[g], nullptr, 0, &nn);
+            std::vector<atz_nested> v(nn ? nn : 1);
+            if (nn && atz_get_nested(ctxs[g], v.data(), nn, &nn) != ATZ_OK) { std::cout << atz_err(ctxs[g], -1) << std::endl; abort(); }
+            const size_t base = nests.size();
+            for (uint64_t j = 0; j < nn; j++) {
+                const atz_stream &a = v[j].s;
+                Nest n{ATZdata::streamOffset(a.offset, a.offsetType, a.streamLength, a.inflatedLength), g, nstreams + j, {}, {}};
+                n.s.zlibparams = ATZdata::zlibParamPack(a.clevel, a.window, a.memlevel);
+                n.s.identBytes = a.identBytes; n.s.firstDiffByte = a.firstDiffByte; n.s.recomp = a.recomp != 0;
+                n.s.diffByteOffsets.assign(doff[g].begin() + a.diff_index, doff[g].begin() + a.diff_index + a.ndiff);
+                n.s.diffByteVal.assign(dval[g].begin() + a.diff_index, dval[g].begin() + a.diff_index + a.ndiff);
+                nests.push_back(std::move(n));
+                const uint64_t p = v[j].parent;
+                if (p < nstreams) kids[p].push_back(base + j);
+                else nests[base + (p - nstreams)].kids.push_back(base + j);
+            }
+        }
         std::cout << std::endl;
         std::cout << "recompressed:" << countRecomp() << "/" << streams.size() << std::endl;
+        if (options.nested) {
+            uint64_t nr = 0; for (auto &n : nests) nr += n.s.recomp;
+            std::cout << "nested recompressed:" << nr << "/" << nests.size() << std::endl;
+        }
         processingState = 3;
         return 0;
     }
@@ -205,12 +231,39 @@ class ATZcreator {
     std::vector<atz_ctx *> ctxs;
     std::vector<uint32_t> owner;   // shard that holds stream i's record and plaintext
     std::vector<ATZdata::streamOffset> streams;
+    struct Nest { ATZdata::streamOffset s; int g; uint64_t idx; std::vector<size_t> kids; std::vector<uint8_t> plain; };   // g: context, idx: its atz_get_inflated index
+    std::vector<Nest> nests; std::vector<std::vector<size_t>> kids;
 
     uint64_t countRecomp() { uint64_t n = 0; for (auto &s : streams) if (s.recomp) n++; return n; }
 
     // ATZ1 layout (main.cpp:775-831): header, per recompressed stream {descriptor, diffs, inflated data}, residue.  A stream split over
     // PNG IDAT chunks (--png) has bit 7 of its window byte set and, behind the diffs, u64 npieces, npieces u32 piece lengths and the
     // (npieces - 1) x 12 framing bytes between the pieces, copied from the input (its CRCs stay exact even where they are wrong).
+    // A stream with recompressed nested streams (--nested) has bit 6 of its window byte set, and its payload P is replaced by u64 nchild,
+    // the records of those nchild streams in offset order (the same layout, recursively; never bit 7) and P without their bytes.
+    static bool any_recomp(const std::vector<Nest> &ns, const std::vector<size_t> &k) { for (size_t i : k) if (ns[i].s.recomp) return true; return false; }
+    void put_payload(std::vector<uint8_t> &out, const uint8_t *P, uint64_t U, const std::vector<size_t> &k) {
+        if (!any_recomp(nests, k)) { out.insert(out.end(), P, P + U); return; }
+        uint64_t nc = 0; for (size_t i : k) nc += nests[i].s.recomp;
+        put8(out, nc);
+        for (size_t i : k) {
+            const Nest &n = nests[i]; const auto &s = n.s;
+            if (!s.recomp) continue;
+            put8(out, s.offset); put8(out, s.streamLength); put8(out, s.inflatedLength);
+            out.push_back(s.zlibparams.clevel); out.push_back(s.zlibparams.window | (any_recomp(nests, n.kids) ? 0x40 : 0)); out.push_back(s.zlibparams.memlevel);
+            const uint64_t nd = s.diffByteOffsets.size();
+            put8(out, nd);
+            if (nd > 0) {
+                put8(out, (uint64_t)s.firstDiffByte);
+                for (uint64_t q = 0; q < nd; q++) put8(out, s.diffByteOffsets[q]);
+                for (uint64_t q = 0; q < nd; q++) out.push_back(s.diffByteVal[q]);
+            }
+            put_payload(out, n.plain.data(), s.inflatedLength, n.kids);
+        }
+        uint64_t at = 0;    // the residue
+        for (size_t i : k) if (nests[i].s.recomp) { out.insert(out.end(), P + at, P + nests[i].s.offset); at = nests[i].s.offset + nests[i].s.streamLength; }
+        out.insert(out.end(), P + at, P + U);
+    }
     void writeATZfile() {
         uint64_t total = 28, nrec = countRecomp();
         for (auto &s : streams) if (s.recomp) total += 35 + (s.diffByteOffsets.empty() ? 0 : 8 + 9 * s.diffByteOffsets.size()) + s.inflatedLength + (s.pieces.empty() ? 0 : 8 + 16 * s.pieces.size() - 12);
@@ -234,12 +287,23 @@ class ATZcreator {
             fetch(0);
             for (auto &t : th) t.join();
             for (int g = 0; g < ng; g++) if (rcs[g] != ATZ_OK || got[g] != (which[g].empty() ? 0 : paybytes[g])) { std::cout << atz_err(ctxs[g], rcs[g]) << std::endl; abort(); }
+            // the plaintext of the recompressed nested streams, from the context that found them
+            for (int g = 0; g < ng && !nests.empty(); g++) {
+                std::vector<uint64_t> idx; std::vector<size_t> at; uint64_t tot = 0, got2 = 0;
+                for (size_t i = 0; i < nests.size(); i++) if (nests[i].g == g && nests[i].s.recomp) { idx.push_back(nests[i].idx); at.push_back(i); tot += nests[i].s.inflatedLength; }
+                if (idx.empty()) continue;
+                std::vector<uint8_t> buf(tot ? tot : 1);
+                const int rc = atz_get_inflated_list(ctxs[g], idx.data(), idx.size(), buf.data(), tot, &got2);
+                if (rc != ATZ_OK || got2 != tot) { std::cout << atz_err(ctxs[g], rc) << std::endl; abort(); }
+                uint64_t o = 0;
+                for (size_t i : at) { nests[i].plain.assign(buf.begin() + o, buf.begin() + o + nests[i].s.inflatedLength); o += nests[i].s.inflatedLength; }
+            }
         }
         for (uint64_t i = 0; i < streams.size(); i++) {
             auto &s = streams[i];
             if (!s.recomp) continue;
             put8(out, s.offset); put8(out, s.streamLength); put8(out, s.inflatedLength);
-            out.push_back(s.zlibparams.clevel); out.push_back(s.zlibparams.window | (s.pieces.empty() ? 0 : 0x80)); out.push_back(s.zlibparams.memlevel);
+            out.push_back(s.zlibparams.clevel); out.push_back(s.zlibparams.window | (s.pieces.empty() ? 0 : 0x80) | (any_recomp(nests, kids[i]) ? 0x40 : 0)); out.push_back(s.zlibparams.memlevel);
             uint64_t nd = s.diffByteOffsets.size();
             put8(out, nd);
             if (nd > 0) {
@@ -254,7 +318,7 @@ class ATZcreator {
                 for (size_t k = 0; k + 1 < s.pieces.size(); k++) { at += s.pieces[k]; out.insert(out.end(), file.begin() + at, file.begin() + at + 12); at += 12; }
             }
             const uint32_t g = owner[i];
-            out.insert(out.end(), payload[g].begin() + pay_at[g], payload[g].begin() + pay_at[g] + s.inflatedLength); pay_at[g] += s.inflatedLength;
+            put_payload(out, payload[g].data() + pay_at[g], s.inflatedLength, kids[i]); pay_at[g] += s.inflatedLength;
         }
         uint64_t lastos = 0, lastlen = 0;   // residue: gaps, non-recompressed streams, tail (main.cpp:784-796)
         for (auto &s : streams) {
@@ -321,6 +385,7 @@ class ATZreconstructor {
             gaps += origlen - end;
             if (residueos > atzfileSize || gaps > atzfileSize - residueos) return invalid("residue exceeds the ATZ file");
         }
+        if (!nodes.empty() && rebuildNested(ctx, atz, list) != ATZ_OK) abort();
         std::vector<uint64_t> in_off(n), in_len(n), out_off(n), out_cap(n), out_len(n);
         std::vector<uint8_t> cl(n), wb(n), ml(n);
         uint64_t oo = 0;
@@ -372,6 +437,9 @@ class ATZreconstructor {
 
   private:
     std::string atzfileName, reconfileName; int dev;
+    struct Tree { std::vector<size_t> kids; uint64_t residueAt = 0; };   // a record's nested streams (indices into nodes) and where its residue starts
+    struct Node { ATZdata::streamOffset s; Tree t; int depth; };
+    std::vector<Tree> tops; std::vector<Node> nodes;
     int parseATZheader(std::vector<uint8_t> &atz, uint64_t &origlen, uint64_t &nstrms) {   // main.cpp:1011-1030
         uint64_t infileSize = 0;
         if (getFilesize(atzfileName, infileSize) != 0) return -1;
@@ -383,47 +451,135 @@ class ATZreconstructor {
     }
     uint64_t readStreamdesc_ALL(const std::vector<uint8_t> &atz, std::vector<ATZdata::streamOffset> &list, uint64_t nstrms, uint64_t origlen) {   // main.cpp:1031-1063
         uint64_t lastos = 28;
-        auto need = [&](uint64_t end) { if (end > atz.size()) { std::cout << "Invalid file: truncated stream description" << std::endl; std::exit(1); } };
-        auto invalid = [](const char *what) { std::cout << "Invalid file: " << what << std::endl; std::exit(1); };
+        tops.assign(nstrms, Tree());
         for (uint64_t j = 0; j < nstrms; j++) {
-            need(lastos + 35);
-            list.push_back(ATZdata::streamOffset(get8(&atz[lastos]), -1, get8(&atz[lastos + 8]), get8(&atz[lastos + 16])));
-            auto &s = list[j];
-            s.zlibparams.clevel = atz[lastos + 24]; s.zlibparams.window = atz[lastos + 25]; s.zlibparams.memlevel = atz[lastos + 26];
-            uint64_t diffbytes = get8(&atz[lastos + 27]);
-            if (diffbytes > 0) {
-                if (diffbytes > (atz.size() - lastos) / 9) need(atz.size() + 1);   // (the multiplication below cannot wrap)
-                need(lastos + 43 + diffbytes * 9);
-                s.firstDiffByte = (int_fast64_t)get8(&atz[lastos + 35]);
-                for (uint64_t i = 0; i < diffbytes; i++) {
-                    s.diffByteOffsets.push_back(get8(&atz[43 + 8 * i + lastos]));
-                    s.diffByteVal.push_back(atz[43 + diffbytes * 8 + i + lastos]);
-                }
-                s.atzInfos = 43 + diffbytes * 9 + lastos;
-            } else {
-                s.firstDiffByte = -1;
-                s.atzInfos = 35 + lastos;
-            }
-            if (s.zlibparams.window & 0x80) {   // split over PNG IDAT chunks (--png): piece table and framing bytes, checked before any GPU work
-                s.zlibparams.window &= 0x7f;
-                if (s.zlibparams.window < 9 || s.zlibparams.window > 15) invalid("bad window of a split stream");
-                need(s.atzInfos + 8);
-                const uint64_t np = get8(&atz[s.atzInfos]);
-                if (np < 2) invalid("a split stream needs at least 2 pieces");
-                if (np > (atz.size() - s.atzInfos - 8) / 16 + 1) need(atz.size() + 1);   // (the sizes below cannot wrap)
-                need(s.atzInfos + 8 + 16 * np - 12);
-                uint64_t sum = 0;
-                for (uint64_t k = 0; k < np; k++) { uint32_t l; std::memcpy(&l, &atz[s.atzInfos + 8 + 4 * k], 4); s.pieces.push_back(l); sum += l; }
-                if (sum != s.streamLength) invalid("piece lengths of a split stream do not sum to its length");
-                if (s.offset > origlen || s.spanLength() > origlen - s.offset) invalid("split stream outside the original file");
-                s.gapsAt = s.atzInfos + 8 + 4 * np;
-                s.atzInfos += 8 + 16 * np - 12;
-            }
-            lastos = s.atzInfos + s.inflatedLength;
-            if (s.inflatedLength > atz.size()) need(atz.size() + 1);
-            need(lastos);
+            list.push_back(ATZdata::streamOffset(0, -1, 0, 0));
+            lastos = readRecord(atz, lastos, origlen, 0, list[j], tops[j]);
         }
         return lastos;
+    }
+    // One record at `lastos`: descriptor, diffs, (window bit 7, --png) the piece table and framing bytes, then the payload or (bit 6,
+    // --nested) u64 nchild, the nested records and the residue.  depth 0 = a top-level record.  Returns the end of the record.
+    uint64_t readRecord(const std::vector<uint8_t> &atz, uint64_t lastos, uint64_t origlen, int depth, ATZdata::streamOffset &s, Tree &t) {
+        auto need = [&](uint64_t end) { if (end > atz.size()) { std::cout << "Invalid file: truncated stream description" << std::endl; std::exit(1); } };
+        auto invalid = [](const char *what) { std::cout << "Invalid file: " << what << std::endl; std::exit(1); };
+        need(lastos + 35);
+        s = ATZdata::streamOffset(get8(&atz[lastos]), -1, get8(&atz[lastos + 8]), get8(&atz[lastos + 16]));
+        s.zlibparams.clevel = atz[lastos + 24]; s.zlibparams.window = atz[lastos + 25]; s.zlibparams.memlevel = atz[lastos + 26];
+        uint64_t diffbytes = get8(&atz[lastos + 27]);
+        if (diffbytes > 0) {
+            if (diffbytes > (atz.size() - lastos) / 9) need(atz.size() + 1);   // (the multiplication below cannot wrap)
+            need(lastos + 43 + diffbytes * 9);
+            s.firstDiffByte = (int_fast64_t)get8(&atz[lastos + 35]);
+            for (uint64_t i = 0; i < diffbytes; i++) {
+                s.diffByteOffsets.push_back(get8(&atz[43 + 8 * i + lastos]));
+                s.diffByteVal.push_back(atz[43 + diffbytes * 8 + i + lastos]);
+            }
+            s.atzInfos = 43 + diffbytes * 9 + lastos;
+        } else {
+            s.firstDiffByte = -1;
+            s.atzInfos = 35 + lastos;
+        }
+        const bool has_nested = s.zlibparams.window & 0x40;
+        s.zlibparams.window &= 0xbf;
+        if (depth > 0) {
+            if (s.zlibparams.window & 0x80) invalid("a nested stream cannot be split over IDAT chunks");
+            if ((s.zlibparams.clevel & 15) > 9 || (s.zlibparams.clevel >> 4) > 4 || s.zlibparams.window < 9 || s.zlibparams.window > 15 || s.zlibparams.memlevel < 1 || s.zlibparams.memlevel > 9) invalid("bad zlib parameters");
+            if (s.streamLength >= 0xffff0000ull || s.inflatedLength >= 0xffffff00ull) invalid("stream too large");
+        }
+        if (s.zlibparams.window & 0x80) {   // split over PNG IDAT chunks (--png): piece table and framing bytes, checked before any GPU work
+            s.zlibparams.window &= 0x7f;
+            if (s.zlibparams.window < 9 || s.zlibparams.window > 15) invalid("bad window of a split stream");
+            need(s.atzInfos + 8);
+            const uint64_t np = get8(&atz[s.atzInfos]);
+            if (np < 2) invalid("a split stream needs at least 2 pieces");
+            if (np > (atz.size() - s.atzInfos - 8) / 16 + 1) need(atz.size() + 1);   // (the sizes below cannot wrap)
+            need(s.atzInfos + 8 + 16 * np - 12);
+            uint64_t sum = 0;
+            for (uint64_t k = 0; k < np; k++) { uint32_t l; std::memcpy(&l, &atz[s.atzInfos + 8 + 4 * k], 4); s.pieces.push_back(l); sum += l; }
+            if (sum != s.streamLength) invalid("piece lengths of a split stream do not sum to its length");
+            if (s.offset > origlen || s.spanLength() > origlen - s.offset) invalid("split stream outside the original file");
+            s.gapsAt = s.atzInfos + 8 + 4 * np;
+            s.atzInfos += 8 + 16 * np - 12;
+        }
+        if (s.inflatedLength > atz.size()) need(atz.size() + 1);
+        if (!has_nested) {
+            lastos = s.atzInfos + s.inflatedLength;
+            need(lastos);
+            return lastos;
+        }
+        // nested records: ascending, disjoint, inside [0, U) of this plaintext; the residue is U minus their compressed bytes
+        if (depth >= 8) invalid("streams nested deeper than 8 levels");
+        need(s.atzInfos + 8);
+        const uint64_t nchild = get8(&atz[s.atzInfos]);
+        if (nchild == 0) invalid("a stream marked as holding nested streams has none");
+        if (nchild > (atz.size() - s.atzInfos - 8) / 35) need(atz.size() + 1);
+        uint64_t pos = s.atzInfos + 8, end = 0, sumc = 0;
+        for (uint64_t k = 0; k < nchild; k++) {
+            ATZdata::streamOffset c(0, -1, 0, 0); Tree ct;
+            pos = readRecord(atz, pos, origlen, depth + 1, c, ct);
+            if (c.offset < end || c.offset >= s.inflatedLength || c.streamLength > s.inflatedLength - c.offset) invalid("nested streams out of order or outside their parent's plaintext");
+            end = c.offset + c.streamLength; sumc += c.streamLength;
+            nodes.push_back(Node{std::move(c), std::move(ct), depth + 1});
+            t.kids.push_back(nodes.size() - 1);
+        }
+        t.residueAt = pos;
+        lastos = pos + (s.inflatedLength - sumc);
+        need(lastos);
+        return lastos;
+    }
+    // --nested: the plaintext of every stream with nested streams, deepest level first: the level's streams are deflated in one batch and
+    // patched, then each parent's plaintext is put together from its residue and its children's bytes and appended to `atz`, where the
+    // parent's atzInfos then points
+    int rebuildNested(atz_ctx *ctx, std::vector<uint8_t> &atz, std::vector<ATZdata::streamOffset> &list) {
+        int maxd = 0;
+        for (const Node &n : nodes) maxd = std::max(maxd, n.depth);
+        std::vector<std::vector<uint8_t>> comp(nodes.size());
+        for (int d = maxd; d >= 1; d--) {
+            std::vector<size_t> lv;
+            for (size_t i = 0; i < nodes.size(); i++) if (nodes[i].depth == d) lv.push_back(i);
+            const uint64_t n = lv.size();
+            std::vector<uint64_t> in_off(n), in_len(n), out_off(n), out_cap(n), out_len(n);
+            std::vector<uint8_t> cl(n), wb(n), ml(n);
+            uint64_t oo = 0;
+            for (uint64_t j = 0; j < n; j++) {
+                const auto &s = nodes[lv[j]].s;
+                in_off[j] = s.atzInfos; in_len[j] = s.inflatedLength;
+                out_off[j] = oo; out_cap[j] = s.streamLength + 65535; oo += out_cap[j];
+                cl[j] = s.zlibparams.clevel; wb[j] = s.zlibparams.window; ml[j] = s.zlibparams.memlevel;
+            }
+            std::vector<uint8_t> out(oo ? oo : 1);
+            const int rc = atz_deflate_batch(ctx, atz.data(), in_off.data(), in_len.data(), cl.data(), wb.data(), ml.data(), n, out.data(), out_off.data(), out_cap.data(), out_len.data());
+            if (rc != ATZ_OK) { std::cout << "deflate() failed with exit code:" << rc << " " << atz_last_error(ctx) << std::endl; return rc; }
+            for (uint64_t j = 0; j < n; j++) {
+                const auto &s = nodes[lv[j]].s;
+                uint8_t *cb = out.data() + out_off[j];
+                if (s.firstDiffByte >= 0) {
+                    uint64_t sum = 0;
+                    for (uint64_t i = 0; i < s.diffByteOffsets.size(); i++) {
+                        const uint64_t pos = (uint64_t)s.firstDiffByte + s.diffByteOffsets[i] + sum;
+                        if (pos < out_cap[j]) cb[pos] = s.diffByteVal[i];
+                        sum += s.diffByteOffsets[i];
+                    }
+                }
+                comp[lv[j]].assign(cb, cb + s.streamLength);
+            }
+            auto splice = [&](ATZdata::streamOffset &s, const Tree &t) {
+                std::vector<uint8_t> P; P.reserve(s.inflatedLength);
+                uint64_t res = t.residueAt, at = 0;
+                for (size_t k : t.kids) {
+                    const auto &c = nodes[k].s;
+                    P.insert(P.end(), atz.begin() + res, atz.begin() + res + (c.offset - at)); res += c.offset - at;
+                    P.insert(P.end(), comp[k].begin(), comp[k].end()); at = c.offset + c.streamLength;
+                }
+                P.insert(P.end(), atz.begin() + res, atz.begin() + res + (s.inflatedLength - at));
+                s.atzInfos = atz.size();
+                atz.insert(atz.end(), P.begin(), P.end());
+            };
+            for (Node &p : nodes) if (p.depth == d - 1 && !p.t.kids.empty()) splice(p.s, p.t);
+            if (d == 1) for (size_t j = 0; j < list.size(); j++) if (!tops[j].kids.empty()) splice(list[j], tops[j]);
+        }
+        return ATZ_OK;
     }
 };
 
@@ -455,6 +611,7 @@ static const CliArg kExtArgs[] = {   // antiz_b200 only: listed after the refere
     {"", "strategies", nullptr, false, "For streams that no plain parameter set reproduces, also try zlib's other strategies (Z_FILTERED, Z_FIXED, Z_RLE, Z_HUFFMAN_ONLY). More streams are recompressed, but the ATZ file then differs from the reference's and only this program can reconstruct from it. Default: disabled"},
     {"", "small-windows", nullptr, false, "Also look for zlib streams with 256- and 512-byte windows (header bytes 0x08 and 0x18). More streams are found and recompressed, so the ATZ file differs from the reference's, but the reference can still reconstruct from it. Default: disabled"},
     {"", "png", nullptr, false, "Also find zlib streams that PNG files split over consecutive IDAT chunks, and recompress them with the chunk framing between the pieces stored verbatim. The ATZ file then differs from the reference's and only this program can reconstruct from it. Default: disabled"},
+    {"", "nested", "integer", false, "Also recompress zlib streams found inside the decompressed data of recompressed streams, down to this many levels (0-8). The ATZ file then differs from the reference's and only this program can reconstruct from it. Default: 0"},
 };
 static std::string cli_short_id(const CliArg &a) {
     std::string id = a.flag[0] ? std::string("-") + a.flag : std::string("--") + a.name;
@@ -565,11 +722,13 @@ static void parseCLI(int argc, char *argv[], std::string &infile_name, std::stri
         else if (n == "strategies") options.strategies = true;
         else if (n == "small-windows") options.smallWindows = true;
         else if (n == "png") options.png = true;
+        else if (n == "nested") options.nested = (int)std::min<uint64_t>(x, 9);
         else if (n == "help") { usage(argv[0]); std::exit(0); }
         else if (n == "version") { std::cout << std::endl << argv[0] << "  version: " << antiz_ver << std::endl << std::endl; std::exit(0); }
     }
     if (!in_set) parse_error(argv[0], "Required argument missing: input", "");
     if (options.chunksize < 2) parse_error(argv[0], "chunksize must be at least 2", "(--chunksize)");
+    if (options.nested > 8) parse_error(argv[0], "nested depth must be at most 8", "(--nested)");
     std::cout << "Input file: " << in << std::endl;
     if (options.recon) {   // main.cpp:1118-1127
         std::cout << "assuming input file is an ATZ file, attempting to reconstruct" << std::endl;

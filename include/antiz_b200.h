@@ -58,6 +58,16 @@ typedef struct {
 /* `clevel` bytes (atz_stream.clevel, atz_deflate_stream / _batch / atz_trial arguments): level 0..9 in the low nibble, zlib strategy
  * 0..4 in bits 4-6 (0 = Z_DEFAULT_STRATEGY: plain levels are unchanged). */
 #define ATZ_CLEVEL(level, strategy) ((uint8_t)((level) | ((strategy) << 4)))
+/* Extension (SURVEY.md 8 f4; not in the reference): also recompress zlib streams inside the plaintext of recompressed streams, down to
+ * `depth` levels (0..8; 0 = off; ATZ_E_ARG above 8).  After the level-d streams have been searched (d = 0: the file's), the plaintext P
+ * of every recompressed level-d stream this context owns is walked ascending: at a position p where (P[p], P[p+1]) is a header of the
+ * context's scan set (ATZ_SCAN_SMALL_WINDOWS counts; IDAT runs are not looked for), P[p:] is inflated with its input cut at the end of
+ * P; a stream that ends there with a correct adler32 after more than 16 bytes (C) is accepted and the walk goes on at p + C, otherwise at
+ * p + 1.  The level-(d+1) streams are searched like top-level ones (same candidate sequences, --brute-window, strategies, thresholds,
+ * diff lists) and belong to their parent's owner; atz_get_nested returns them.  Stats n_streams / n_recomp stay top-level; ref_trials
+ * and gpu_trials include the nested trials.  Carried in atz_options.flags, bits 8 and up, so that atz_options keeps its layout; any value
+ * of those bits above 8 (a negative flags word too) is ATZ_E_ARG. */
+#define ATZ_F_NESTED_DEPTH(d) ((d) << 8)
 
 /* ATZdata::streamOffset (ATZData.h:42-77), flattened. */
 typedef struct {
@@ -160,6 +170,11 @@ int atz_search(atz_ctx *ctx, const atz_options *opt);
  * The host gathers stream i's record from the context that owns it. */
 int atz_search_shard(atz_ctx *ctx, const atz_options *opt, uint32_t shard, uint32_t nshards);
 
+/* A stream found inside the plaintext of another (ATZ_F_NESTED_DEPTH).  parent < n_streams: the top-level stream `parent`; otherwise
+ * entry parent - n_streams of the same atz_get_nested list (always an earlier one).  depth: 1 under a top-level stream, 2 under a
+ * depth-1 stream, ...  s.offset is relative to the start of the parent's plaintext; s.diff_index points into atz_get_diffs' arrays. */
+typedef struct { uint64_t parent; uint32_t depth; uint32_t reserved; atz_stream s; } atz_nested;
+
 /* Results.  `streams` must have room for n_streams entries. */
 int atz_get_streams(atz_ctx *ctx, atz_stream *streams, uint64_t cap);
 /* owner[i] = shard that owns stream i: set by atz_scan_finish (sharded scan) or by the last atz_search_shard (0 before that).  The
@@ -169,13 +184,18 @@ int atz_get_owners(atz_ctx *ctx, uint32_t *owner, uint64_t cap);
  * lengths (summing to streamLength; piece k+1 starts 12 bytes after piece k ends) go to len[0 .. min(npieces, cap)).  ATZ_E_SMALL if
  * cap < npieces.  Every context of a sharded run reports the same pieces. */
 int atz_get_pieces(atz_ctx *ctx, uint64_t stream_index, uint32_t *len, uint64_t cap, uint64_t *npieces);
-/* diffByteOffsets (delta-encoded, main.cpp:757-763) and diffByteVal of all recomp streams, concatenated. */
+/* diffByteOffsets (delta-encoded, main.cpp:757-763) and diffByteVal of all recomp streams, concatenated: the top-level streams', then
+ * those of the nested streams (atz_get_nested order). */
 int atz_get_diffs(atz_ctx *ctx, uint64_t *offsets, uint8_t *values, uint64_t cap, uint64_t *n);
-/* Inflated payload of stream i (what writeStreamdesc re-inflates, main.cpp:824-828). */
+/* The nested streams the last search found under the streams this context owns, recompressed or not (ATZ_F_NESTED_DEPTH): level by
+ * level, then by parent, then by offset.  *n receives their number; ATZ_E_SMALL if cap is smaller. */
+int atz_get_nested(atz_ctx *ctx, atz_nested *out, uint64_t cap, uint64_t *n);
+/* Inflated payload of stream i (what writeStreamdesc re-inflates, main.cpp:824-828); i = n_streams + j is nested entry j. */
 int atz_get_inflated(atz_ctx *ctx, uint64_t stream_index, uint8_t *dst, uint64_t cap);
 /* All payloads of recomp streams (of a sharded run: the ones this context owns), concatenated in stream order, into one host buffer (one D2H). */
 int atz_get_inflated_recomp(atz_ctx *ctx, uint8_t *dst, uint64_t cap, uint64_t *n);
-/* The payloads of the given streams, concatenated in the given order (ATZ_E_STATE for a stream another shard owns). */
+/* The payloads of the given streams (indices as atz_get_inflated takes them), concatenated in the given order (ATZ_E_STATE for a stream
+ * another shard owns). */
 int atz_get_inflated_list(atz_ctx *ctx, const uint64_t *indices, uint64_t count, uint8_t *dst, uint64_t cap, uint64_t *n);
 int atz_get_stats(atz_ctx *ctx, atz_stats *st);
 /* CUDA-event stopwatch on the context's stream (the stream every kernel of this library is launched on):

@@ -75,6 +75,22 @@ static const struct { uint16_t good, lazy, nice, chain; uint8_t kind; } CFG[10] 
 
 typedef struct { uint16_t fc; uint16_t dl; } node_t; /* freq|code, dad|len as in ct_data */
 
+/* Branch counters of the block flush (tests only: they write nothing into the output).  oracle_flush_counts() reads and resets them. */
+enum { FC_OVER_L, FC_OVER_D, FC_OVER_B,                                  /* gen_bitlen depth-limit repair, per tree kind */
+       FC_FORCE_L_LOW, FC_FORCE_L_HIGH, FC_FORCE_D_LOW, FC_FORCE_D_HIGH,  /* heap_len < 2 forcing, max_code < 2 / >= 2 */
+       FC_FORCE_B_LOW, FC_FORCE_B_HIGH,
+       FC_STORED, FC_STATIC, FC_DYNAMIC, FC_UNSTORABLE,                   /* block kinds; flushes with buf == NULL after a slide */
+       FC_TIE_STORED, FC_TIE_STATIC,                                      /* stored_len + 4 == opt_lenb; static_lenb == opt_lenb == opt_len */
+       FC_REP16_6, FC_REP17_3, FC_REP17_10, FC_REP18_11, FC_REP18_138,   /* scan_tree runs at the limits of their codes */
+       FC_ZRUN_SPLIT,                                                     /* a run of more than 138 zero lengths, split */
+       FC_N };
+static uint64_t g_fc[FC_N];
+int oracle_flush_counts(uint64_t *out, int n) {
+    if (out) for (int i = 0; i < n && i < FC_N; i++) out[i] = g_fc[i];
+    memset(g_fc, 0, sizeof g_fc);
+    return FC_N;
+}
+
 typedef struct {
     const uint8_t *in; uint32_t in_len, in_pos;
     uint8_t *out; uint64_t out_cap, out_len; int overflow;
@@ -105,6 +121,7 @@ static void putbits(zd_t *s, unsigned v, int n) { /* LSB-first packing == Z/tree
 static void align_byte(zd_t *s) { if (s->bitcnt > 0) { put8(s, (unsigned)(s->bitbuf & 0xff)); } s->bitbuf = 0; s->bitcnt = 0; } /* bi_windup Z/trees.c:1186 */
 
 /* ---- Huffman construction: Z/trees.c:451-699 ---- */
+static int tree_kind(zd_t *s, node_t *t) { return t == s->lt ? 0 : t == s->dt ? 1 : 2; }
 #define LESS(t, n, m) ((t)[n].fc < (t)[m].fc || ((t)[n].fc == (t)[m].fc && s->depth[n] <= s->depth[m]))
 static void sift(zd_t *s, node_t *t, int k) { /* pqdownheap Z/trees.c:451-478 */
     int v = s->heap[k], j = k << 1;
@@ -130,6 +147,7 @@ static void bit_lengths(zd_t *s, node_t *t, int max_code, const uint8_t *st_len,
         if (st_len) s->static_len += (long)t[n].fc * (st_len[n] + xb);
     }
     if (!over) return;
+    g_fc[FC_OVER_L + tree_kind(s, t)]++;
     do {
         int bits = maxlen - 1;
         while (s->blcount[bits] == 0) bits--;
@@ -157,6 +175,7 @@ static int make_tree(zd_t *s, node_t *t, int elems, const uint8_t *st_len, const
     for (n = 0; n < elems; n++) {
         if (t[n].fc != 0) { s->heap[++s->heap_len] = max_code = n; s->depth[n] = 0; } else t[n].dl = 0;
     }
+    if (s->heap_len < 2) g_fc[FC_FORCE_L_LOW + 2 * tree_kind(s, t) + (max_code >= 2)]++;
     while (s->heap_len < 2) { /* force two codes, Z/trees.c:648-654 */
         int nn = s->heap[++s->heap_len] = (max_code < 2 ? ++max_code : 0);
         t[nn].fc = 1; s->depth[nn] = 0; s->opt_len--; if (st_len) s->static_len -= st_len[nn];
@@ -184,6 +203,11 @@ static void walk_lengths(zd_t *s, node_t *t, int max_code, int emit) {
     for (int n = 0; n <= max_code; n++) {
         int cur = nextlen; nextlen = t[n + 1].dl;
         if (++count < maxc && cur == nextlen) continue;
+        if (!emit && count >= minc) {
+            if (cur != 0) g_fc[FC_REP16_6] += count - (cur != prevlen) == 6;
+            else if (count <= 10) { g_fc[FC_REP17_3] += count == 3; g_fc[FC_REP17_10] += count == 10; }
+            else { g_fc[FC_REP18_11] += count == 11; g_fc[FC_REP18_138] += count == 138; g_fc[FC_ZRUN_SPLIT] += count == 138 && nextlen == 0; }
+        }
         if (count < minc) {
             if (emit) { do putbits(s, s->bt[cur].fc, s->bt[cur].dl); while (--count != 0); } else s->bt[cur].fc += (uint16_t)count;
         } else if (cur != 0) {
@@ -231,14 +255,20 @@ static void flush_block(zd_t *s, int last) {
         s->opt_len += 3 * (max_bl + 1) + 5 + 5 + 4;
         opt_lenb = (unsigned long)(s->opt_len + 3 + 7) >> 3; static_lenb = (unsigned long)(s->static_len + 3 + 7) >> 3;
         if (static_lenb <= opt_lenb) opt_lenb = static_lenb;
+        if (stored_len + 4 == opt_lenb && buf != NULL) g_fc[FC_TIE_STORED]++;
+        else if (!(stored_len + 4 <= opt_lenb && buf != NULL) && static_lenb == opt_lenb && static_lenb == (unsigned long)(s->opt_len + 3 + 7) >> 3) g_fc[FC_TIE_STATIC]++;
     } else opt_lenb = static_lenb = stored_len + 5;
+    if (buf == NULL) g_fc[FC_UNSTORABLE]++;
     if (stored_len + 4 <= opt_lenb && buf != NULL) { /* _tr_stored_block + copy_block Z/trees.c:865-877,1205-1226 */
+        g_fc[FC_STORED]++;
         putbits(s, (unsigned)last, 3); align_byte(s);
         put8(s, stored_len & 0xff); put8(s, (stored_len >> 8) & 0xff); put8(s, ~stored_len & 0xff); put8(s, (~stored_len >> 8) & 0xff);
         for (unsigned long i = 0; i < stored_len; i++) put8(s, buf[i]);
     } else if (static_lenb == opt_lenb) {
+        g_fc[FC_STATIC]++;
         putbits(s, 2 + (unsigned)last, 3); emit_symbols(s, 0);
     } else {
+        g_fc[FC_DYNAMIC]++;
         putbits(s, 4 + (unsigned)last, 3);
         putbits(s, (unsigned)(s->l_max + 1 - 257), 5); putbits(s, (unsigned)(s->d_max + 1 - 1), 5); putbits(s, (unsigned)(max_bl + 1 - 4), 4);
         for (int r = 0; r <= max_bl; r++) putbits(s, s->bt[BLORD[r]].dl, 3);

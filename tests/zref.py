@@ -141,6 +141,26 @@ def oracle_deflate(data: bytes, level: int, wbits: int, memlevel: int, limit_out
     return dst.raw[:n]
 
 
+FLUSH_COUNTERS = ("over_lit", "over_dist", "over_bl",
+                  "force_lit_low", "force_lit_high", "force_dist_low", "force_dist_high", "force_bl_low", "force_bl_high",
+                  "stored", "static", "dynamic", "unstorable", "tie_stored", "tie_static",
+                  "rep16_6", "rep17_3", "rep17_10", "rep18_11", "rep18_138", "zrun_split")
+
+
+def oracle_flush_counts():
+    """Branch counters of the oracle's block flush since the last call (which resets them), by name:
+    over_*: gen_bitlen's depth-limit repair of the literal/length, distance and bit-length tree (Z/trees.c:530-564);
+    force_*_low / _high: build_tree's heap_len < 2 forcing with max_code < 2 / >= 2 (Z/trees.c:648-654);
+    stored / static / dynamic: block kinds written; unstorable: flushes whose block start has slid out of the window (buf == NULL);
+    tie_stored: stored_len + 4 == opt_lenb with a stored block written; tie_static: static_lenb == opt_lenb == the dynamic size;
+    rep16_6, rep17_3, rep17_10, rep18_11, rep18_138: scan_tree runs at the limits of their codes; zrun_split: a zero run over 138."""
+    o = oracle()
+    n = len(FLUSH_COUNTERS)
+    buf = (C.c_uint64 * n)()
+    assert o.oracle_flush_counts(buf, n) == n
+    return dict(zip(FLUSH_COUNTERS, buf))
+
+
 def ref_inflate_scan(buf: bytes, start: int, outcap: int, segments=None):
     """Re-enact ZBuffSearcher's calls on one candidate (main.cpp:228-239): inflateInit,
     inflate(Z_SYNC_FLUSH) with avail_in = len(buf)-start, avail_out = outcap, then drain

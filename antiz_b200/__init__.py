@@ -16,6 +16,7 @@ ATZ_F_EXACT_RECORDS = 1
 ATZ_F_STRATEGIES = 2     # extension: also try Z_FILTERED / Z_FIXED / Z_RLE / Z_HUFFMAN_ONLY (include/antiz_b200.h)
 ATZ_SCAN_SMALL_WINDOWS = 1   # extension: the scan also accepts CINFO 0 and 1 headers (offsetType 24..31, searched at window 9)
 ATZ_SCAN_PNG_IDAT = 4        # extension: the scan also finds zlib streams split over consecutive PNG IDAT chunks (Context.pieces)
+ATZ_SCAN_APNG_FDAT = 16      # extension: the same for APNG frames split over consecutive fdAT chunks (Context.framing)
 
 
 def clevel(level, strategy=0):
@@ -97,7 +98,9 @@ def lib():
         L.atz_host_partition.argtypes = [C.POINTER(C.c_uint64), C.POINTER(C.c_uint32), C.c_uint32, C.c_uint32, C.POINTER(C.c_uint32)]
         L.atz_get_owners.argtypes = [C.c_void_p, C.POINTER(C.c_uint32), C.c_uint64]
         L.atz_get_pieces.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(C.c_uint32), C.c_uint64, C.POINTER(C.c_uint64)]
+        L.atz_get_framing.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(C.c_uint32)]
         L.atz_host_idat_run.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.POINTER(C.c_uint32), C.c_uint64, C.POINTER(C.c_uint64)]
+        L.atz_host_fdat_run.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.POINTER(C.c_uint32), C.c_uint64, C.POINTER(C.c_uint64)]
         L.atz_search.argtypes = [C.c_void_p, C.POINTER(Options)]
         L.atz_search_shard.argtypes = [C.c_void_p, C.POINTER(Options), C.c_uint32, C.c_uint32]
         L.atz_get_streams.argtypes = [C.c_void_p, C.POINTER(Stream), C.c_uint64]
@@ -119,8 +122,8 @@ def lib():
 
 
 EXPORTS = ["atz_version", "atz_last_error", "atz_ctx_create", "atz_ctx_destroy", "atz_ctx_set_budget", "atz_ctx_set_scan_flags", "atz_load", "atz_load_device",
-           "atz_scan", "atz_attach", "atz_scan_shard", "atz_probe_export", "atz_probe_import", "atz_scan_finish", "atz_host_partition", "atz_search", "atz_search_shard", "atz_get_streams", "atz_get_owners", "atz_get_pieces", "atz_get_diffs", "atz_get_nested", "atz_get_inflated", "atz_get_inflated_recomp", "atz_get_inflated_list", "atz_get_stats", "atz_timer_start", "atz_timer_stop",
-           "atz_inflate_stream", "atz_deflate_stream", "atz_deflate_batch", "atz_trial"]
+           "atz_scan", "atz_attach", "atz_scan_shard", "atz_probe_export", "atz_probe_import", "atz_scan_finish", "atz_host_partition", "atz_search", "atz_search_shard", "atz_get_streams", "atz_get_owners", "atz_get_pieces", "atz_get_framing", "atz_get_diffs", "atz_get_nested", "atz_get_inflated", "atz_get_inflated_recomp", "atz_get_inflated_list", "atz_get_stats", "atz_timer_start", "atz_timer_stop",
+           "atz_inflate_stream", "atz_deflate_stream", "atz_deflate_batch", "atz_trial", "atz_host_fdat_run"]
 
 
 def _buf(b):
@@ -247,7 +250,8 @@ class Context:
         return ow[:n].tolist()
 
     def pieces(self, i):
-        """the piece lengths of stream i in the file: [] for an ordinary stream, >= 2 for one split over PNG IDAT chunks (atz_get_pieces)"""
+        """the piece lengths of stream i in the file: [] for an ordinary stream, >= 2 for one split over PNG IDAT or APNG fdAT chunks
+        (atz_get_pieces)"""
         n = C.c_uint64()
         rc = lib().atz_get_pieces(self._h, i, None, 0, C.byref(n))     # the size query: ATZ_E_SMALL for a split stream
         if rc not in (ATZ_OK, ATZ_E_SMALL):
@@ -256,6 +260,13 @@ class Context:
         if n.value:
             self._ck(lib().atz_get_pieces(self._h, i, out, n.value, C.byref(n)))
         return list(out[:n.value])
+
+    def framing(self, i):
+        """the bytes between two pieces of stream i in the file: 0 for an ordinary stream, 12 for IDAT chunks, 16 for fdAT chunks
+        (atz_get_framing)"""
+        b = C.c_uint32()
+        self._ck(lib().atz_get_framing(self._h, i, C.byref(b)))
+        return b.value
 
     def stream_table(self):
         """the same records as one numpy structured array (field names of Stream), without a Python object per stream"""

@@ -35,8 +35,8 @@ uint32_t scan_tiles_for(uint64_t lo, uint64_t hi);
 cudaError_t launch_scan_count(const uint8_t *, uint64_t, uint64_t, uint64_t, uint32_t, uint32_t *, uint16_t *, uint32_t *, cudaStream_t);
 cudaError_t launch_scan_write(const uint8_t *, uint64_t, uint64_t, const uint16_t *, const uint32_t *, uint32_t *, uint8_t *, uint32_t, cudaStream_t);
 cudaError_t launch_inflate(const uint8_t *, const InflateJob *, InflateResult *, InflateResult *, uint32_t, uint32_t *, uint8_t *, uint64_t, uint64_t, int, int, cudaStream_t);
-cudaError_t launch_idat_count(const uint8_t *, uint64_t, uint64_t, uint64_t, const uint32_t *, uint32_t, uint32_t *, cudaStream_t);
-cudaError_t launch_idat_write(const uint8_t *, uint64_t, uint64_t, uint64_t, const uint32_t *, const uint32_t *, const uint32_t *, const uint64_t *, uint32_t, uint32_t *, cudaStream_t);
+cudaError_t launch_split_count(const uint8_t *, uint64_t, uint64_t, uint64_t, uint32_t, const uint32_t *, uint32_t, uint32_t *, cudaStream_t);
+cudaError_t launch_split_write(const uint8_t *, uint64_t, uint64_t, uint64_t, uint32_t, const uint32_t *, const uint32_t *, const uint32_t *, const uint64_t *, uint32_t, uint32_t *, cudaStream_t);
 } // namespace atz
 using namespace atz;
 
@@ -66,9 +66,10 @@ struct StreamRec {
     uint32_t owner = 0;                 // shard that searches this stream (atz_host_partition)
     uint32_t adler = 0;
     std::vector<uint64_t> diff_off; std::vector<uint8_t> diff_val;
-    std::vector<uint32_t> pieces;       // ATZ_SCAN_PNG_IDAT: the piece lengths of a split stream (empty: an ordinary stream)
+    std::vector<uint32_t> pieces;       // ATZ_SCAN_PNG_IDAT / ATZ_SCAN_APNG_FDAT: the piece lengths of a split stream (empty: an ordinary stream)
+    uint32_t frame = 0;                 // bytes between two of its pieces: 12 (IDAT) or 16 (fdAT)
     uint64_t parent = 0; uint32_t depth = 0;   // a nested stream (ATZ_F_NESTED_DEPTH): atz_nested.parent and .depth; s.offset is relative to the parent's plaintext
-    uint64_t span() const { return s.streamLength + (pieces.empty() ? 0 : 12 * (pieces.size() - 1)); }   // bytes from s.offset to the stream's end in the file
+    uint64_t span() const { return s.streamLength + (pieces.empty() ? 0 : (uint64_t)frame * (pieces.size() - 1)); }   // bytes from s.offset to the stream's end in the file
 };
 
 struct Params { uint8_t c, w, m, s = 0; };   // level, windowBits, memLevel, strategy (0 = Z_DEFAULT_STRATEGY: all the reference ever uses)
@@ -79,11 +80,12 @@ struct ProbeX {
     uint64_t off, avail, p_in, p_out, p_cap, c_in, c_out, c_cap;
     int32_t p_status, c_status; uint32_t p_adler, c_adler, local, type;
 };
-// A split stream (ATZ_SCAN_PNG_IDAT) as a shard found it: the header offset, C and U of the de-chunked stream, its adler32 and header
-// type, and its piece lengths (the run's IDAT data lengths up to the one that holds the stream's last byte, that one cut at C)
+// A split stream (ATZ_SCAN_PNG_IDAT, ATZ_SCAN_APNG_FDAT) as a shard found it: the header offset, C and U of the de-chunked stream, its
+// adler32 and header type, its piece lengths (the run's piece lengths up to the one that holds the stream's last byte, that one cut at
+// C) and the framing bytes between two pieces (12: IDAT chunks, 16: fdAT chunks)
 struct SplitX {
-    uint64_t off, c, u; uint32_t adler, type; std::vector<uint32_t> pieces;
-    uint64_t span() const { return c + 12 * (pieces.size() - 1); }
+    uint64_t off, c, u; uint32_t adler, type; std::vector<uint32_t> pieces; uint32_t frame;
+    uint64_t span() const { return c + (uint64_t)frame * (pieces.size() - 1); }
 };
 struct SplitDev { const uint8_t *comp, *plain, *tmap; };   // where the probing shard keeps a split stream's bytes
 // State of a (possibly sharded) scan between atz_scan_shard and atz_scan_finish
@@ -784,7 +786,7 @@ void atz_ctx_destroy(atz_ctx *ctx) {
 }
 int atz_ctx_set_budget(atz_ctx *ctx, uint64_t bytes) { if (!ctx || bytes < (1u << 20)) return ATZ_E_ARG; ctx->budget = bytes; return ATZ_OK; }
 int atz_ctx_set_scan_flags(atz_ctx *ctx, uint32_t flags) {
-    if (!ctx || (flags & ~(uint32_t)(ATZ_SCAN_SMALL_WINDOWS | ATZ_SCAN_PNG_IDAT))) return ATZ_E_ARG;
+    if (!ctx || (flags & ~(uint32_t)(ATZ_SCAN_SMALL_WINDOWS | ATZ_SCAN_PNG_IDAT | ATZ_SCAN_APNG_FDAT))) return ATZ_E_ARG;
     if (ctx->scan_flags_fixed) { ctx->set_err("atz_ctx_set_scan_flags: the context has already loaded a file"); return ATZ_E_STATE; }
     ctx->scan_flags = flags;
     return ATZ_OK;
@@ -865,8 +867,9 @@ static int run_inflate(atz_ctx *ctx, const uint8_t *base, std::vector<InflateJob
     return ATZ_OK;
 }
 
-// ---- ATZ_SCAN_PNG_IDAT ----
-struct RunBytes { uint64_t off; const uint32_t *len; size_t npieces; uint64_t total; };   // a run's pieces in the file: piece k+1 starts 12 bytes after piece k
+// ---- ATZ_SCAN_PNG_IDAT, ATZ_SCAN_APNG_FDAT ----
+#define SPLIT_FLAGS (ATZ_SCAN_PNG_IDAT | ATZ_SCAN_APNG_FDAT)
+struct RunBytes { uint64_t off; const uint32_t *len; size_t npieces; uint64_t total; uint32_t frame; };   // a run's pieces in the file: piece k+1 starts frame bytes after piece k
 // The pieces of every run put together in one new device buffer (freed with plain_extra at the next scan), each run at at[i] with ATZ_PAD
 // zeroed bytes behind it: one gather launch over the file image for the runs inside the mapped range, host copies from the attached file
 // for the others.
@@ -878,14 +881,14 @@ static int dechunk(atz_ctx *ctx, const std::vector<RunBytes> &runs, uint8_t *&ba
     std::vector<CopyJob> cj; std::vector<uint8_t> stage;
     for (size_t i = 0; i < runs.size(); i++) {
         const RunBytes &r = runs[i];
-        const bool mapped = ctx->d_file && r.off >= ctx->r0 && r.off + r.total + 12 * (r.npieces - 1) <= ctx->r1;
-        if (!mapped && !ctx->h_file) { ctx->set_err("IDAT run outside the resident file range"); return ATZ_E_STATE; }
+        const bool mapped = ctx->d_file && r.off >= ctx->r0 && r.off + r.total + (uint64_t)r.frame * (r.npieces - 1) <= ctx->r1;
+        if (!mapped && !ctx->h_file) { ctx->set_err("chunk run outside the resident file range"); return ATZ_E_STATE; }
         if (!mapped) stage.resize(r.total);
         uint64_t src = r.off, dst = 0;
         for (size_t k = 0; k < r.npieces; k++) {
             if (mapped) cj.push_back(CopyJob{ctx->d_file + src, base + at[i] + dst, r.len[k]});
             else memcpy(stage.data() + dst, ctx->h_file + src, r.len[k]);
-            dst += r.len[k]; src += r.len[k] + 12;
+            dst += r.len[k]; src += r.len[k] + r.frame;
         }
         if (!mapped && r.total) { CK(cudaMemcpyAsync(base + at[i], stage.data(), r.total, cudaMemcpyHostToDevice, ctx->stream)); CK(cudaStreamSynchronize(ctx->stream)); }
     }
@@ -898,30 +901,30 @@ static int dechunk(atz_ctx *ctx, const std::vector<RunBytes> &runs, uint8_t *&ba
     return ATZ_OK;
 }
 
-// The split streams of this shard: the K1 candidates (cand, type: K1's own list) that start an IDAT run (png.cu), each inflated by K2
-// over its run's data put together; a stream that ends there beyond its first piece and is longer than 16 bytes is recorded (SplitX)
-// with its plaintext and token map left resident, like a probed ordinary stream's.
-static int probe_idat_runs(atz_ctx *ctx, const std::vector<uint32_t> &cand, const std::vector<uint8_t> &type) {
-    ScanState &sc = ctx->sc; const uint64_t N = ctx->n;
+// The split streams of this shard: the K1 candidates (cand, type: K1's own list) that start an IDAT or fdAT run (png.cu; the kinds the
+// scan flags enable), each inflated by K2 over its run's pieces put together; a stream that ends there beyond its first piece and is
+// longer than 16 bytes is recorded (SplitX) with its plaintext and token map left resident, like a probed ordinary stream's.
+static int probe_split_runs(atz_ctx *ctx, const std::vector<uint32_t> &cand, const std::vector<uint8_t> &type) {
+    ScanState &sc = ctx->sc; const uint64_t N = ctx->n; const uint32_t flags = ctx->scan_flags;
     const uint32_t nc = (uint32_t)cand.size();
-    std::vector<uint32_t> which, cnt; std::vector<uint64_t> at; std::vector<uint32_t> lens;   // run i: candidate which[i], cnt[i] lengths at lens[at[i]]
+    std::vector<uint32_t> which, cnt, frame; std::vector<uint64_t> at; std::vector<uint32_t> lens;   // run i: candidate which[i], cnt[i] lengths at lens[at[i]]
     if (nc) {
         std::vector<uint32_t> counts(nc);
         Phase ph(ctx, &ctx->st.ms_scan);
         CK(ctx->idat_counts.ensure((size_t)nc * 4));
-        CK(launch_idat_count(ctx->d_file, N, ctx->r0, ctx->r1, ctx->cand.as<uint32_t>(), nc, ctx->idat_counts.as<uint32_t>(), ctx->stream)); ctx->st.kernel_launches++;
+        CK(launch_split_count(ctx->d_file, N, ctx->r0, ctx->r1, flags, ctx->cand.as<uint32_t>(), nc, ctx->idat_counts.as<uint32_t>(), ctx->stream)); ctx->st.kernel_launches++;
         CK(cudaMemcpyAsync(counts.data(), ctx->idat_counts.p, (size_t)nc * 4, cudaMemcpyDeviceToHost, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
         std::vector<uint32_t> dw; std::vector<uint64_t> dat; uint64_t tot = 0;
-        for (uint32_t k = 0; k < nc; k++) if (counts[k] && counts[k] != IDAT_FAR) { dw.push_back(k); dat.push_back(tot); tot += counts[k]; }
+        for (uint32_t k = 0; k < nc; k++) if (counts[k] && counts[k] != IDAT_FAR) { dw.push_back(k); dat.push_back(tot); tot += counts[k] & ~RUN_FDAT; }
         lens.resize(tot);
         if (!dw.empty()) {
             CK(ctx->idat_runs.ensure(dw.size() * 12)); CK(ctx->idat_lens.ensure(tot * 4));
             uint64_t *d_at = ctx->idat_runs.as<uint64_t>(); uint32_t *d_which = (uint32_t *)(d_at + dw.size());   // (the 8-byte offsets first: aligned)
             CK(cudaMemcpyAsync(d_at, dat.data(), dw.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
             CK(cudaMemcpyAsync(d_which, dw.data(), dw.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
-            CK(launch_idat_write(ctx->d_file, N, ctx->r0, ctx->r1, ctx->cand.as<uint32_t>(), ctx->idat_counts.as<uint32_t>(), d_which, d_at, (uint32_t)dw.size(),
-                                 ctx->idat_lens.as<uint32_t>(), ctx->stream));
+            CK(launch_split_write(ctx->d_file, N, ctx->r0, ctx->r1, flags, ctx->cand.as<uint32_t>(), ctx->idat_counts.as<uint32_t>(), d_which, d_at, (uint32_t)dw.size(),
+                                  ctx->idat_lens.as<uint32_t>(), ctx->stream));
             ctx->st.kernel_launches++;
             CK(cudaMemcpyAsync(lens.data(), ctx->idat_lens.p, tot * 4, cudaMemcpyDeviceToHost, ctx->stream));
         }
@@ -929,19 +932,22 @@ static int probe_idat_runs(atz_ctx *ctx, const std::vector<uint32_t> &cand, cons
         // runs that leave the resident range (atz_attach): walked again over the whole attached file
         size_t j = 0;
         for (uint32_t k = 0; k < nc; k++) {
-            if (counts[k] == IDAT_FAR) {
-                if (!ctx->h_file) { ctx->set_err("IDAT run outside the resident file range"); return ATZ_E_STATE; }
-                const uint32_t m = idat_run(ctx->h_file, N, 0, N, cand[k], nullptr, 0);
+            uint32_t m = counts[k];
+            if (m == IDAT_FAR) {
+                if (!ctx->h_file) { ctx->set_err("chunk run outside the resident file range"); return ATZ_E_STATE; }
+                m = split_run(ctx->h_file, N, 0, N, cand[k], flags, nullptr, 0);
                 if (!m) continue;
-                which.push_back(k); cnt.push_back(m); at.push_back(lens.size()); lens.resize(lens.size() + m);
-                idat_run(ctx->h_file, N, 0, N, cand[k], lens.data() + at.back(), m);
-            } else if (j < dw.size() && dw[j] == k) { which.push_back(k); cnt.push_back(counts[k]); at.push_back(dat[j]); j++; }
+                at.push_back(lens.size()); lens.resize(lens.size() + (m & ~RUN_FDAT));
+                split_run(ctx->h_file, N, 0, N, cand[k], flags, lens.data() + at.back(), m & ~RUN_FDAT);
+            } else if (j < dw.size() && dw[j] == k) at.push_back(dat[j++]);
+            else continue;
+            which.push_back(k); cnt.push_back(m & ~RUN_FDAT); frame.push_back(m & RUN_FDAT ? 16 : 12);
         }
     }
     const size_t nr = which.size();
     std::vector<RunBytes> runs(nr);
     for (size_t i = 0; i < nr; i++) {
-        RunBytes r{cand[which[i]], lens.data() + at[i], cnt[i], 0};
+        RunBytes r{cand[which[i]], lens.data() + at[i], cnt[i], 0, frame[i]};
         for (size_t k = 0; k < cnt[i]; k++) r.total += r.len[k];
         runs[i] = r;
     }
@@ -977,7 +983,7 @@ static int probe_idat_runs(atz_ctx *ctx, const std::vector<uint32_t> &cand, cons
     for (size_t i = 0; i < nr; i++) {
         const InflateResult &r = fin[i]; const uint64_t C = r.total_in;
         if (r.status != INF_END || C <= runs[i].len[0] || C <= 16) continue;
-        SplitX x{runs[i].off, C, r.total_out, r.adler, type[which[i]], {}};
+        SplitX x{runs[i].off, C, r.total_out, r.adler, type[which[i]], {}, runs[i].frame};
         for (uint64_t k = 0, got = 0; got < C; k++) { const uint64_t l = std::min<uint64_t>(runs[i].len[k], C - got); x.pieces.push_back((uint32_t)l); got += l; }
         sc.split[sc.shard].push_back(std::move(x)); sc.split_dev.push_back(SplitDev{comp + cat[i], plain[i], tmap[i]});
     }
@@ -1012,7 +1018,7 @@ int atz_scan_shard(atz_ctx *ctx, uint64_t chunksize, uint32_t shard, uint32_t ns
     sc.QS = QS; sc.SLOT = SLOT;
     std::vector<uint32_t> &cand = sc.cand; std::vector<uint8_t> &ctype = sc.ctype;
     std::vector<InflateJob> &jobs = sc.jobs; std::vector<InflateResult> &res = sc.res, &cres = sc.cres;
-    std::vector<uint32_t> k1cand; std::vector<uint8_t> k1type;    // ATZ_SCAN_PNG_IDAT: K1's own candidates (the real file bytes, no chunk-start fix-up)
+    std::vector<uint32_t> k1cand; std::vector<uint8_t> k1type;    // SPLIT_FLAGS: K1's own candidates (the real file bytes, no chunk-start fix-up)
     // a continuation (a stream that runs over the end of its chunk) reads the following chunks: map `extra` of them behind the
     // shard's own; in the rare case that one needs more than that, the probe is repeated with four times as many
     for (size_t extra = 1;; extra *= 4) {
@@ -1038,7 +1044,7 @@ int atz_scan_shard(atz_ctx *ctx, uint64_t chunksize, uint32_t shard, uint32_t ns
             }
             ph.stop();
             CK(cudaGetLastError());
-            if (ctx->scan_flags & ATZ_SCAN_PNG_IDAT) { k1cand = cand; k1type = ctype; }
+            if (ctx->scan_flags & SPLIT_FLAGS) { k1cand = cand; k1type = ctype; }
         }
         // ---- the first position of every chunk k >= 2 holds file[start_k - 1] in the reference's buffer (see chunk_list): fix those up ----
         std::vector<uint8_t> special;    // per candidate: 1 = its first byte is file[off - 1]
@@ -1188,26 +1194,28 @@ int atz_scan_shard(atz_ctx *ctx, uint64_t chunksize, uint32_t shard, uint32_t ns
         if (res[k].status == INF_NEED_INPUT && cres[k].status >= 0) { x.c_status = cres[k].status; x.c_in = cres[k].total_in; x.c_out = cres[k].total_out; x.c_cap = cres[k].in_at_outcap; x.c_adler = cres[k].adler; }
         mine.push_back(x);
     }
-    if (ctx->scan_flags & ATZ_SCAN_PNG_IDAT) { int rc = probe_idat_runs(ctx, k1cand, k1type); if (rc) return rc; }
+    if (ctx->scan_flags & SPLIT_FLAGS) { int rc = probe_split_runs(ctx, k1cand, k1type); if (rc) return rc; }
     sc.have[shard] = 1; sc.probed = true;
     ctx->st.algo_bytes += f1 - f0;
     return ATZ_OK;
 }
 
 // the export: the exporting context's scan flags (8 bytes; the records were found with that header set), then the records; with
-// ATZ_SCAN_PNG_IDAT then the split streams (SPLIT_HEAD bytes each: off, C, U, adler, type, number of pieces; then the piece lengths)
-// and the size of that part (8 bytes)
+// ATZ_SCAN_PNG_IDAT or ATZ_SCAN_APNG_FDAT then the split streams (SPLIT_HEAD bytes each: off, C, U, adler, type, number of pieces; then
+// the piece lengths) and the size of that part (8 bytes).  The type word of a stream split over fdAT chunks has SPLIT_FDAT set (an
+// IDAT one's is the header type alone, as before fdAT runs existed).
 #define SPLIT_HEAD 36
+#define SPLIT_FDAT 0x10000u
 int atz_probe_export(atz_ctx *ctx, void *buf, uint64_t cap, uint64_t *nbytes) {
     if (!ctx || !nbytes) return ATZ_E_ARG;
     if (!ctx->sc.probed) return ATZ_E_STATE;
     const std::vector<ProbeX> &v = ctx->sc.px[ctx->sc.shard];
     const uint64_t flags = ctx->scan_flags;
     std::vector<uint8_t> split;
-    if (flags & ATZ_SCAN_PNG_IDAT) {
+    if (flags & SPLIT_FLAGS) {
         for (const SplitX &x : ctx->sc.split[ctx->sc.shard]) {
-            uint8_t h[SPLIT_HEAD]; const uint32_t np = (uint32_t)x.pieces.size();
-            memcpy(h, &x.off, 8); memcpy(h + 8, &x.c, 8); memcpy(h + 16, &x.u, 8); memcpy(h + 24, &x.adler, 4); memcpy(h + 28, &x.type, 4); memcpy(h + 32, &np, 4);
+            uint8_t h[SPLIT_HEAD]; const uint32_t np = (uint32_t)x.pieces.size(), t = x.type | (x.frame == 16 ? SPLIT_FDAT : 0);
+            memcpy(h, &x.off, 8); memcpy(h + 8, &x.c, 8); memcpy(h + 16, &x.u, 8); memcpy(h + 24, &x.adler, 4); memcpy(h + 28, &t, 4); memcpy(h + 32, &np, 4);
             split.insert(split.end(), h, h + SPLIT_HEAD);
             split.insert(split.end(), (const uint8_t *)x.pieces.data(), (const uint8_t *)(x.pieces.data() + np));
         }
@@ -1225,7 +1233,7 @@ int atz_probe_import(atz_ctx *ctx, uint32_t shard, const void *buf, uint64_t nby
     if (!ctx || !buf || nbytes < sizeof flags) return ATZ_E_ARG;
     const uint8_t *b = (const uint8_t *)buf;
     memcpy(&flags, b, sizeof flags);
-    if (flags & ATZ_SCAN_PNG_IDAT) {     // the split streams and their size behind the probe records
+    if (flags & SPLIT_FLAGS) {     // the split streams and their size behind the probe records
         if (nbytes < 2 * sizeof flags) return ATZ_E_ARG;
         memcpy(&split_bytes, b + nbytes - 8, 8);
         if (split_bytes > nbytes - 16) return ATZ_E_ARG;
@@ -1243,9 +1251,12 @@ int atz_probe_import(atz_ctx *ctx, uint32_t shard, const void *buf, uint64_t nby
     std::vector<SplitX> &sv = ctx->sc.split[shard]; sv.clear();
     for (const uint8_t *q = b + sizeof flags + nbytes, *e = q + (split_bytes ? split_bytes - 8 : 0); q < e;) {
         if (e - q < SPLIT_HEAD) return ATZ_E_ARG;
-        SplitX x; uint32_t np = 0;
-        memcpy(&x.off, q, 8); memcpy(&x.c, q + 8, 8); memcpy(&x.u, q + 16, 8); memcpy(&x.adler, q + 24, 4); memcpy(&x.type, q + 28, 4); memcpy(&np, q + 32, 4);
+        SplitX x; uint32_t np = 0, t = 0;
+        memcpy(&x.off, q, 8); memcpy(&x.c, q + 8, 8); memcpy(&x.u, q + 16, 8); memcpy(&x.adler, q + 24, 4); memcpy(&t, q + 28, 4); memcpy(&np, q + 32, 4);
         q += SPLIT_HEAD;
+        const bool fdat = t & SPLIT_FDAT;    // the kind must be one the scan flags enable
+        x.type = t & ~SPLIT_FDAT; x.frame = fdat ? 16 : 12;
+        if (!(flags & (fdat ? ATZ_SCAN_APNG_FDAT : ATZ_SCAN_PNG_IDAT))) return ATZ_E_ARG;
         if (np < 2 || (uint64_t)(e - q) / 4 < np) return ATZ_E_ARG;
         x.pieces.resize(np); memcpy(x.pieces.data(), q, 4ull * np); q += 4ull * np;
         uint64_t sum = 0; for (uint32_t l : x.pieces) sum += l;
@@ -1279,7 +1290,8 @@ int atz_scan_finish(atz_ctx *ctx, uint64_t *n_streams) {
         }
         scan_fold(cstart, clen, xc.data(), nx, pr.data(), avail.data(), cont_of.data(), cr.data(), acc);
     }
-    // ---- ATZ_SCAN_PNG_IDAT, after the fold and the same on every context: a split stream (file order) is dropped if an accepted stream
+    // ---- ATZ_SCAN_PNG_IDAT / ATZ_SCAN_APNG_FDAT, after the fold and the same on every context: a split stream (IDAT and fdAT runs in one
+    // list, file order) is dropped if an accepted stream
     // or a split stream kept before it overlaps its span without lying inside it; otherwise it takes the place of the accepted streams
     // inside its span (accidents of inflating compressed bytes) ----
     struct SplitRef { const SplitX *x; uint32_t src, local; };
@@ -1327,7 +1339,7 @@ int atz_scan_finish(atz_ctx *ctx, uint64_t *n_streams) {
         r.s.clevel = 9; r.s.window = 15; r.s.memlevel = 9; r.s.firstDiffByte = -1;
         if (split_of[s] >= 0) {     // a split stream: its bytes are resident where it was probed; another owner puts its pieces together and inflates them again
             const SplitRef &q = spl[split_of[s]];
-            r.s.offsetType = (int32_t)q.x->type; r.owner = owner[s]; r.adler = q.x->adler; r.pieces = q.x->pieces;
+            r.s.offsetType = (int32_t)q.x->type; r.owner = owner[s]; r.adler = q.x->adler; r.pieces = q.x->pieces; r.frame = q.x->frame;
             if (r.owner != sc.shard) continue;
             if (q.src == sc.shard) { const SplitDev &d = sc.split_dev[q.local]; r.d_comp = d.comp; r.d_plain = d.plain; r.d_tmap = d.tmap; }
             else { far_runs.push_back(s); recheck.push_back(s); }
@@ -1350,7 +1362,7 @@ int atz_scan_finish(atz_ctx *ctx, uint64_t *n_streams) {
     }
     if (!far_runs.empty()) {   // (before the staging below, which takes every owned stream that has no compressed bytes yet)
         std::vector<RunBytes> rb;
-        for (size_t s : far_runs) { const StreamRec &r = ctx->streams[s]; rb.push_back(RunBytes{r.s.offset, r.pieces.data(), r.pieces.size(), r.s.streamLength}); }
+        for (size_t s : far_runs) { const StreamRec &r = ctx->streams[s]; rb.push_back(RunBytes{r.s.offset, r.pieces.data(), r.pieces.size(), r.s.streamLength, r.frame}); }
         uint8_t *base = nullptr; std::vector<uint64_t> at;
         { int rc = dechunk(ctx, rb, base, at); if (rc) return rc; }
         for (size_t i = 0; i < far_runs.size(); i++) ctx->streams[far_runs[i]].d_comp = base + at[i];
@@ -1879,7 +1891,7 @@ int atz_search_shard(atz_ctx *ctx, const atz_options *opt, uint32_t shard, uint3
     uint64_t di = 0, nrec = 0, atz = 28, lastend = 0;
     for (auto &r : ctx->streams) {
         r.s.diff_index = di; di += r.s.ndiff;
-        if (r.s.recomp) { nrec++; atz += 35 + (r.s.ndiff ? 8 + 9 * r.s.ndiff : 0) + r.s.inflatedLength + (r.pieces.empty() ? 0 : 8 + 16 * r.pieces.size() - 12); }
+        if (r.s.recomp) { nrec++; atz += 35 + (r.s.ndiff ? 8 + 9 * r.s.ndiff : 0) + r.s.inflatedLength + (r.pieces.empty() ? 0 : 8 + 4 * r.pieces.size() + (uint64_t)r.frame * (r.pieces.size() - 1)); }
         else atz += r.span();
         if (r.s.offset >= lastend) { atz += r.s.offset - lastend; }
         lastend = r.s.offset + r.span();
@@ -1916,6 +1928,13 @@ int atz_get_pieces(atz_ctx *ctx, uint64_t i, uint32_t *len, uint64_t cap, uint64
     *npieces = p.size();
     if (cap < p.size()) return ATZ_E_SMALL;
     if (!p.empty()) memcpy(len, p.data(), p.size() * 4);
+    return ATZ_OK;
+}
+int atz_get_framing(atz_ctx *ctx, uint64_t i, uint32_t *bytes) {
+    if (!ctx || !bytes) return ATZ_E_ARG;
+    if (ctx->state < 2) return ATZ_E_STATE;
+    if (i >= ctx->streams.size()) return ATZ_E_ARG;
+    *bytes = ctx->streams[i].pieces.empty() ? 0 : ctx->streams[i].frame;
     return ATZ_OK;
 }
 int atz_get_diffs(atz_ctx *ctx, uint64_t *offsets, uint8_t *values, uint64_t cap, uint64_t *n) {
@@ -2173,6 +2192,11 @@ int atz_host_header_type(uint32_t scan_flags, uint32_t b0, uint32_t b1) { return
 int atz_host_idat_run(const uint8_t *file, uint64_t n, uint64_t p, uint32_t *len, uint64_t cap, uint64_t *npieces) {
     if (!file || !npieces || (!len && cap)) return ATZ_E_ARG;
     *npieces = p < n ? idat_run(file, n, 0, n, p, len, (uint32_t)std::min<uint64_t>(cap, 0xffffffffull)) : 0;
+    return ATZ_OK;
+}
+int atz_host_fdat_run(const uint8_t *file, uint64_t n, uint64_t p, uint32_t *len, uint64_t cap, uint64_t *npieces) {
+    if (!file || !npieces || (!len && cap)) return ATZ_E_ARG;
+    *npieces = p < n ? fdat_run(file, n, 0, n, p, len, (uint32_t)std::min<uint64_t>(cap, 0xffffffffull)) : 0;
     return ATZ_OK;
 }
 int atz_host_candidate_sequence(int offsetType, int brute, uint8_t *clevel, uint8_t *window, uint8_t *memlevel, uint32_t cap) {

@@ -101,35 +101,63 @@ __host__ __device__ __forceinline__ int zlib_header_type(uint32_t b0, uint32_t b
 }
 
 // ---------------------------------------------------------------------------------------------
-// PNG IDAT runs (ATZ_SCAN_PNG_IDAT; png.cu, api.cu).  A header at p starts a run when p >= 8, file[p-4..p) == "IDAT", the chunk's
-// length L1 = BE32(file[p-8..p-4]) >= 2 and the chunk behind its CRC (header at p + L1 + 4) is an IDAT too.  The run goes on over
-// consecutive IDATs whose data and CRC lie inside the file [0, n) and ends at another chunk type or at one that would run past the
-// end.  Returns the number of chunks (0: p starts no run; a run has >= 2) and their data lengths in len[0 .. min(count, cap)).
-// Only [lo, lim) is read (the part of the file the caller can address); a walk that would need a byte outside returns IDAT_FAR,
-// and the caller walks again over the whole file.  One dependent 8-byte read per chunk.
+// PNG chunk runs (ATZ_SCAN_PNG_IDAT, ATZ_SCAN_APNG_FDAT; png.cu, api.cu).  A chunk is a BE32 length L, a 4-byte tag, L data bytes and
+// a CRC.  The data of an IDAT is a piece of the image's zlib stream; the data of an APNG fdAT is a 4-byte sequence number, then a piece
+// of its frame's stream: `pre` = 0 or 4 bytes in front of each piece.  A header at p starts a run of `tag` chunks when p >= 8 + pre,
+// the tag lies at file[p-pre-4 .. p-pre), the chunk's length L1 = BE32(file[p-pre-8 ..]) >= pre + 2 and the chunk behind its CRC is
+// a `tag` chunk with L >= pre too.  The run goes on over consecutive `tag` chunks with L >= pre whose data and CRC lie inside the file
+// [0, n) and ends at another chunk type, at a shorter one or at one that would run past the end.  Sequence numbers and CRCs are not
+// looked at.  Returns the number of chunks (0: p starts no run; a run has >= 2) and their piece lengths L - pre in len[0 ..
+// min(count, cap)); piece k+1 starts 12 + pre bytes after piece k ends.  Only [lo, lim) is read (the part of the file the caller can
+// address); a walk that would need a byte outside returns IDAT_FAR, and the caller walks again over the whole file.  One dependent
+// 8-byte read per chunk.
 // ---------------------------------------------------------------------------------------------
 #define IDAT_FAR 0xffffffffu
+#define TAG_IDAT 0x49444154u    // "IDAT"
+#define TAG_FDAT 0x66644154u    // "fdAT"
 __host__ __device__ __forceinline__ uint32_t be32(const uint8_t *q) { return (uint32_t)q[0] << 24 | (uint32_t)q[1] << 16 | (uint32_t)q[2] << 8 | q[3]; }
-__host__ __device__ __forceinline__ bool is_idat(const uint8_t *q) { return q[0] == 'I' && q[1] == 'D' && q[2] == 'A' && q[3] == 'T'; }
-__host__ __device__ inline uint32_t idat_run(const uint8_t *file, uint64_t n, uint64_t lo, uint64_t lim, uint64_t p, uint32_t *len, uint32_t cap) {
-    if (p < 8) return 0;
-    if (p - 8 < lo || p > lim) return IDAT_FAR;
-    if (!is_idat(file + p - 4)) return 0;
-    uint64_t L = be32(file + p - 8), d = p;     // the current chunk: data at d, L bytes
-    if (L < 2) return 0;
+__host__ __device__ inline uint32_t chunk_run(const uint8_t *file, uint64_t n, uint64_t lo, uint64_t lim, uint64_t p, uint32_t tag, uint32_t pre,
+                                              uint32_t *len, uint32_t cap) {
+    if (p < 8 + pre) return 0;
+    if (p - 8 - pre < lo || p > lim) return IDAT_FAR;
+    if (be32(file + p - pre - 4) != tag) return 0;
+    uint64_t L = be32(file + p - pre - 8), d = p - pre;   // the current chunk: data at d, L bytes
+    if (L < pre + 2) return 0;
     uint32_t cnt = 0;
     for (;;) {
         if (d + L + 4 > n) break;                 // data or CRC past the end of the file: not part of the run
         if (d + L + 4 > lim) return IDAT_FAR;
-        if (cnt < cap) len[cnt] = (uint32_t)L;
+        if (cnt < cap) len[cnt] = (uint32_t)(L - pre);
         cnt++;
         const uint64_t q = d + L + 4;             // the next chunk's header
         if (q + 8 > n) break;
         if (q + 8 > lim) return IDAT_FAR;
-        if (!is_idat(file + q + 4)) break;
+        if (be32(file + q + 4) != tag) break;
         L = be32(file + q); d = q + 8;
+        if (L < pre) break;
     }
     return cnt >= 2 ? cnt : 0;
+}
+__host__ __device__ __forceinline__ uint32_t idat_run(const uint8_t *file, uint64_t n, uint64_t lo, uint64_t lim, uint64_t p, uint32_t *len, uint32_t cap) {
+    return chunk_run(file, n, lo, lim, p, TAG_IDAT, 0, len, cap);
+}
+__host__ __device__ __forceinline__ uint32_t fdat_run(const uint8_t *file, uint64_t n, uint64_t lo, uint64_t lim, uint64_t p, uint32_t *len, uint32_t cap) {
+    return chunk_run(file, n, lo, lim, p, TAG_FDAT, 4, len, cap);
+}
+// The run the scan takes at p under the ATZ_SCAN_* set `flags`: an IDAT run if that flag is on and p starts one, otherwise an fdAT
+// run if that flag is on (a header whose fdAT sequence number spells "IDAT" can start both).  The count of chunk_run, RUN_FDAT set
+// for an fdAT run; IDAT_FAR as there.
+#define RUN_FDAT 0x80000000u
+__host__ __device__ __forceinline__ uint32_t split_run(const uint8_t *file, uint64_t n, uint64_t lo, uint64_t lim, uint64_t p, uint32_t flags, uint32_t *len, uint32_t cap) {
+    if (flags & ATZ_SCAN_PNG_IDAT) {
+        const uint32_t m = idat_run(file, n, lo, lim, p, len, cap);
+        if (m) return m;
+    }
+    if (flags & ATZ_SCAN_APNG_FDAT) {
+        const uint32_t m = fdat_run(file, n, lo, lim, p, len, cap);
+        if (m) return m == IDAT_FAR ? m : m | RUN_FDAT;
+    }
+    return 0;
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -28,6 +28,7 @@ struct programOptions {
     bool strategies = false;             // ATZ_F_STRATEGIES: also try zlib's other strategies (changes the ATZ file vs the reference)
     bool smallWindows = false;           // ATZ_SCAN_SMALL_WINDOWS: also accept CINFO 0 and 1 headers (the reference can still reconstruct)
     bool png = false;                    // ATZ_SCAN_PNG_IDAT: also find zlib streams split over PNG IDAT chunks (changes the ATZ file vs the reference)
+    bool apng = false;                   // ATZ_SCAN_APNG_FDAT: also find zlib streams split over APNG fdAT chunks (changes the ATZ file vs the reference)
     int nested = 0;                      // ATZ_F_NESTED_DEPTH: also recompress zlib streams inside recompressed ones, this many levels deep (changes the ATZ file vs the reference)
 };
 
@@ -54,11 +55,12 @@ class streamOffset {
     std::vector<uint8_t> diffByteVal;      // the original bytes at those positions
     bool recomp;
     uint64_t atzInfos;                     // reconstruct: offset of the inflated payload inside the ATZ file
-    // antiz_b200 extension (ATZ_SCAN_PNG_IDAT): a stream split over PNG IDAT chunks has npieces >= 2 pieces in the file, 12 bytes of
-    // chunk framing between two; streamLength is the sum of the pieces
+    // antiz_b200 extension (ATZ_SCAN_PNG_IDAT, ATZ_SCAN_APNG_FDAT): a stream split over PNG IDAT or APNG fdAT chunks has npieces >= 2
+    // pieces in the file, `frame` bytes of chunk framing between two (12: IDAT, 16: fdAT); streamLength is the sum of the pieces
     std::vector<uint32_t> pieces;
+    uint32_t frame = 12;
     uint64_t gapsAt = 0;                   // reconstruct: offset of the framing bytes inside the ATZ file
-    uint64_t spanLength() const { return streamLength + (pieces.empty() ? 0 : 12 * (pieces.size() - 1)); }   // bytes of the original the stream covers
+    uint64_t spanLength() const { return streamLength + (pieces.empty() ? 0 : (uint64_t)frame * (pieces.size() - 1)); }   // bytes of the original the stream covers
 };
 
 class fileOffset {   // unused by the reference's live code; kept for source compatibility

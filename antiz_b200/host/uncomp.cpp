@@ -6,7 +6,7 @@
 // same built-in self test (testATZfile main.cpp:1173-1203).  The host keeps what the reference's L1/L2 layers do
 // (CLI, file IO, ATZ1 layout, phase order); phases 1 and 3 and the per-stream deflate of the reconstructor run on
 // the GPU.  Extensions: --gpus N (static shard of the stream x parameter grid), --device D, --exact-records, --stats, --strategies,
-// --small-windows, --png, --nested.
+// --small-windows, --png, --nested, --apng.
 #include "ATZData.h"
 #include "antiz_b200.h"
 #include <chrono>
@@ -102,7 +102,7 @@ class ATZcreator {
             mk(0);
             for (auto &t : th) t.join();
             for (int g = 0; g < ng; g++) if (crc[g] != ATZ_OK) { std::cout << "error: no usable CUDA device " << (options.device + g) << " (antiz_b200 has no CPU path)" << std::endl; std::exit(1); }
-            const uint32_t scan_flags = (options.smallWindows ? ATZ_SCAN_SMALL_WINDOWS : 0) | (options.png ? ATZ_SCAN_PNG_IDAT : 0);
+            const uint32_t scan_flags = (options.smallWindows ? ATZ_SCAN_SMALL_WINDOWS : 0) | (options.png ? ATZ_SCAN_PNG_IDAT : 0) | (options.apng ? ATZ_SCAN_APNG_FDAT : 0);
             for (int g = 0; g < ng && scan_flags; g++) {   // before any load: every shard scans with the same header set
                 const int rc = atz_ctx_set_scan_flags(ctxs[g], scan_flags);
                 if (rc != ATZ_OK) { std::cout << atz_err(ctxs[g], rc) << std::endl; abort(); }
@@ -176,10 +176,10 @@ class ATZcreator {
             s.identBytes = a.identBytes; s.firstDiffByte = a.firstDiffByte; s.recomp = a.recomp != 0;
             s.diffByteOffsets.assign(doff[g].begin() + a.diff_index, doff[g].begin() + a.diff_index + a.ndiff);
             s.diffByteVal.assign(dval[g].begin() + a.diff_index, dval[g].begin() + a.diff_index + a.ndiff);
-            if (options.png) {
+            if (options.png || options.apng) {
                 uint64_t np = 0; atz_get_pieces(ctxs[g], i, nullptr, 0, &np);
                 s.pieces.resize(np);
-                if (np && atz_get_pieces(ctxs[g], i, s.pieces.data(), np, &np) != ATZ_OK) { std::cout << atz_err(ctxs[g], -1) << std::endl; abort(); }
+                if (np && (atz_get_pieces(ctxs[g], i, s.pieces.data(), np, &np) != ATZ_OK || atz_get_framing(ctxs[g], i, &s.frame) != ATZ_OK)) { std::cout << atz_err(ctxs[g], -1) << std::endl; abort(); }
             }
             streams.push_back(std::move(s));
         }
@@ -238,7 +238,8 @@ class ATZcreator {
 
     // ATZ1 layout (main.cpp:775-831): header, per recompressed stream {descriptor, diffs, inflated data}, residue.  A stream split over
     // PNG IDAT chunks (--png) has bit 7 of its window byte set and, behind the diffs, u64 npieces, npieces u32 piece lengths and the
-    // (npieces - 1) x 12 framing bytes between the pieces, copied from the input (its CRCs stay exact even where they are wrong).
+    // (npieces - 1) x 12 framing bytes between the pieces, copied from the input (its CRCs stay exact even where they are wrong).  One
+    // split over APNG fdAT chunks (--apng) sets bits 7 and 5, and its framing is 16 bytes per gap (the sequence numbers stay exact too).
     // A stream with recompressed nested streams (--nested) has bit 6 of its window byte set, and its payload P is replaced by u64 nchild,
     // the records of those nchild streams in offset order (the same layout, recursively; never bit 7) and P without their bytes.
     static bool any_recomp(const std::vector<Nest> &ns, const std::vector<size_t> &k) { for (size_t i : k) if (ns[i].s.recomp) return true; return false; }
@@ -266,7 +267,7 @@ class ATZcreator {
     }
     void writeATZfile() {
         uint64_t total = 28, nrec = countRecomp();
-        for (auto &s : streams) if (s.recomp) total += 35 + (s.diffByteOffsets.empty() ? 0 : 8 + 9 * s.diffByteOffsets.size()) + s.inflatedLength + (s.pieces.empty() ? 0 : 8 + 16 * s.pieces.size() - 12);
+        for (auto &s : streams) if (s.recomp) total += 35 + (s.diffByteOffsets.empty() ? 0 : 8 + 9 * s.diffByteOffsets.size()) + s.inflatedLength + (s.pieces.empty() ? 0 : 8 + 4 * s.pieces.size() + (uint64_t)s.frame * (s.pieces.size() - 1));
         std::vector<uint8_t> out; out.reserve(total + infileSize);
         out.insert(out.end(), {'A', 'T', 'Z', 1});
         put8(out, 0); put8(out, infileSize); put8(out, nrec);
@@ -303,7 +304,7 @@ class ATZcreator {
             auto &s = streams[i];
             if (!s.recomp) continue;
             put8(out, s.offset); put8(out, s.streamLength); put8(out, s.inflatedLength);
-            out.push_back(s.zlibparams.clevel); out.push_back(s.zlibparams.window | (s.pieces.empty() ? 0 : 0x80) | (any_recomp(nests, kids[i]) ? 0x40 : 0)); out.push_back(s.zlibparams.memlevel);
+            out.push_back(s.zlibparams.clevel); out.push_back(s.zlibparams.window | (s.pieces.empty() ? 0 : s.frame == 16 ? 0xa0 : 0x80) | (any_recomp(nests, kids[i]) ? 0x40 : 0)); out.push_back(s.zlibparams.memlevel);
             uint64_t nd = s.diffByteOffsets.size();
             put8(out, nd);
             if (nd > 0) {
@@ -315,7 +316,7 @@ class ATZcreator {
                 put8(out, s.pieces.size());
                 for (uint32_t l : s.pieces) for (int b = 0; b < 4; b++) out.push_back((uint8_t)(l >> (8 * b)));
                 uint64_t at = s.offset;
-                for (size_t k = 0; k + 1 < s.pieces.size(); k++) { at += s.pieces[k]; out.insert(out.end(), file.begin() + at, file.begin() + at + 12); at += 12; }
+                for (size_t k = 0; k + 1 < s.pieces.size(); k++) { at += s.pieces[k]; out.insert(out.end(), file.begin() + at, file.begin() + at + s.frame); at += s.frame; }
             }
             const uint32_t g = owner[i];
             put_payload(out, payload[g].data() + pay_at[g], s.inflatedLength, kids[i]); pay_at[g] += s.inflatedLength;
@@ -425,7 +426,7 @@ class ATZreconstructor {
                 uint64_t at = 0;
                 for (size_t k = 0; k < s.pieces.size(); k++) {
                     recfile.write(reinterpret_cast<const char *>(cb + at), (std::streamsize)s.pieces[k]); at += s.pieces[k];
-                    if (k + 1 < s.pieces.size()) recfile.write(reinterpret_cast<const char *>(atz.data() + s.gapsAt + 12 * k), 12);
+                    if (k + 1 < s.pieces.size()) recfile.write(reinterpret_cast<const char *>(atz.data() + s.gapsAt + s.frame * k), s.frame);
                 }
             }
             lastos = s.offset; lastlen = s.spanLength();
@@ -458,7 +459,7 @@ class ATZreconstructor {
         }
         return lastos;
     }
-    // One record at `lastos`: descriptor, diffs, (window bit 7, --png) the piece table and framing bytes, then the payload or (bit 6,
+    // One record at `lastos`: descriptor, diffs, (window bit 7, --png; with bit 5, --apng) the piece table and framing bytes, then the payload or (bit 6,
     // --nested) u64 nchild, the nested records and the residue.  depth 0 = a top-level record.  Returns the end of the record.
     uint64_t readRecord(const std::vector<uint8_t> &atz, uint64_t lastos, uint64_t origlen, int depth, ATZdata::streamOffset &s, Tree &t) {
         auto need = [&](uint64_t end) { if (end > atz.size()) { std::cout << "Invalid file: truncated stream description" << std::endl; std::exit(1); } };
@@ -484,23 +485,26 @@ class ATZreconstructor {
         s.zlibparams.window &= 0xbf;
         if (depth > 0) {
             if (s.zlibparams.window & 0x80) invalid("a nested stream cannot be split over IDAT chunks");
+            if (s.zlibparams.window & 0x20) invalid("a nested stream cannot be split over fdAT chunks");
             if ((s.zlibparams.clevel & 15) > 9 || (s.zlibparams.clevel >> 4) > 4 || s.zlibparams.window < 9 || s.zlibparams.window > 15 || s.zlibparams.memlevel < 1 || s.zlibparams.memlevel > 9) invalid("bad zlib parameters");
             if (s.streamLength >= 0xffff0000ull || s.inflatedLength >= 0xffffff00ull) invalid("stream too large");
         }
-        if (s.zlibparams.window & 0x80) {   // split over PNG IDAT chunks (--png): piece table and framing bytes, checked before any GPU work
-            s.zlibparams.window &= 0x7f;
+        if ((s.zlibparams.window & 0xa0) == 0x20) invalid("fdAT framing on a stream that is not split");
+        if (s.zlibparams.window & 0x80) {   // split over PNG IDAT chunks (--png) or, bit 5, APNG fdAT chunks (--apng): piece table and framing bytes, checked before any GPU work
+            if (s.zlibparams.window & 0x20) s.frame = 16;
+            s.zlibparams.window &= 0x5f;
             if (s.zlibparams.window < 9 || s.zlibparams.window > 15) invalid("bad window of a split stream");
             need(s.atzInfos + 8);
             const uint64_t np = get8(&atz[s.atzInfos]);
             if (np < 2) invalid("a split stream needs at least 2 pieces");
-            if (np > (atz.size() - s.atzInfos - 8) / 16 + 1) need(atz.size() + 1);   // (the sizes below cannot wrap)
-            need(s.atzInfos + 8 + 16 * np - 12);
+            if (np > (atz.size() - s.atzInfos - 8) / (4 + s.frame) + 1) need(atz.size() + 1);   // (the sizes below cannot wrap)
+            need(s.atzInfos + 8 + 4 * np + s.frame * (np - 1));
             uint64_t sum = 0;
             for (uint64_t k = 0; k < np; k++) { uint32_t l; std::memcpy(&l, &atz[s.atzInfos + 8 + 4 * k], 4); s.pieces.push_back(l); sum += l; }
             if (sum != s.streamLength) invalid("piece lengths of a split stream do not sum to its length");
             if (s.offset > origlen || s.spanLength() > origlen - s.offset) invalid("split stream outside the original file");
             s.gapsAt = s.atzInfos + 8 + 4 * np;
-            s.atzInfos += 8 + 16 * np - 12;
+            s.atzInfos += 8 + 4 * np + s.frame * (np - 1);
         }
         if (s.inflatedLength > atz.size()) need(atz.size() + 1);
         if (!has_nested) {
@@ -612,6 +616,7 @@ static const CliArg kExtArgs[] = {   // antiz_b200 only: listed after the refere
     {"", "small-windows", nullptr, false, "Also look for zlib streams with 256- and 512-byte windows (header bytes 0x08 and 0x18). More streams are found and recompressed, so the ATZ file differs from the reference's, but the reference can still reconstruct from it. Default: disabled"},
     {"", "png", nullptr, false, "Also find zlib streams that PNG files split over consecutive IDAT chunks, and recompress them with the chunk framing between the pieces stored verbatim. The ATZ file then differs from the reference's and only this program can reconstruct from it. Default: disabled"},
     {"", "nested", "integer", false, "Also recompress zlib streams found inside the decompressed data of recompressed streams, down to this many levels (0-8). The ATZ file then differs from the reference's and only this program can reconstruct from it. Default: 0"},
+    {"", "apng", nullptr, false, "Also find zlib streams that animated PNG files split over consecutive fdAT chunks, and recompress them with the chunk framing and sequence numbers between the pieces stored verbatim. Does not imply --png, which the default image needs. The ATZ file then differs from the reference's and only this program can reconstruct from it. Default: disabled"},
 };
 static std::string cli_short_id(const CliArg &a) {
     std::string id = a.flag[0] ? std::string("-") + a.flag : std::string("--") + a.name;
@@ -722,6 +727,7 @@ static void parseCLI(int argc, char *argv[], std::string &infile_name, std::stri
         else if (n == "strategies") options.strategies = true;
         else if (n == "small-windows") options.smallWindows = true;
         else if (n == "png") options.png = true;
+        else if (n == "apng") options.apng = true;
         else if (n == "nested") options.nested = (int)std::min<uint64_t>(x, 9);
         else if (n == "help") { usage(argv[0]); std::exit(0); }
         else if (n == "version") { std::cout << std::endl << argv[0] << "  version: " << antiz_ver << std::endl << std::endl; std::exit(0); }

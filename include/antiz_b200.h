@@ -124,6 +124,16 @@ int  atz_ctx_set_scan_flags(atz_ctx *ctx, uint32_t flags);
  * that span and is dropped if an accepted stream overlaps the span without lying inside it.  May be ORed with ATZ_SCAN_SMALL_WINDOWS.
  * The ATZ file of a run with split streams can only be read by this library's reconstructor. */
 #define ATZ_SCAN_PNG_IDAT 4
+/* Extension (SURVEY.md 8 f4; not in the reference): an animated PNG keeps every frame but its default image in a zlib stream of its own,
+ * split over consecutive fdAT chunks whose data start with a 4-byte sequence number, so 16 bytes of framing (CRC, next length, type and
+ * sequence number) lie between two pieces.  With this flag a K1 candidate that starts an fdAT run (header right behind an "fdAT" tag and
+ * its sequence number, whose chunk is followed by another fdAT; see atz_host_fdat_run) is inflated over the run's pieces like an IDAT
+ * run, with the same rule for what is a split stream; its span in the file is C + 16 * (pieces - 1) bytes (atz_get_framing).  Sequence
+ * numbers and CRCs are not checked.  A header that starts both kinds of run (its sequence number spells "IDAT") is taken as an IDAT run
+ * when ATZ_SCAN_PNG_IDAT is set.  Does not imply ATZ_SCAN_PNG_IDAT (an APNG's default image is in IDAT chunks); may be ORed with it and
+ * with ATZ_SCAN_SMALL_WINDOWS.  Bits 2 and 8 stay unassigned.  The ATZ file of a run with split streams can only be read by this
+ * library's reconstructor. */
+#define ATZ_SCAN_APNG_FDAT 16
 
 /* ---- precompress path ------------------------------------------------------------------------------ */
 
@@ -180,10 +190,13 @@ int atz_get_streams(atz_ctx *ctx, atz_stream *streams, uint64_t cap);
 /* owner[i] = shard that owns stream i: set by atz_scan_finish (sharded scan) or by the last atz_search_shard (0 before that).  The
  * host gathers stream i's record, diff list and plaintext from that context; every context of a run reports the same list. */
 int atz_get_owners(atz_ctx *ctx, uint32_t *owner, uint64_t cap);
-/* The pieces of stream i in the file (ATZ_SCAN_PNG_IDAT): *npieces = 0 for an ordinary stream, >= 2 for a split one, whose piece
- * lengths (summing to streamLength; piece k+1 starts 12 bytes after piece k ends) go to len[0 .. min(npieces, cap)).  ATZ_E_SMALL if
- * cap < npieces.  Every context of a sharded run reports the same pieces. */
+/* The pieces of stream i in the file (ATZ_SCAN_PNG_IDAT, ATZ_SCAN_APNG_FDAT): *npieces = 0 for an ordinary stream, >= 2 for a split
+ * one, whose piece lengths (summing to streamLength; piece k+1 starts atz_get_framing bytes after piece k ends) go to
+ * len[0 .. min(npieces, cap)).  ATZ_E_SMALL if cap < npieces.  Every context of a sharded run reports the same pieces. */
 int atz_get_pieces(atz_ctx *ctx, uint64_t stream_index, uint32_t *len, uint64_t cap, uint64_t *npieces);
+/* The framing bytes between two pieces of stream i: 0 for an ordinary stream, 12 for one split over IDAT chunks (CRC, length, type),
+ * 16 for one split over fdAT chunks (CRC, length, type, sequence number). */
+int atz_get_framing(atz_ctx *ctx, uint64_t stream_index, uint32_t *bytes);
 /* diffByteOffsets (delta-encoded, main.cpp:757-763) and diffByteVal of all recomp streams, concatenated: the top-level streams', then
  * those of the nested streams (atz_get_nested order). */
 int atz_get_diffs(atz_ctx *ctx, uint64_t *offsets, uint8_t *values, uint64_t cap, uint64_t *n);
@@ -241,6 +254,9 @@ int atz_host_header_type(uint32_t scan_flags, uint32_t b0, uint32_t b1);
 /* The IDAT run walker of ATZ_SCAN_PNG_IDAT (the same function the run-detection kernel runs) at file offset p: *npieces = number of
  * IDAT chunks of the run (0: p starts none; a run has >= 2), their data lengths into len[0 .. min(*npieces, cap)). */
 int atz_host_idat_run(const uint8_t *file, uint64_t n, uint64_t p, uint32_t *len, uint64_t cap, uint64_t *npieces);
+/* The same for the fdAT run walker of ATZ_SCAN_APNG_FDAT: p is where the stream's piece starts, behind the first chunk's sequence
+ * number; the lengths are the pieces', L - 4 per chunk. */
+int atz_host_fdat_run(const uint8_t *file, uint64_t n, uint64_t p, uint32_t *len, uint64_t cap, uint64_t *npieces);
 /* owner[k] = shard that searches the k-th accepted stream of a scan, given the streams' inflated lengths.  probed_by == NULL: longest
  * first, each to the least loaded shard (what atz_search_shard uses after a plain atz_scan).  probed_by[k] = shard whose chunk range
  * stream k starts in (what atz_scan_finish uses): a stream stays where its plaintext already is unless that shard holds more than 2 %
